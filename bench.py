@@ -6,8 +6,12 @@ bench.py -- headline benchmark of the photon-transport path: photons/s on the 3-
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # CPU arm: the oracle port on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the tallies of the last timed step to DIR
 
 One "step" = one complete `mcarats_ng` job set (Nrun x Ng jobs = 3 x 1e8 photons) over the synthetic scene.
+`--dump-outputs DIR`: after the timed steps, every tally the timed step returns (`Solver.results()`: radiance, and flux /
+heating when the target has them) is written as DIR/<name>.npy in float64.  The inputs and photon seeds are fixed, so two
+builds run with the same arguments can be compared array for array; above 64 MB in all, a fixed seeded sample is written.
 `value`  : photons/s with the scene already resident in HBM (b200rt_run only; CUDA events on the launching stream).
 `e2e`    : photons/s through the public API, starting from the RAW cloud fields (extinction, effective radius) as host
            numpy arrays: mca_atm_3d(device_props=True) + mcarats_ng + mca_out_ng -- the input builder, scene packing
@@ -209,6 +213,22 @@ def accuracy_summary(sol):
     return out
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(outdir, results):
+    """Write the non-empty tally arrays of `results` as outdir/<name>.npy (float64).  When they exceed DUMP_LIMIT bytes in
+    all, each array is flattened and cut to the same fraction by a sorted sample of positions drawn with a fixed seed."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in results.items() if k != 'stats' and v is not None}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in sorted(arrays.items()):
+        if total > DUMP_LIMIT:
+            keep = a.size * DUMP_LIMIT // total
+            a = a.ravel()[np.sort(np.random.default_rng(SEED).choice(a.size, size=keep, replace=False, shuffle=False))]
+        np.save(os.path.join(outdir, name + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -224,7 +244,13 @@ def main():
     ap.add_argument('--c4-photons', type=float, default=1e9, help='N > 1: photons of the config-4 sweep leg (0 = skip)')
     ap.add_argument('--sv', type=str, default='0,0,0')
     ap.add_argument('--empty-runs', type=int, default=0, help='A/B switch of the resident leg: -1 = no vertical merging of empty coarse cells')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the tallies of the last timed step as DIR/<name>.npy (float64, at most 64 MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs needs the CUDA arm: the reference arm sizes its photon sample from a timing probe')
 
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -330,6 +356,9 @@ def main():
         ms = float(t.item())
     clocks = sampler.stop() if sampler is not None else None
     value = photons_step * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # before the legs below upload other scenes into the same handle
+        dump_outputs(args.dump_outputs, sol.results())
 
     # ---- strong scaling (N > 1): the FIXED BASELINE job set (3 x 1e8 photons) sharded over the ranks, same timing rules
     strong = None

@@ -1,10 +1,14 @@
-"""bench.py contract (CPU side): the reference arm prints exactly ONE JSON line on stdout with the keys the driver reads,
-also when a launcher exports OMP_NUM_THREADS=1 (torchrun does); without a GPU the CUDA arm fails loudly."""
+"""bench.py contract: the reference arm prints exactly ONE JSON line on stdout with the keys a caller reads, also when a
+launcher exports OMP_NUM_THREADS=1 (torchrun does); without a GPU the CUDA arm fails loudly; on the GPU, --dump-outputs
+writes what the last timed step computed."""
 
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), '..'))
 
@@ -36,6 +40,27 @@ def test_reference_arm_other_ranks_print_nothing():
     r = _run(['--impl', 'reference', '--gpus', '2', '--steps', '1', '--warmup', '1', '--photons', '5e4', '--nx', '32', '--nz3', '8'],
              {'RANK': '1', 'WORLD_SIZE': '2', 'LOCAL_RANK': '1'})
     assert r.returncode == 0 and r.stdout.strip() == ''
+
+
+@pytest.mark.gpu
+def test_cuda_arm_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs writes the tallies of the last timed step.  Every step traces the same seeded job set into zeroed
+    tallies, so one timed step and three dump the same arrays, and --steps sets the number of launches timed."""
+    small = ['--gpus', '1', '--warmup', '1', '--photons', '1e5', '--nx', '32', '--nz3', '8', '--e2e-steps', '1',
+             '--no-cpu-baseline', '--no-accuracy']
+    lines, dumps = {}, {}
+    for k in (1, 3):
+        d = tmp_path / ('steps%d' % k)
+        r = _run(small + ['--steps', str(k), '--dump-outputs', str(d)])
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines[k] = json.loads(r.stdout)
+        dumps[k] = {f: np.load(str(d / f)) for f in os.listdir(str(d))}
+    assert lines[1]['steps'] == 1 and lines[3]['steps'] == 3
+    assert lines[3]['gpu_launches'] == 3 * lines[1]['gpu_launches'] > 0
+    a, b = dumps[1], dumps[3]
+    assert sorted(a) == sorted(b) == ['rad.npy']
+    assert a['rad.npy'].dtype == np.float64 and a['rad.npy'].size == 3 * 32 * 32 and a['rad.npy'].max() > 0.0
+    assert np.allclose(a['rad.npy'], b['rad.npy'], rtol=1e-9, atol=1e-15)
 
 
 def test_cuda_arm_fails_loudly_without_a_gpu():

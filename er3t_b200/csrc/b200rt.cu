@@ -84,6 +84,8 @@ struct DevScene {
     int nx, ny, nz, iz0, nz3, np1d, np3d;
     float dx, dy, Lx, Ly, inv_dx, inv_dy, inv_Lx, inv_Ly;
     int svx, svy, svz, ncx, ncy, ncz;
+    unsigned svx_mul, svy_mul;   // fine column -> fine cell without a divide: fx / svx == div_exact(fx, svx_mul, svx_sh)
+    int svx_sh, svy_sh;
     float Sx, Sy, inv_Sx, inv_Sy;
     float Lux, Luy;           // domain size in units of fine cells (nx / svx, ny / svy; the last cell may be partial)
     int nslab_z;
@@ -489,6 +491,12 @@ __device__ __forceinline__ void pool_store_accept(float* __restrict__ f, int s, 
     f[F_LAY * NP + s] = __uint_as_float(unsigned(p.is) | (unsigned(p.iz) << 16));
     f[F_ORD * NP + s] = __uint_as_float(unsigned(p.flags) | (unsigned(p.order) << 8));
     f[F_LEG * NP + s] = apf; f[F_ZA * NP + s] = uz; f[F_AUX * NP + s] = uw; f[F_M * NP + s] = s3;
+}
+
+// x / d for 0 <= x < 2^31 and a divisor fixed per scene, in two instructions instead of the ~28 of a run-time integer
+// divide: (mul, sh) from div_magic() on the host, which also checks the result over the range it is used on
+__device__ __forceinline__ int div_exact(int x, unsigned mul, int sh) {
+    return int((__umulhi(unsigned(x), mul) + unsigned(x)) >> sh);
 }
 
 __device__ __forceinline__ float wrapf(float x, float L, float invL) {
@@ -1393,8 +1401,9 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     if (p.w > 0.0f) {
                         accepted = true;
                         c_apf = apf; c_uz = u.z; c_uw = u.w; c_s3 = s3;
-                        // the fine cell indices follow the collision point (it may lie anywhere in an empty coarse cell)
-                        if (ev_in3 && !frozen) { p.cix = min(S.ncx - 1, fx / S.svx); p.ciy = min(S.ncy - 1, fy / S.svy); }
+                        // the fine cell indices follow the collision point (it may lie anywhere in an empty coarse cell);
+                        // 0 <= fx < nx, so the quotient is below ncx
+                        if (ev_in3 && !frozen) { p.cix = div_exact(fx, S.svx_mul, S.svx_sh); p.ciy = div_exact(fy, S.svy_mul, S.svy_sh); }
                     }
                 }
             }
@@ -1838,6 +1847,18 @@ const char* b200rt_last_error(void* handle) {
     return H ? H->err.c_str() : "null handle";
 }
 
+// (mul, sh) of div_exact(): x / d == (umulhi(x, mul) + x) >> sh with sh = ceil(log2 d) and mul = ceil(2^(32+sh) / d) - 2^32.
+// The error of the 33-bit reciprocal stays below 1/d for every 0 <= x < 2^31; a power of two gives mul = 0, a plain shift.
+static void div_magic(int d, unsigned* mul, int* sh) {
+    int s = 0;
+    while ((1ll << s) < d) ++s;
+    *sh = s;
+    *mul = unsigned(((1ull << (32 + s)) + unsigned(d) - 1) / unsigned(d) - (1ull << 32));
+}
+static int div_exact_host(int x, unsigned mul, int sh) {
+    return int((unsigned((unsigned long long)unsigned(x) * mul >> 32) + unsigned(x)) >> sh);
+}
+
 int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_options* opt) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
@@ -1926,6 +1947,11 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     svx = std::min(svx, sc->nx); svy = std::min(svy, sc->ny); svz = std::max(1, std::min(svz, std::max(1, nz3)));
     S.svx = svx; S.svy = svy; S.svz = svz;
     S.ncx = (sc->nx + svx - 1) / svx; S.ncy = (sc->ny + svy - 1) / svy; S.ncz = nz3 > 0 ? (nz3 + svz - 1) / svz : 0;
+    div_magic(svx, &S.svx_mul, &S.svx_sh); div_magic(svy, &S.svy_mul, &S.svy_sh);
+    for (int x = 0; x < sc->nx; ++x)
+        if (div_exact_host(x, S.svx_mul, S.svx_sh) != x / svx) return fail(H, B200RT_ERR_ARG, "no exact reciprocal of the fine-cell width");
+    for (int y = 0; y < sc->ny; ++y)
+        if (div_exact_host(y, S.svy_mul, S.svy_sh) != y / svy) return fail(H, B200RT_ERR_ARG, "no exact reciprocal of the fine-cell depth");
     // the z-group tables live in shared memory: at most 128 groups in the 3-D block unless the caller chose cmz
     if (opt->cmz <= 0 && !per_level && S.ncz > 128 * cmz) cmz = (S.ncz + 127) / 128;
     H->cmz = cmz;

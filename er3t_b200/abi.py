@@ -13,10 +13,10 @@ import ctypes as C
 
 import numpy as np
 
-__all__ = ['Sensor', 'SceneStruct', 'Job', 'Options', 'Stats', 'load_library', 'library_path',
+__all__ = ['Sensor', 'SceneStruct', 'Job', 'Kd', 'Options', 'Stats', 'load_library', 'library_path',
            'SFC_LAMBERT', 'SFC_DSM', 'SFC_RPV', 'SFC_LSRT',
            'SOLVER_3D', 'SOLVER_PARTIAL_3D', 'SOLVER_IPA',
-           'TARGET_FLUX', 'TARGET_RADIANCE', 'TARGET_HEATING', 'HostScene', 'make_jobs', 'make_options']
+           'TARGET_FLUX', 'TARGET_RADIANCE', 'TARGET_HEATING', 'HostScene', 'make_jobs', 'make_kd', 'make_options']
 
 SFC_LAMBERT, SFC_DSM, SFC_RPV, SFC_LSRT = 1, 2, 3, 4
 SOLVER_3D, SOLVER_PARTIAL_3D, SOLVER_IPA = 0, 1, 2
@@ -58,6 +58,10 @@ class Job(C.Structure):
                 ('abs1d', C.c_void_p), ('flx_scale', C.c_void_p), ('rad_scale', C.c_double)]
 
 
+class Kd(C.Structure):
+    _fields_ = [('nkd', C.c_int32), ('_pad', C.c_int32), ('wkd', C.c_void_p), ('abs1d', C.c_void_p), ('rad_scale', C.c_void_p)]
+
+
 class Options(C.Structure):
     _fields_ = [('solver', C.c_int32), ('target', C.c_int32), ('nslab', C.c_int32),
                 ('shard_rank', C.c_int32), ('shard_world', C.c_int32),
@@ -84,7 +88,7 @@ class Stats(C.Structure):
 
 # every symbol include/b200rt.h declares (tests check the library exports all of them)
 EXPORTS = ['b200rt_version', 'b200rt_create', 'b200rt_destroy', 'b200rt_last_error', 'b200rt_upload_scene',
-           'b200rt_run', 'b200rt_sync', 'b200rt_read_flux', 'b200rt_read_rad', 'b200rt_read_heat',
+           'b200rt_run', 'b200rt_run_kd', 'b200rt_sync', 'b200rt_read_flux', 'b200rt_read_rad', 'b200rt_read_heat',
            'b200rt_tally_ptrs', 'b200rt_stats_get', 'b200rt_philox_fill', 'b200rt_phase_eval',
            'b200rt_phase_sample', 'b200rt_brdf_eval']
 
@@ -121,6 +125,7 @@ def load_library(path=None):
     lib.b200rt_last_error.restype = C.c_char_p
     lib.b200rt_upload_scene.argtypes = [vp, C.POINTER(SceneStruct), C.POINTER(Options)]
     lib.b200rt_run.argtypes = [vp, C.POINTER(Job), C.c_int, C.c_int, vp]
+    lib.b200rt_run_kd.argtypes = [vp, C.POINTER(Job), C.POINTER(Kd), C.c_int, C.c_int, vp]
     lib.b200rt_sync.argtypes = [vp]
     for name in ('b200rt_read_flux', 'b200rt_read_rad', 'b200rt_read_heat'):
         getattr(lib, name).argtypes = [vp, vp, C.c_int64]
@@ -315,6 +320,23 @@ def make_jobs(nphot, seeds, slabs, abs1d=None, flx_scale=None, rad_scale=None):
             jobs[i].flx_scale = _ptr(f)
         jobs[i].rad_scale = 1.0 if rad_scale is None else float(rad_scale[i])
     return jobs, keep
+
+
+def make_kd(abs1d, wkd, rad_scale=None, njob=1):
+    """The k-distribution terms of a spectral run (b200rt_run_kd): `abs1d` (nkd, nz) gas absorption per term (1/m), `wkd`
+    (nkd,) term weights (Atm_wkd0), `rad_scale` (nkd,) per-term radiance factors (default 1).  Returns a ctypes array of
+    `njob` identical Kd records (one per job) plus the list of numpy arrays that must stay alive."""
+    a = _arr(np.atleast_2d(abs1d), np.float64)
+    nkd = a.shape[0]
+    w = _arr(np.ravel(wkd), np.float64)
+    r = _arr(np.ones(nkd) if rad_scale is None else np.ravel(rad_scale), np.float64)
+    if w.size != nkd or r.size != nkd:
+        raise ValueError('Error [make_kd]: <abs1d>, <wkd> and <rad_scale> disagree in the number of terms.')
+    kd = (Kd * int(njob))()
+    for j in range(int(njob)):
+        kd[j].nkd = nkd
+        kd[j].wkd, kd[j].abs1d, kd[j].rad_scale = _ptr(w), _ptr(a), _ptr(r)
+    return kd, [a, w, r]
 
 
 def make_options(solver=SOLVER_3D, target=TARGET_FLUX, nslab=1, shard_rank=0, shard_world=1,

@@ -151,6 +151,12 @@ struct DevScene {
     double* heat;
     unsigned long long* counter;
     DevStats* stats;
+    // spectral runs (b200rt_run_kd, read by the KD kernels only): kd_n gas-absorption terms per job, zero-padded
+    int kd_n;
+    const float2* kd_tab;     // [njob][nz+2][kd_n] row 0: (normalised Atm_wkd0, 0); row 1 + iz: (cumulative gas optical depth at
+                              // level iz, absorption coefficient of layer iz)
+    const double* kd_rf;      // [njob][kd_n] norm x job.rad_scale x kd.rad_scale[g]
+    float* kd_r;              // [block][warp][pool slot][kd_n] per-term state of the photon in each slot (see kd_leg)
 };
 
 // ============================================================================ setup kernels
@@ -629,6 +635,67 @@ __device__ __forceinline__ float abs_tau(const DevScene& S, const Smem& sm, int 
                       dist, inv_absdz);
 }
 
+// ---- spectral runs: kd_n gas-absorption terms (Atm_nkd) share one history -------------------------------------------
+// Gas absorption never changes a trajectory, so every term can ride on the same flights, collisions and draws.  Per term
+// g the photon carries r_g = a_g / sum_h q_h a_h, where a_g = exp(-T_g) is its gas transmission so far in term g and q the
+// normalised term weights, while p.w holds the term-weighted weight W = w sum_h q_h a_h (w: the gas-free weight).  Then
+// w a_g = W r_g for every term, and everything that acts on p.w -- single-scattering albedo, surface reflection, Russian
+// roulette, the energy sums -- acts on W unchanged: roulette on W keeps histories that are absorbed in every term from
+// running forever, and the factor it applies (wfac / W) is common to all terms.  r_g <= 1 / q_g, so the state never
+// overflows.  Regeneration sets r_g = 1.
+// Where a leg ends (collision, surface, escape): e_g = exp(-tau_g(leg)), s = sum_g q_g r_g e_g, W <- W s,
+// r_g <- r_g e_g / s.  Returns s; UPD = false (escape) leaves r alone.  Two passes over the slot's terms, out of line (the
+// terms live in global scratch, DevScene::kd_r, not in registers).  tab: the job's rows of DevScene::kd_tab; dza, dzb:
+// heights of the leg's ends above the bottom of their layers iza, izb; f: the leg's length when iza == izb, else 1 / |u_z|.
+template <bool UPD>
+__device__ __noinline__ float kd_leg(const float2* __restrict__ tab, float* __restrict__ r, int nkd, float dza, int iza, float dzb, int izb,
+                                     float f) {
+    const float2* ta = tab + size_t(1 + iza) * nkd;
+    const float2* tb = tab + size_t(1 + izb) * nkd;
+    float s = 0.0f;
+    for (int g = 0; g < nkd; ++g) {
+        const float2 A = __ldg(ta + g);
+        float t;
+        if (iza == izb) t = A.y * f;
+        else {
+            const float2 B = __ldg(tb + g);
+            t = fabsf((B.x + B.y * dzb) - (A.x + A.y * dza)) * f;
+        }
+        const float re = r[g] * __expf(-t);
+        s = fmaf(__ldg(tab + g).x, re, s);
+        if (UPD) r[g] = re;
+    }
+    if (UPD) {
+        const float inv = s > 0.0f ? 1.0f / s : 0.0f;
+        for (int g = 0; g < nkd; ++g) r[g] *= inv;
+    }
+    return s;
+}
+// Radiance factor of one local estimate from the event (dz above the bottom of layer iz) to the sensor level (dzt above the
+// bottom of layer lt), summed over the terms: sum_g rf_g r_g exp(-tau_abs_g), tau_abs_g = |C_g(zt) - C_g(z)| / |mu_v| from
+// the cumulative gas profiles (O(1) per term).
+__device__ __noinline__ double kd_le_sum(const float2* __restrict__ tab, const double* __restrict__ rf, const float* __restrict__ r,
+                                         int nkd, float dz, int iz, float dzt, int lt, float inv_sz) {
+    const float2* ta = tab + size_t(1 + iz) * nkd;
+    const float2* tb = tab + size_t(1 + lt) * nkd;
+    double sum = 0.0;
+    for (int g = 0; g < nkd; ++g) {
+        const float2 A = __ldg(ta + g), B = __ldg(tb + g);
+        const float t = fabsf((B.x + B.y * dzt) - (A.x + A.y * dz)) * inv_sz;
+        sum += __ldg(rf + g) * double(r[g] * __expf(-t));
+    }
+    return sum;
+}
+__device__ __noinline__ void kd_init(float* __restrict__ r, int nkd) {
+    for (int g = 0; g < nkd; ++g) r[g] = 1.0f;
+}
+// the per-term state of pool slot `slot` of the calling warp (a slot belongs to one warp; __syncwarp after every queue pop
+// orders these accesses as it orders the pool)
+template <int NP>
+__device__ __forceinline__ float* kd_state(const DevScene& S, int slot) {
+    return S.kd_r + ((size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot)) * S.kd_n;
+}
+
 // Exact optical depth toward a sensor for oblique views and sensors inside the atmosphere.
 //   * 1-D extinction and gas absorption are horizontally uniform: their integral over the whole segment is a difference
 //     of the cumulative profiles, O(1) whatever the number of layers;
@@ -745,7 +812,8 @@ __device__ __noinline__ float le_tau_generic(const DevScene& S, const float* __r
 
 // Optical depth (extinction + gas absorption) from the photon position along the sensor direction to the sensor's
 // target level.  fx, fy: fine column if the start point lies in a 3-D layer (else recomputed); s3: 3-D extinction of
-// the start voxel.
+// the start voxel.  KD: without the gas term (kd_le_sum adds it per term).
+template <bool KD>
 __device__ __forceinline__ float le_tau(const DevScene& S, const Smem& sm, const DevSensor& se, const Photon& p, int fx, int fy,
                                         float s3) {
     const int iz = p.iz;
@@ -754,7 +822,7 @@ __device__ __forceinline__ float le_tau(const DevScene& S, const Smem& sm, const
     if (se.fast_ok && se.s.z > 0.0f && (frozen || se.vertical_up)) {
         // ---- vertical (or column-frozen) fast path: O(1) look-ups in the precomputed tables
         float t1 = (sm.e1cum[se.lt] + sm.e1tot[se.lt] * (se.zt - sm.z[se.lt])) - (sm.e1cum[iz] + sm.e1tot[iz] * (p.z - sm.z[iz]));
-        if (p.flags & FL_ABS) {
+        if (!KD && (p.flags & FL_ABS)) {
             const float* ab = S.job_abs + size_t(p.job) * S.nz;
             const float* cb = S.job_cabs + size_t(p.job) * (S.nz + 1);
             t1 += (__ldg(cb + se.lt) + __ldg(ab + se.lt) * (se.zt - sm.z[se.lt])) - (__ldg(cb + iz) + __ldg(ab + iz) * (p.z - sm.z[iz]));
@@ -775,16 +843,18 @@ __device__ __forceinline__ float le_tau(const DevScene& S, const Smem& sm, const
     if (frozen) { fx = p.cix; fy = p.ciy; }
     unsigned nv = 0;
     const RayTarget rt = {se.s, se.zt, se.lt};
-    const float t = le_tau_generic(S, sm.z, sm.e1tot, sm.e1cum, rt, p.x, p.y, p.z, iz, p.job, p.flags & FL_ABS, frozen ? 1 : 0, fx, fy, in3, &nv);
+    const float t = le_tau_generic(S, sm.z, sm.e1tot, sm.e1cum, rt, p.x, p.y, p.z, iz, p.job, KD ? 0 : (p.flags & FL_ABS), frozen ? 1 : 0, fx,
+                                   fy, in3, &nv);
     CNT_ADD(CNT_VISIT, nv);
     return t;
 }
 
 // deposit one local-estimate contribution (fw = weight x angular density toward the sensor, 1/sr)
-template <bool SMT>
+// KD: kdr = the photon's per-term state; the radiance factor is the sum over the terms (kd_le_sum) instead of the job's
+template <bool SMT, bool KD = false>
 __device__ __forceinline__ void le_deposit(const DevScene& S, const Smem& sm, const DevSensor& se, const Photon& p, float fw,
-                                           int fx, int fy, float s3) {
-    const float tau = le_tau(S, sm, se, p, fx, fy, s3);
+                                           int fx, int fy, float s3, const float* kdr = nullptr) {
+    const float tau = le_tau<KD>(S, sm, se, p, fx, fy, s3);
     const float contrib = fw * __expf(-tau) * se.inv_sz;
     int px, py;
     if (p.flags & FL_FROZEN) {
@@ -797,7 +867,12 @@ __device__ __forceinline__ void le_deposit(const DevScene& S, const Smem& sm, co
         py = min(se.nyr - 1, max(0, int(yr * S.inv_Ly * float(se.nyr))));
     }
     const DevJob& J = S.jobs[p.job];
-    rad_add<SMT>(S, sm, size_t(J.slab) * S.rad_slab + se.off + py * se.nxr + px, double(contrib) * J.rad_fac * se.npix);
+    const size_t idx = size_t(J.slab) * S.rad_slab + se.off + py * se.nxr + px;
+    if (KD) {
+        const double fac = kd_le_sum(S.kd_tab + size_t(p.job) * (S.nz + 2) * S.kd_n, S.kd_rf + size_t(p.job) * S.kd_n, kdr, S.kd_n,
+                                     p.z - sm.z[p.iz], p.iz, se.zt - sm.z[se.lt], se.lt, se.inv_sz);
+        rad_add<SMT>(S, sm, idx, double(contrib) * fac * se.npix);
+    } else rad_add<SMT>(S, sm, idx, double(contrib) * J.rad_fac * se.npix);
     CNT_ADD(CNT_LE, 1u);
 }
 
@@ -921,7 +996,9 @@ __device__ __noinline__ float2 pick_component3(const float* __restrict__ ext3, c
 //     slab: the fine slab of a photon that left a box sideways follows from its height, and the layer search for unequal
 //     layers is not part of the flight loop at all (the other kernels keep both, decided at run time).  Measured on config 2: the ~35 never-executed instructions of that search cost 3.4 % (the loop is
 //     instruction-fetch sensitive, profiles/README.md r02_f), hence a template parameter instead of a run-time test.
-template <bool PL, bool FZ, int NP, bool CAM, bool UZ, bool RAD, bool NO3>
+// KD (radiance kernels of b200rt_run_kd only): every history serves S.kd_n gas-absorption terms (kd_leg, kd_le_sum); with
+//     KD = false none of that code exists, so the other kernels are unchanged.
+template <bool PL, bool FZ, int NP, bool CAM, bool UZ, bool RAD, bool NO3, bool KD>
 __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid_constant__ DevScene S) {
     extern __shared__ float4 smem_f4[];
     constexpr bool SMT = PL && UZ;      // block-private tallies exist only in the kernels of plane-parallel / few-column scenes
@@ -1018,6 +1095,10 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
         out = philox_u01x4(p.rc0, p.rc1, p.rc2, unsigned(seed_), unsigned(seed_ >> 32));              \
         p.rc2++;                                                                                      \
     }
+// KD: factor of W for the gas absorption of the leg from (p.za, p.iza) to (zb, layer izb) of photon p in pool slot `slot`
+#define KD_LEG(zb, izb, upd)                                                                                              \
+    kd_leg<upd>(S.kd_tab + size_t(p.job) * (S.nz + 2) * S.kd_n, kd_state<NP>(S, slot), S.kd_n, p.za - sm.z[p.iza], p.iza,             \
+                (zb) - sm.z[(izb)], (izb), p.iza == (izb) ? p.leg : inv_absdz)
 // push the slots of the lanes for which `cond` holds onto queue `q` (length `cnt`); `val` is the queue entry
 #define QPUSH(q, cnt, cond, val)                                              \
     {                                                                         \
@@ -1087,6 +1168,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                 CNT_ADD(CNT_PHOT, 1u);
                 if (want_flux) { flux_tally<SMT>(S, sm, p, 0, S.nz); flux_tally<SMT>(S, sm, p, 1, S.nz); }
                 pool_store<NP>(pool, slot, p, S.inv_Sx, S.inv_Sy);
+                if (KD) kd_init(kd_state<NP>(S, slot), S.kd_n);
             }
             QPUSH(qF, nF, born, slot);
             if (exhausted) nD = ND_DONE;
@@ -1324,7 +1406,10 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
             if (ev == EV_ESC) {
                 if (!PL && (p.flags & FL_ABS)) {
                     const float inv_absdz = p.d.z != 0.0f ? fabsf(1.0f / p.d.z) : RT_INF;
-                    const float wn = p.w * __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, S.nz - 1, p.leg, inv_absdz));
+                    float tr;
+                    if (KD) tr = KD_LEG(p.z, S.nz - 1, false);
+                    else tr = __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, S.nz - 1, p.leg, inv_absdz));
+                    const float wn = p.w * tr;
                     ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                     p.w = wn;
                 }
@@ -1368,7 +1453,10 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     // ---- real collision: gas absorption of the finished leg, scattering component, implicit capture
                     if (!PL && (p.flags & FL_ABS)) {
                         const float inv_absdz = p.d.z != 0.0f ? fabsf(1.0f / p.d.z) : RT_INF;
-                        const float wn = p.w * __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, izn, p.leg, inv_absdz));
+                        float tr;
+                        if (KD) tr = KD_LEG(p.z, izn, true);
+                        else tr = __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, izn, p.leg, inv_absdz));
+                        const float wn = p.w * tr;
                         ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                         p.w = wn;
                     }
@@ -1458,7 +1546,10 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                 p.iz = 0; p.is = 0; p.z = sm.z[0]; p.flags &= ~FL_STALE;
                 if (!PL && (p.flags & FL_ABS)) {
                     const float inv_absdz = p.d.z != 0.0f ? fabsf(1.0f / p.d.z) : RT_INF;
-                    const float wn = p.w * __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, 0, p.leg, inv_absdz));
+                    float tr;
+                    if (KD) tr = KD_LEG(p.z, 0, true);
+                    else tr = __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, 0, p.leg, inv_absdz));
+                    const float wn = p.w * tr;
                     ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                     p.w = wn;
                 }
@@ -1512,7 +1603,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     } else {
                         f = se.s.z > 0.0f ? brdf_eval(sfc_type, prm[0], prm[1], prm[2], prm[3], prm[4], wi, se.s) * se.s.z : 0.0f;
                     }
-                    if (f > 0.0f) le_deposit<SMT>(S, sm, se, p, f * p.w, fx, fy, s3);
+                    if (f > 0.0f) le_deposit<SMT, KD>(S, sm, se, p, f * p.w, fx, fy, s3, KD ? kd_state<NP>(S, slot) : nullptr);
                 }
             }
 
@@ -1562,6 +1653,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
         QPUSH_DEAD(have && !alive, slot);
     }
 #undef RNG4
+#undef KD_LEG
 #undef QPUSH
 #undef QPUSH_DEAD
 
@@ -1628,30 +1720,35 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
 
 typedef void (*transport_fn)(const DevScene);
 template <int NP>
-static transport_fn pick_transport_np(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3) {
+static transport_fn pick_transport_np(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, bool kd) {
     // CAM (all-sky camera sensors present) is its own specialisation: the camera's local estimate is a large cold path
     // whose register pressure must not tax the satellite-view kernels; it needs the 3-D solver (FZ = false).
     // UZ: see the kernel.  RAD = false exists for the per-level kernels only: a pure flux / heating run carries no
     // local-estimate code at all (those kernels are instruction-fetch bound).
-    if (pl) {
-        if (cam) return transport_kernel<true, false, NP, true, false, true, false>;
-        if (rad) {
-            if (fz) return uz ? transport_kernel<true, true, NP, false, true, true, false> : transport_kernel<true, true, NP, false, false, true, false>;
-            return uz ? transport_kernel<true, false, NP, false, true, true, false> : transport_kernel<true, false, NP, false, false, true, false>;
-        }
-        if (fz) return uz ? transport_kernel<true, true, NP, false, true, false, false> : transport_kernel<true, true, NP, false, false, false, false>;
-        if (uz && no3) return transport_kernel<true, false, NP, false, true, false, true>;
-        return uz ? transport_kernel<true, false, NP, false, true, false, false> : transport_kernel<true, false, NP, false, false, false, false>;
+    // KD (b200rt_run_kd): radiance kernels with satellite sensors only; the caller has rejected every other case.
+    if (kd) {
+        if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, true> : transport_kernel<false, true, NP, false, false, true, false, true>;
+        return uz ? transport_kernel<false, false, NP, false, true, true, false, true> : transport_kernel<false, false, NP, false, false, true, false, true>;
     }
-    if (cam) return uz ? transport_kernel<false, false, NP, true, true, true, false> : transport_kernel<false, false, NP, true, false, true, false>;
-    if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false> : transport_kernel<false, true, NP, false, false, true, false>;
-    return uz ? transport_kernel<false, false, NP, false, true, true, false> : transport_kernel<false, false, NP, false, false, true, false>;
+    if (pl) {
+        if (cam) return transport_kernel<true, false, NP, true, false, true, false, false>;
+        if (rad) {
+            if (fz) return uz ? transport_kernel<true, true, NP, false, true, true, false, false> : transport_kernel<true, true, NP, false, false, true, false, false>;
+            return uz ? transport_kernel<true, false, NP, false, true, true, false, false> : transport_kernel<true, false, NP, false, false, true, false, false>;
+        }
+        if (fz) return uz ? transport_kernel<true, true, NP, false, true, false, false, false> : transport_kernel<true, true, NP, false, false, false, false, false>;
+        if (uz && no3) return transport_kernel<true, false, NP, false, true, false, true, false>;
+        return uz ? transport_kernel<true, false, NP, false, true, false, false, false> : transport_kernel<true, false, NP, false, false, false, false, false>;
+    }
+    if (cam) return uz ? transport_kernel<false, false, NP, true, true, true, false, false> : transport_kernel<false, false, NP, true, false, true, false, false>;
+    if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, false> : transport_kernel<false, true, NP, false, false, true, false, false>;
+    return uz ? transport_kernel<false, false, NP, false, true, true, false, false> : transport_kernel<false, false, NP, false, false, true, false, false>;
 }
-static transport_fn pick_transport(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, int np) {
+static transport_fn pick_transport(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, bool kd, int np) {
     switch (np) {
-        case 64: return pick_transport_np<64>(pl, fz, cam, uz, rad, no3);
-        case 128: return pick_transport_np<128>(pl, fz, cam, uz, rad, no3);
-        default: return pick_transport_np<96>(pl, fz, cam, uz, rad, no3);
+        case 64: return pick_transport_np<64>(pl, fz, cam, uz, rad, no3, kd);
+        case 128: return pick_transport_np<128>(pl, fz, cam, uz, rad, no3, kd);
+        default: return pick_transport_np<96>(pl, fz, cam, uz, rad, no3, kd);
     }
 }
 
@@ -1707,6 +1804,7 @@ struct Handle {
     DevBuf st_e, st_o, st_a, st_b, f2c;
     DevBuf ext3tot, prop3, ext3, maj, tu3, pmu, pp, pcdf, pgs, pge, sfc_type, sfc_param;
     DevBuf jobs, job_abs, job_cabs, job_fscale, counter, stats, flag;
+    DevBuf kd_tab, kd_rf, kd_r;   // spectral runs: per-term tables and the per-slot term state
     DevBuf flux, rad, heat;
     size_t nflux = 0, nrad = 0, nheat = 0;
     std::vector<float> h_zgrd;
@@ -1833,7 +1931,7 @@ int b200rt_destroy(void* handle) {
                      &H->st_e, &H->st_o, &H->st_a, &H->st_b, &H->f2c, &H->slab_cg, &H->group_lo, &H->group_cz, &H->group_maj1d, &H->gz_lo, &H->empty3, &H->runcode,
                      &H->ext3tot, &H->prop3, &H->ext3, &H->maj, &H->tu3, &H->pmu, &H->pp, &H->pcdf, &H->pgs, &H->pge, &H->sfc_type,
                      &H->sfc_param, &H->jobs, &H->job_abs, &H->job_cabs, &H->job_fscale, &H->counter, &H->stats, &H->flag,
-                     &H->flux, &H->rad, &H->heat};
+                     &H->kd_tab, &H->kd_rf, &H->kd_r, &H->flux, &H->rad, &H->heat};
     for (DevBuf* b : all) b->release();
     if (H->ev0) cudaEventDestroy(H->ev0);
     if (H->ev1) cudaEventDestroy(H->ev1);
@@ -2310,22 +2408,52 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     return B200RT_OK;
 }
 
-int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream) {
-    Handle* H = static_cast<Handle*>(handle);
-    if (!H) return B200RT_ERR_ARG;
+}  // extern "C"
+
+// b200rt_run (kd == nullptr) and b200rt_run_kd (kd[njob]: the gas-absorption terms of every job)
+static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream) {
     if (!H->have_scene) return fail(H, B200RT_ERR_STATE, "b200rt_run called before b200rt_upload_scene");
     if (!jobs || njob < 1) return fail(H, B200RT_ERR_ARG, "no jobs");
     if (njob > 65535) return fail(H, B200RT_ERR_ARG, "at most 65535 jobs per run");
+    DevScene& S = H->S;
+    const int nz = S.nz;
+    const bool k_rad = (S.target & B200RT_TARGET_RADIANCE) != 0 && S.nrad > 0;
+    const char* kenv = getenv("B200RT_KERNEL");
+    const int kver = kenv ? atoi(kenv) : (H->opt.kernel == 9 ? 9 : 8);
+    int kd_n = 0;
+    if (kd) {
+        if (H->k_pl)
+            return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: radiance targets only (no flux / heating; tiny radiance tallies held in shared memory "
+                                           "need options.smem_tally = -1)");
+        if (!k_rad) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: needs the radiance target and at least one sensor");
+        if (H->k_cam) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: the all-sky camera (Rad_mrkind = 1) is not supported");
+        if (kver == 9) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: not available with options.kernel = 9");
+        for (int j = 0; j < njob; ++j) {
+            const b200rt_kd& k = kd[j];
+            if (k.nkd < 1 || k.nkd > 32) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: nkd must be 1 ... 32");
+            if (!k.wkd || !k.abs1d || !k.rad_scale) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: wkd, abs1d and rad_scale are required");
+            if (jobs[j].abs1d || jobs[j].flx_scale) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: job.abs1d and job.flx_scale must be NULL");
+            double sw = 0;
+            for (int g = 0; g < k.nkd; ++g) {
+                if (!(k.wkd[g] >= 0) || !std::isfinite(k.wkd[g]) || !std::isfinite(k.rad_scale[g]))
+                    return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: wkd must be finite and >= 0, rad_scale finite");
+                sw += k.wkd[g];
+            }
+            if (!(sw > 0)) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: the weights wkd sum to zero");
+            kd_n = std::max(kd_n, k.nkd);
+        }
+    }
     CK(cudaSetDevice(H->device));
     CK(drain(H));                 // one run in flight per handle: the previous one still reads the job tables and counters
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    DevScene& S = H->S;
-    const int nz = S.nz;
-    // per-job tables are built in page-locked memory and uploaded asynchronously on the caller's stream
+    // per-job tables (and the per-term tables of a spectral run) are built in page-locked memory and uploaded
+    // asynchronously on the caller's stream
+    auto al = [](size_t b) { return (b + 15) & ~size_t(15); };
     const size_t b_jobs = size_t(njob) * sizeof(DevJob), b_abs = size_t(njob) * nz * 4, b_cabs = size_t(njob) * (nz + 1) * 4,
-                 b_fs = size_t(njob) * (nz + 1) * 8;
-    const size_t o_jobs = 0, o_fs = (b_jobs + 15) & ~size_t(15), o_abs = o_fs + ((b_fs + 15) & ~size_t(15)), o_cabs = o_abs + ((b_abs + 15) & ~size_t(15));
-    const size_t need = o_cabs + b_cabs + 16;
+                 b_fs = size_t(njob) * (nz + 1) * 8, b_kt = size_t(njob) * (nz + 2) * kd_n * 8, b_kr = size_t(njob) * kd_n * 8;
+    const size_t o_jobs = 0, o_fs = al(b_jobs), o_abs = o_fs + al(b_fs), o_cabs = o_abs + al(b_abs), o_kt = o_cabs + al(b_cabs),
+                 o_kr = o_kt + al(b_kt);
+    const size_t need = o_kr + b_kr + 16;
     if (need > H->pin_bytes) {
         if (H->pin) cudaFreeHost(H->pin);
         H->pin = nullptr; H->pin_bytes = 0;
@@ -2337,8 +2465,12 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
     double* jfs = reinterpret_cast<double*>(pin + o_fs);
     float* jabs = reinterpret_cast<float*>(pin + o_abs);
     float* jcabs = reinterpret_cast<float*>(pin + o_cabs);
+    float2* kt = reinterpret_cast<float2*>(pin + o_kt);
+    double* kr = reinterpret_cast<double*>(pin + o_kr);
     std::memset(jabs, 0, b_abs);
     std::memset(jcabs, 0, b_cabs);
+    std::memset(kt, 0, b_kt);                    // terms beyond a job's nkd: no absorption, weight 0, radiance factor 0
+    std::memset(kr, 0, b_kr);
     unsigned long long acc = 0;
     for (int j = 0; j < njob; ++j) {
         const b200rt_job& q = jobs[j];
@@ -2365,6 +2497,25 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
             }
             jcabs[size_t(j) * (nz + 1) + nz] = float(c);
         }
+        if (kd) {
+            const b200rt_kd& k = kd[j];
+            double sw = 0;
+            for (int g = 0; g < k.nkd; ++g) sw += k.wkd[g];
+            float2* tj = kt + size_t(j) * (nz + 2) * kd_n;
+            for (int g = 0; g < k.nkd; ++g) {
+                tj[g] = make_float2(float(k.wkd[g] / sw), 0.0f);
+                kr[size_t(j) * kd_n + g] = d.rad_fac * k.rad_scale[g];
+                double c = 0;
+                for (int i = 0; i < nz; ++i) {
+                    const double a = k.abs1d[size_t(g) * nz + i];
+                    if (!(a >= 0) || !std::isfinite(a)) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: abs1d must be finite and >= 0");
+                    if (a > 0) d.has_abs = 1;
+                    tj[size_t(1 + i) * kd_n + g] = make_float2(float(c), float(a));
+                    c += a * (double(H->h_zgrd[i + 1]) - double(H->h_zgrd[i]));
+                }
+                tj[size_t(1 + nz) * kd_n + g] = make_float2(float(c), 0.0f);
+            }
+        }
         // complete tally scale per level: normalisation x columns in the domain x the caller's per-level factor
         const double nxy_d = double(S.nx) * double(S.ny);
         for (int i = 0; i <= nz; ++i) jfs[size_t(j) * (nz + 1) + i] = d.norm * nxy_d * (q.flx_scale ? q.flx_scale[i] : 1.0);
@@ -2374,12 +2525,18 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
     }
     int rc;
     if ((rc = dev_alloc(H, H->jobs, b_jobs)) || (rc = dev_alloc(H, H->job_abs, b_abs)) || (rc = dev_alloc(H, H->job_cabs, b_cabs)) ||
-        (rc = dev_alloc(H, H->job_fscale, b_fs)))
+        (rc = dev_alloc(H, H->job_fscale, b_fs)) || (rc = dev_alloc(H, H->kd_tab, b_kt)) ||
+        (rc = dev_alloc(H, H->kd_rf, b_kr)))
         return rc;
     CK(cudaMemcpyAsync(H->jobs.p, dj, b_jobs, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(H->job_abs.p, jabs, b_abs, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(H->job_cabs.p, jcabs, b_cabs, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(H->job_fscale.p, jfs, b_fs, cudaMemcpyHostToDevice, st));
+    if (kd) {
+        CK(cudaMemcpyAsync(H->kd_tab.p, kt, b_kt, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(H->kd_rf.p, kr, b_kr, cudaMemcpyHostToDevice, st));
+    }
+    S.kd_n = kd_n; S.kd_tab = (const float2*)H->kd_tab.p; S.kd_rf = (const double*)H->kd_rf.p;
     S.njob = njob; S.jobs = (const DevJob*)H->jobs.p; S.job_abs = (const float*)H->job_abs.p;
     S.job_cabs = (const float*)H->job_cabs.p; S.job_fscale = (const double*)H->job_fscale.p;
     S.nphot_local = acc;
@@ -2395,8 +2552,6 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
     // launch shape: the per-warp photon pools decide how many blocks fit on an SM (shared memory), see DESIGN.md
     int tpb = H->opt.threads_per_block > 0 ? H->opt.threads_per_block : RT_TPB;
     tpb = std::min(RT_TPB, std::max(32, (tpb / 32) * 32));
-    const char* kenv = getenv("B200RT_KERNEL");
-    const int kver = kenv ? atoi(kenv) : (H->opt.kernel == 9 ? 9 : 8);
 #ifndef B200RT_WITH_V9
     if (kver == 9) return fail(H, B200RT_ERR_ARG, "options.kernel = 9 (role-specialised experiment) is not part of this build (-DB200RT_WITH_V9)");
 #else
@@ -2428,8 +2583,7 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
     int bps = 0;
     // UZ kernels: equally thick 3-D layers with runs (S.uz_ok) -- or no 3-D block at all (the layer search is dead code then)
     const bool k_uz = H->k_pl ? (S.nz3 <= 0 || size_t(S.nx) * S.ny <= 64) : ((S.uz_ok != 0 && H->cmz == 1) || S.nz3 <= 0);
-    const bool k_rad = (S.target & B200RT_TARGET_RADIANCE) != 0 && S.nrad > 0;
-    transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, np);
+    transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, kd != nullptr, np);
     const size_t smem = H->smem_tables + 32 * (4 * 8 + 8 * 4) + size_t(tpb) * 8 + size_t(tpb / 32) * size_t(POOL_WORDS(np)) * 4 +
                         8 * size_t(S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem) * size_t(S.tal_per_warp ? RT_TPB / 32 : 1);
     if (smem > 227 * 1024) return fail(H, B200RT_ERR_ARG, "photon pools + 1-D tables exceed shared memory; lower threads_per_block or pool_slots");
@@ -2439,6 +2593,11 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
     if (H->opt.blocks_per_sm > 0) bps = std::min(bps, H->opt.blocks_per_sm);
     unsigned long long want = (acc + tpb - 1) / tpb;
     int grid = int(std::min<unsigned long long>((unsigned long long)H->numSM * bps, std::max<unsigned long long>(1, want)));
+    if (kd) {
+        // per-term state of every pool slot of the launch: [block][warp][slot][kd_n]
+        if ((rc = dev_alloc(H, H->kd_r, size_t(grid) * (tpb / 32) * np * kd_n * 4))) return rc;
+        S.kd_r = (float*)H->kd_r.p;
+    }
     CK(cudaEventRecord(H->ev0, st));
     kern<<<grid, tpb, smem, st>>>(S);
     CK(cudaGetLastError());
@@ -2449,6 +2608,21 @@ int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, v
     H->inflight = true;
     H->launches = 1;
     return B200RT_OK;
+}
+
+extern "C" {
+
+int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    return run_jobs(H, jobs, nullptr, njob, accumulate, cuda_stream);
+}
+
+int b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    if (!kd) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: kd is NULL");
+    return run_jobs(H, jobs, kd, njob, accumulate, cuda_stream);
 }
 
 int b200rt_sync(void* handle) {

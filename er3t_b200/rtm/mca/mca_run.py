@@ -25,17 +25,22 @@ class mca_run:
     seeds   : Philox key per job
     slabs   : output slab per job
     abs1d, flx_scale, rad_scale : per-job arrays / factors (see include/b200rt.h)
+    kd      : keywords of abi.make_kd (spectral run, b200rt_run_kd: every job serves all these terms) or None
 
     Ncpu, mp_mode are accepted for signature compatibility and ignored.
     """
 
     def __init__(self, scene, options, photons, seeds, slabs, abs1d=None, flx_scale=None, rad_scale=None,
-                 device=0, solver_obj=None, Ncpu=None, mp_mode='py', verbose=False, quiet=False, run=True):
+                 device=0, solver_obj=None, Ncpu=None, mp_mode='py', verbose=False, quiet=False, run=True, kd=None):
         self.scene = scene
         self.options = options
         self.quiet = quiet
         self.verbose = verbose
         self.jobs, self._keep = abi.make_jobs(photons, seeds, slabs, abs1d=abs1d, flx_scale=flx_scale, rad_scale=rad_scale)
+        self.kd = None
+        if kd is not None:
+            self.kd, keep = abi.make_kd(njob=len(self.jobs), **kd)
+            self._keep += keep
         self.solver = solver_obj if solver_obj is not None else Solver(device=device)
         self._own = solver_obj is None
         self.results = None
@@ -45,7 +50,10 @@ class mca_run:
     def launch(self):
         """upload the scene and trace all jobs (synchronous); the tallies stay on the device"""
         self.solver.upload_scene(self.scene, self.options)
-        self.solver.run(self.jobs)
+        if self.kd is not None:
+            self.solver.run_kd(self.jobs, self.kd)
+        else:
+            self.solver.run(self.jobs)
 
     def run(self):
         self.launch()

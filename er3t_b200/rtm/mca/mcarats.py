@@ -12,7 +12,7 @@ What is new (keyword-only, all optional): `seed` (reproducible Philox streams; d
 mcarats.py:432), `device`, `raw` (keep per-job fields instead of g-weighted per-run sums), `write_files` (emit the
 namelist text and MCARaTS-style .bin/.ctl outputs), `iz3l_fix`, `supervoxel`, `shard` / `reduce` (multi-GPU),
 `extra_sensors`, `solver_obj` (reuse a handle), `camera_pixels` (all-sky camera grid instead of the reference's fixed
-500 x 500).
+500 x 500), `spectral` (MCARaTS's multi-term mode, Atm_nkd = Ng: one history serves every g of the wavelength).
 """
 
 import datetime
@@ -79,7 +79,12 @@ class mcarats_ng:
                  solver_obj=None,
                  wmin=None,
                  camera_pixels=None,
-                 dry_run=False):
+                 dry_run=False,
+                 spectral=False):
+        """spectral=True: one job per run traces `photons` histories (not photons per g), each of which carries all Ng
+        terms of the correlated-k set (Atm_nkd = Ng, Atm_wkd0 = weights; Iwabuchi and Okamura 2017).  `self.fused` has the
+        same layout and meaning as without it.  Needs target='radiance' with the satellite sensor and an `abs` object;
+        `raw`, `write_files`, flux / heating targets and the all-sky camera raise OSError."""
 
         add_reference(self.reference)
 
@@ -121,6 +126,7 @@ class mcarats_ng:
         self._wmin = wmin
         self.camera_pixels = camera_pixels
         self.dry_run = dry_run
+        self.spectral = spectral
         self.atm_1ds = atm_1ds
         self.atm_3ds = atm_3ds
 
@@ -150,6 +156,7 @@ class mcarats_ng:
             weights = np.repeat(1.0 / self.Ng, Ng)
         else:
             self.np_mode = 'weighted'
+        self.weights = np.asarray(weights, dtype=np.float64)
         photons_dist = distribute_photon(photons, weights, base_ratio=base_ratio)
         self.photons = np.tile(photons_dist, Nrun)
         self.photons_per_set = photons_dist.sum()
@@ -403,6 +410,15 @@ class mcarats_ng:
         else:
             tflag = abi.TARGET_RADIANCE
 
+        if self.spectral:
+            if self.keep_raw:
+                raise OSError('Error [mcarats_ng]: <spectral=True> sums the g terms in every history: <raw> and <write_files> are not available.')
+            if self.target != 'radiance':
+                raise OSError('Error [mcarats_ng]: <spectral=True> supports target=\'radiance\' only (flux and heating rates are not available yet).')
+            if 'satellite' not in self.sensor_type.lower():
+                raise OSError('Error [mcarats_ng]: <spectral=True> supports the satellite sensor only (not the all-sky camera).')
+            if self.abs is None:
+                raise OSError('Error [mcarats_ng]: <spectral=True> needs the gas absorption object of <atm_1ds> (its g weights and solar factors).')
         fuse = (not self.keep_raw) and (self.abs is not None)
         self.fuse = fuse
         if fuse:
@@ -414,7 +430,7 @@ class mcarats_ng:
 
         nphot, seeds, slabs, abs1d, fsc, rsc = [], [], [], [], [], []
         for ir in range(Nrun):
-            for ig in range(Ng):
+            for ig in range(Ng if not self.spectral else 0):
                 nphot.append(int(self.photons[ir * Ng + ig]))
                 seeds.append(int(self.seeds[ir, ig]))
                 slabs.append(ir if fuse else ir * Ng + ig)
@@ -425,10 +441,32 @@ class mcarats_ng:
                 abs1d.append(a1)
                 fsc.append(f_lev[:, ig].astype(np.float64) if fuse else None)
                 rsc.append(float(f_rad[0, ig]) if fuse else 1.0)
+        kd = None
+        if self.spectral:
+            # one job per run; term g: Atm_abs1d(1:, 1) x Atm_fabs1d of self.nml[ig] as above, radiance factor f_rad[0, ig]
+            key = 'Atm_abs1d(1:, 1)'
+            terms = []
+            for ig in range(Ng):
+                a1 = np.asarray(self.nml[ig][key], dtype=np.float64) if key in self.nml[ig] else np.zeros(nz)
+                if 'Atm_fabs1d' in self.nml[ig]:
+                    a1 = a1 * float(self.nml[ig]['Atm_fabs1d'])
+                terms.append(a1)
+            kd = dict(abs1d=np.stack(terms), wkd=self.weights, rad_scale=f_rad[0, :].astype(np.float64))
+            for ir in range(Nrun):
+                nphot.append(int(self.photons_per_set))
+                seeds.append(int(self.seeds[ir, 0]))
+                slabs.append(ir)
+                abs1d.append(None)
+                fsc.append(None)
+                rsc.append(1.0)
         wmin = DEFAULTS['Pho_wmin'] if self._wmin is None else self._wmin
+        # (spectral: tiny radiance tallies go through global atomics; the kernels that keep them in shared memory are the
+        # per-level ones, which have no spectral variant)
         opt = abi.make_options(solver=solvers[self.solver], target=tflag, nslab=nslab, shard_rank=self.shard[0], shard_world=self.shard[1],
-                               sv=self.supervoxel, iso_ss=DEFAULTS['Pho_iso_SS'], iso_max=DEFAULTS['Pho_iso_max'], wmin=wmin, wfac=DEFAULTS['Pho_wfac'])
+                               sv=self.supervoxel, iso_ss=DEFAULTS['Pho_iso_SS'], iso_max=DEFAULTS['Pho_iso_max'], wmin=wmin, wfac=DEFAULTS['Pho_wfac'],
+                               smem_tally=-1 if self.spectral else 0)
         jobs_args = dict(nphot=nphot, seeds=seeds, slabs=slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc)
+        self.kd_args = kd
         self.options, self.jobs_args, self.nslab = opt, jobs_args, nslab
         if self.dry_run:
             # everything is prepared (scene, options, jobs) but nothing is traced; used by bench.py to time the
@@ -437,7 +475,7 @@ class mcarats_ng:
             return
         # the reference hands the job list to `mca_run` (mcarats.py:468); so does this class -- one launch instead of a pool
         runner = mca_run(scene, opt, nphot, seeds, slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc, device=self.device,
-                         solver_obj=self._solver_obj, Ncpu=self.Ncpu, mp_mode=self.mp_mode, quiet=True, run=False)
+                         solver_obj=self._solver_obj, Ncpu=self.Ncpu, mp_mode=self.mp_mode, quiet=True, run=False, kd=kd)
         try:
             self.h2d_bytes = scene.nbytes() + sum(a.nbytes for a in runner._keep)
             runner.launch()

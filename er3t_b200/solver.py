@@ -61,6 +61,14 @@ class Solver:
         if sync:
             self.sync()
 
+    def run_kd(self, jobs, kd, accumulate=False, stream=None, sync=True):
+        """Spectral run: jobs (abi.make_jobs, without abs1d / flx_scale) and kd (abi.make_kd, one record per job): every
+        history serves all k-distribution terms of its job."""
+        self._keep = (jobs, kd)
+        self._check(self.lib.b200rt_run_kd(self.handle, jobs, kd, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run_kd')
+        if sync:
+            self.sync()
+
     def sync(self):
         self._check(self.lib.b200rt_sync(self.handle), 'b200rt_sync')
 

@@ -10,6 +10,8 @@
  *   b200rt_run                       <- mp.Pool.imap(execute_command) over Nrun*Ng jobs,
  *                                       er3t/rtm/mca/mca_run.py:144-159 (photon counts, solver mode,
  *                                       per-job seed of mcarats.py:432-437)
+ *   b200rt_run_kd                    <- MCARaTS's multi-term mode (Atm_nkd > 1, Atm_wkd0; Iwabuchi and Okamura 2017):
+ *                                       one job per run serves all Ng terms of a wavelength
  *   b200rt_read_flux / _rad / _heat  <- `.bin` + `.ctl` parsing, er3t/rtm/mca/mca_out.py:48-103
  *                                       (and, through job.flx_scale / job.rad_scale, the g-weighting of
  *                                        mca_out.py:319-327,354-366,444-452,475-481)
@@ -142,6 +144,17 @@ typedef struct b200rt_job {
     double   rad_scale;           /* factor for radiance (mca_out.py:449-452, iz = 0)          */
 } b200rt_job;
 
+/* Atm_nkd k-distribution terms of one job (b200rt_run_kd): gas absorption never changes a trajectory, so one history
+ * serves every term.  Run r estimates sum_g rad_scale[g] * E[radiance of term g]; Russian roulette and the energy sums of
+ * b200rt_stats act on the term-weighted weight W = w * sum_g q_g exp(-T_g), q_g = wkd[g] / sum(wkd), T_g = the history's
+ * gas-absorption optical path in term g. */
+typedef struct b200rt_kd {
+    int32_t nkd, _pad;              /* 1 ... 32                                                                        */
+    const double* wkd;              /* [nkd] Atm_wkd0: weights of roulette and energy sums (normalised by the library) */
+    const double* abs1d;            /* [nkd][nz] gas absorption per term, 1/m, host pointer                            */
+    const double* rad_scale;        /* [nkd] per-term radiance factor                                                  */
+} b200rt_kd;
+
 typedef struct b200rt_options {
     int32_t solver;               /* B200RT_SOLVER_*                                           */
     int32_t target;               /* OR of B200RT_TARGET_*                                     */
@@ -206,6 +219,11 @@ int          b200rt_upload_scene(void* handle, const b200rt_scene* scene, const 
  * Tallies are zeroed first unless `accumulate` != 0.  ONE run may be in flight per handle: a second b200rt_run,
  * b200rt_upload_scene or b200rt_read_* first waits for the stream of the run in flight. */
 int          b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream);
+
+/* b200rt_run with kd[j] the k-distribution terms of jobs[j] (radiance target with satellite sensors only: flux / heating
+ * targets, the all-sky camera and options.kernel = 9 are rejected).  jobs[j].abs1d and .flx_scale must be NULL;
+ * jobs[j].rad_scale is a factor common to all terms.  Same asynchronous contract as b200rt_run. */
+int          b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream);
 
 /* Wait for the stream of the last run; checks tallies for NaN/Inf. */
 int          b200rt_sync(void* handle);

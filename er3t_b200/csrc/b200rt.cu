@@ -157,6 +157,12 @@ struct DevScene {
                               // level iz, absorption coefficient of layer iz)
     const double* kd_rf;      // [njob][kd_n] norm x job.rad_scale x kd.rad_scale[g]
     float* kd_r;              // [block][warp][pool slot][kd_n] per-term state of the photon in each slot (see kd_leg)
+    // radiance Jacobians (b200rt_run_jac, read by the JAC kernels only): jac_n groups of contiguous layers
+    int jac_n;
+    const int* jac_lev;       // [jac_n+1] group edges as layer indices, 0 = jac_lev[0] < ... < jac_lev[jac_n] = nz
+    const unsigned char* jac_grp;   // [nz] group of every layer
+    float* jac_t;             // [block][warp][pool slot][jac_n] gas optical path of the slot's history per group (see jac_leg)
+    double* jac;              // [nslab][rad_slab][jac_n] tally of dI / dln(a_j)
 };
 
 // ============================================================================ setup kernels
@@ -696,6 +702,67 @@ __device__ __forceinline__ float* kd_state(const DevScene& S, int slot) {
     return S.kd_r + ((size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot)) * S.kd_n;
 }
 
+// ---- radiance Jacobians: dI / dln(a_j), a_j a factor on the gas absorption (job.abs1d) of every layer of group j -------
+// Gas absorption never changes a trajectory, so a local estimate's contribution c = w0 exp(-T_hist - tau_LE) ... depends
+// on a_j only through the gas optical paths, and d c / d ln(a_j) = -c (T_j + tau_LE_j): T_j the gas optical path the
+// history has collected inside group j since it started, tau_LE_j that of the event -> sensor segment.  The score is the
+// photon weight times a function of the history, so Russian roulette (which keeps the expected weight given the past)
+// leaves it unbiased.  The slot carries T_j in global scratch (DevScene::jac_t), updated where a leg ends at a collision
+// or the surface; an escape leg needs nothing (no local estimate follows it).
+// jac_leg splits the gas optical path of the leg from (dza above the bottom of layer iza) to (dzb above the bottom of izb)
+// over the groups it crosses, exactly as abs_tau_at computes the leg's whole path: inside one layer abs * f (f = length),
+// else clamped differences of the cumulative profile times f = 1 / |u_z|, so that sum_j of the increments is the leg's
+// tau to rounding.  ab, cb: the job's rows of DevScene::job_abs / job_cabs.
+__device__ __noinline__ void jac_leg(const float* __restrict__ ab, const float* __restrict__ cb, const int* __restrict__ lev,
+                                     const unsigned char* __restrict__ grp, float* __restrict__ t, float dza, int iza, float dzb,
+                                     int izb, float f) {
+    if (iza == izb) {
+        t[__ldg(grp + iza)] += __ldg(ab + iza) * f;
+        return;
+    }
+    const float ca = __ldg(cb + iza) + __ldg(ab + iza) * dza;
+    const float c2 = __ldg(cb + izb) + __ldg(ab + izb) * dzb;
+    const float lo = fminf(ca, c2), hi = fmaxf(ca, c2);
+    const int g1 = __ldg(grp + max(iza, izb));
+    for (int j = __ldg(grp + min(iza, izb)); j <= g1; ++j) {
+        const float a = fmaxf(lo, __ldg(cb + __ldg(lev + j))), b = fminf(hi, __ldg(cb + __ldg(lev + j + 1)));
+        if (b > a) t[j] += (b - a) * f;
+    }
+}
+// Deposit -c (T_j + tau_LE_j) for every group with a non-zero path into out[0 .. ngrp) (the groups of one radiance pixel,
+// adjacent).  tau_LE_j: overlap of [event (dz above the bottom of layer iz), sensor level (dzt above the bottom of lt)]
+// with group j from the cumulative profile, times inv_sz.  Returns the number of tally updates.
+__device__ __noinline__ unsigned jac_deposit(double* __restrict__ out, const float* __restrict__ t, int ngrp, const float* __restrict__ ab,
+                                             const float* __restrict__ cb, const int* __restrict__ lev,
+                                             const unsigned char* __restrict__ grp, float dz, int iz, float dzt, int lt, float inv_sz,
+                                             double c) {
+    const float ca = __ldg(cb + iz) + __ldg(ab + iz) * dz;
+    const float cs = __ldg(cb + lt) + __ldg(ab + lt) * dzt;
+    const float lo = fminf(ca, cs), hi = fmaxf(ca, cs);
+    const int g0 = __ldg(grp + min(iz, lt)), g1 = __ldg(grp + max(iz, lt));
+    unsigned n = 0;
+    for (int j = 0; j < ngrp; ++j) {
+        float tau = t[j];
+        if (j >= g0 && j <= g1) {
+            const float a = fmaxf(lo, __ldg(cb + __ldg(lev + j))), b = fminf(hi, __ldg(cb + __ldg(lev + j + 1)));
+            if (b > a) tau += (b - a) * inv_sz;
+        }
+        if (tau != 0.0f) {
+            tally_add(out + j, -c * double(tau));
+            ++n;
+        }
+    }
+    return n;
+}
+__device__ __noinline__ void jac_init(float* __restrict__ t, int ngrp) {
+    for (int j = 0; j < ngrp; ++j) t[j] = 0.0f;
+}
+// the per-group state of pool slot `slot` of the calling warp (ordered like kd_state)
+template <int NP>
+__device__ __forceinline__ float* jac_state(const DevScene& S, int slot) {
+    return S.jac_t + ((size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot)) * S.jac_n;
+}
+
 // Exact optical depth toward a sensor for oblique views and sensors inside the atmosphere.
 //   * 1-D extinction and gas absorption are horizontally uniform: their integral over the whole segment is a difference
 //     of the cumulative profiles, O(1) whatever the number of layers;
@@ -851,7 +918,8 @@ __device__ __forceinline__ float le_tau(const DevScene& S, const Smem& sm, const
 
 // deposit one local-estimate contribution (fw = weight x angular density toward the sensor, 1/sr)
 // KD: kdr = the photon's per-term state; the radiance factor is the sum over the terms (kd_le_sum) instead of the job's
-template <bool SMT, bool KD = false>
+// JAC: kdr = the photon's per-group gas optical paths; the same contribution also goes to the Jacobian tally (jac_deposit)
+template <bool SMT, bool KD = false, bool JAC = false>
 __device__ __forceinline__ void le_deposit(const DevScene& S, const Smem& sm, const DevSensor& se, const Photon& p, float fw,
                                            int fx, int fy, float s3, const float* kdr = nullptr) {
     const float tau = le_tau<KD>(S, sm, se, p, fx, fy, s3);
@@ -872,6 +940,15 @@ __device__ __forceinline__ void le_deposit(const DevScene& S, const Smem& sm, co
         const double fac = kd_le_sum(S.kd_tab + size_t(p.job) * (S.nz + 2) * S.kd_n, S.kd_rf + size_t(p.job) * S.kd_n, kdr, S.kd_n,
                                      p.z - sm.z[p.iz], p.iz, se.zt - sm.z[se.lt], se.lt, se.inv_sz);
         rad_add<SMT>(S, sm, idx, double(contrib) * fac * se.npix);
+    } else if (JAC) {
+        const double c = double(contrib) * J.rad_fac * se.npix;
+        rad_add<SMT>(S, sm, idx, c);
+        if (p.flags & FL_ABS) {
+            const unsigned n = jac_deposit(S.jac + idx * S.jac_n, kdr, S.jac_n, S.job_abs + size_t(p.job) * S.nz,
+                                           S.job_cabs + size_t(p.job) * (S.nz + 1), S.jac_lev, S.jac_grp, p.z - sm.z[p.iz], p.iz,
+                                           se.zt - sm.z[se.lt], se.lt, se.inv_sz, c);
+            CNT_ADD(CNT_TALLY, n);
+        }
     } else rad_add<SMT>(S, sm, idx, double(contrib) * J.rad_fac * se.npix);
     CNT_ADD(CNT_LE, 1u);
 }
@@ -996,11 +1073,16 @@ __device__ __noinline__ float2 pick_component3(const float* __restrict__ ext3, c
 //     slab: the fine slab of a photon that left a box sideways follows from its height, and the layer search for unequal
 //     layers is not part of the flight loop at all (the other kernels keep both, decided at run time).  Measured on config 2: the ~35 never-executed instructions of that search cost 3.4 % (the loop is
 //     instruction-fetch sensitive, profiles/README.md r02_f), hence a template parameter instead of a run-time test.
-// KD (radiance kernels of b200rt_run_kd only): every history serves S.kd_n gas-absorption terms (kd_leg, kd_le_sum); with
-//     KD = false none of that code exists, so the other kernels are unchanged.
-template <bool PL, bool FZ, int NP, bool CAM, bool UZ, bool RAD, bool NO3, bool KD>
+// XM: what the radiance kernels carry besides the radiance (XM_NONE for every other kernel).
+//   XM_KD (b200rt_run_kd): every history serves S.kd_n gas-absorption terms (kd_leg, kd_le_sum).
+//   XM_JAC (b200rt_run_jac): every history also tallies the radiance's derivatives with respect to the gas absorption of
+//     S.jac_n layer groups (jac_leg, jac_deposit); radiance, draws and event counters are those of XM_NONE.
+//   With XM_NONE none of that code exists, so the other kernels are unchanged.
+enum { XM_NONE = 0, XM_KD = 1, XM_JAC = 2 };
+template <bool PL, bool FZ, int NP, bool CAM, bool UZ, bool RAD, bool NO3, int XM>
 __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid_constant__ DevScene S) {
     extern __shared__ float4 smem_f4[];
+    constexpr bool KD = XM == XM_KD, JAC = XM == XM_JAC;
     constexpr bool SMT = PL && UZ;      // block-private tallies exist only in the kernels of plane-parallel / few-column scenes
     Smem sm;
     float* pool;
@@ -1099,6 +1181,10 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
 #define KD_LEG(zb, izb, upd)                                                                                              \
     kd_leg<upd>(S.kd_tab + size_t(p.job) * (S.nz + 2) * S.kd_n, kd_state<NP>(S, slot), S.kd_n, p.za - sm.z[p.iza], p.iza,             \
                 (zb) - sm.z[(izb)], (izb), p.iza == (izb) ? p.leg : inv_absdz)
+// JAC: add the gas optical path of that leg, per layer group, to the state of pool slot `slot`
+#define JAC_LEG(zb, izb)                                                                                                  \
+    jac_leg(S.job_abs + size_t(p.job) * S.nz, S.job_cabs + size_t(p.job) * (S.nz + 1), S.jac_lev, S.jac_grp, jac_state<NP>(S, slot), \
+            p.za - sm.z[p.iza], p.iza, (zb) - sm.z[(izb)], (izb), p.iza == (izb) ? p.leg : inv_absdz)
 // push the slots of the lanes for which `cond` holds onto queue `q` (length `cnt`); `val` is the queue entry
 #define QPUSH(q, cnt, cond, val)                                              \
     {                                                                         \
@@ -1169,6 +1255,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                 if (want_flux) { flux_tally<SMT>(S, sm, p, 0, S.nz); flux_tally<SMT>(S, sm, p, 1, S.nz); }
                 pool_store<NP>(pool, slot, p, S.inv_Sx, S.inv_Sy);
                 if (KD) kd_init(kd_state<NP>(S, slot), S.kd_n);
+                if (JAC && (p.flags & FL_ABS)) jac_init(jac_state<NP>(S, slot), S.jac_n);
             }
             QPUSH(qF, nF, born, slot);
             if (exhausted) nD = ND_DONE;
@@ -1456,6 +1543,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                         float tr;
                         if (KD) tr = KD_LEG(p.z, izn, true);
                         else tr = __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, izn, p.leg, inv_absdz));
+                        if (JAC) JAC_LEG(p.z, izn);
                         const float wn = p.w * tr;
                         ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                         p.w = wn;
@@ -1549,6 +1637,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     float tr;
                     if (KD) tr = KD_LEG(p.z, 0, true);
                     else tr = __expf(-abs_tau(S, sm, p.job, p.za, p.iza, p.z, 0, p.leg, inv_absdz));
+                    if (JAC) JAC_LEG(p.z, 0);
                     const float wn = p.w * tr;
                     ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                     p.w = wn;
@@ -1603,7 +1692,9 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     } else {
                         f = se.s.z > 0.0f ? brdf_eval(sfc_type, prm[0], prm[1], prm[2], prm[3], prm[4], wi, se.s) * se.s.z : 0.0f;
                     }
-                    if (f > 0.0f) le_deposit<SMT, KD>(S, sm, se, p, f * p.w, fx, fy, s3, KD ? kd_state<NP>(S, slot) : nullptr);
+                    if (f > 0.0f)
+                        le_deposit<SMT, KD, JAC>(S, sm, se, p, f * p.w, fx, fy, s3,
+                                                 KD ? kd_state<NP>(S, slot) : (JAC ? jac_state<NP>(S, slot) : nullptr));
                 }
             }
 
@@ -1654,6 +1745,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
     }
 #undef RNG4
 #undef KD_LEG
+#undef JAC_LEG
 #undef QPUSH
 #undef QPUSH_DEAD
 
@@ -1720,35 +1812,40 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
 
 typedef void (*transport_fn)(const DevScene);
 template <int NP>
-static transport_fn pick_transport_np(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, bool kd) {
+static transport_fn pick_transport_np(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, int xm) {
     // CAM (all-sky camera sensors present) is its own specialisation: the camera's local estimate is a large cold path
     // whose register pressure must not tax the satellite-view kernels; it needs the 3-D solver (FZ = false).
     // UZ: see the kernel.  RAD = false exists for the per-level kernels only: a pure flux / heating run carries no
     // local-estimate code at all (those kernels are instruction-fetch bound).
-    // KD (b200rt_run_kd): radiance kernels with satellite sensors only; the caller has rejected every other case.
-    if (kd) {
-        if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, true> : transport_kernel<false, true, NP, false, false, true, false, true>;
-        return uz ? transport_kernel<false, false, NP, false, true, true, false, true> : transport_kernel<false, false, NP, false, false, true, false, true>;
+    // KD (b200rt_run_kd) and JAC (b200rt_run_jac): radiance kernels with satellite sensors only; the caller has rejected every other case.
+    if (xm == XM_KD) {
+        if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, XM_KD> : transport_kernel<false, true, NP, false, false, true, false, XM_KD>;
+        return uz ? transport_kernel<false, false, NP, false, true, true, false, XM_KD> : transport_kernel<false, false, NP, false, false, true, false, XM_KD>;
+    }
+    // JAC (b200rt_run_jac): the same kernels as KD, carrying the Jacobian tally instead of the terms
+    if (xm == XM_JAC) {
+        if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, XM_JAC> : transport_kernel<false, true, NP, false, false, true, false, XM_JAC>;
+        return uz ? transport_kernel<false, false, NP, false, true, true, false, XM_JAC> : transport_kernel<false, false, NP, false, false, true, false, XM_JAC>;
     }
     if (pl) {
-        if (cam) return transport_kernel<true, false, NP, true, false, true, false, false>;
+        if (cam) return transport_kernel<true, false, NP, true, false, true, false, XM_NONE>;
         if (rad) {
-            if (fz) return uz ? transport_kernel<true, true, NP, false, true, true, false, false> : transport_kernel<true, true, NP, false, false, true, false, false>;
-            return uz ? transport_kernel<true, false, NP, false, true, true, false, false> : transport_kernel<true, false, NP, false, false, true, false, false>;
+            if (fz) return uz ? transport_kernel<true, true, NP, false, true, true, false, XM_NONE> : transport_kernel<true, true, NP, false, false, true, false, XM_NONE>;
+            return uz ? transport_kernel<true, false, NP, false, true, true, false, XM_NONE> : transport_kernel<true, false, NP, false, false, true, false, XM_NONE>;
         }
-        if (fz) return uz ? transport_kernel<true, true, NP, false, true, false, false, false> : transport_kernel<true, true, NP, false, false, false, false, false>;
-        if (uz && no3) return transport_kernel<true, false, NP, false, true, false, true, false>;
-        return uz ? transport_kernel<true, false, NP, false, true, false, false, false> : transport_kernel<true, false, NP, false, false, false, false, false>;
+        if (fz) return uz ? transport_kernel<true, true, NP, false, true, false, false, XM_NONE> : transport_kernel<true, true, NP, false, false, false, false, XM_NONE>;
+        if (uz && no3) return transport_kernel<true, false, NP, false, true, false, true, XM_NONE>;
+        return uz ? transport_kernel<true, false, NP, false, true, false, false, XM_NONE> : transport_kernel<true, false, NP, false, false, false, false, XM_NONE>;
     }
-    if (cam) return uz ? transport_kernel<false, false, NP, true, true, true, false, false> : transport_kernel<false, false, NP, true, false, true, false, false>;
-    if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, false> : transport_kernel<false, true, NP, false, false, true, false, false>;
-    return uz ? transport_kernel<false, false, NP, false, true, true, false, false> : transport_kernel<false, false, NP, false, false, true, false, false>;
+    if (cam) return uz ? transport_kernel<false, false, NP, true, true, true, false, XM_NONE> : transport_kernel<false, false, NP, true, false, true, false, XM_NONE>;
+    if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, XM_NONE> : transport_kernel<false, true, NP, false, false, true, false, XM_NONE>;
+    return uz ? transport_kernel<false, false, NP, false, true, true, false, XM_NONE> : transport_kernel<false, false, NP, false, false, true, false, XM_NONE>;
 }
-static transport_fn pick_transport(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, bool kd, int np) {
+static transport_fn pick_transport(bool pl, bool fz, bool cam, bool uz, bool rad, bool no3, int xm, int np) {
     switch (np) {
-        case 64: return pick_transport_np<64>(pl, fz, cam, uz, rad, no3, kd);
-        case 128: return pick_transport_np<128>(pl, fz, cam, uz, rad, no3, kd);
-        default: return pick_transport_np<96>(pl, fz, cam, uz, rad, no3, kd);
+        case 64: return pick_transport_np<64>(pl, fz, cam, uz, rad, no3, xm);
+        case 128: return pick_transport_np<128>(pl, fz, cam, uz, rad, no3, xm);
+        default: return pick_transport_np<96>(pl, fz, cam, uz, rad, no3, xm);
     }
 }
 
@@ -1805,6 +1902,10 @@ struct Handle {
     DevBuf ext3tot, prop3, ext3, maj, tu3, pmu, pp, pcdf, pgs, pge, sfc_type, sfc_param;
     DevBuf jobs, job_abs, job_cabs, job_fscale, counter, stats, flag;
     DevBuf kd_tab, kd_rf, kd_r;   // spectral runs: per-term tables and the per-slot term state
+    DevBuf jac_lev, jac_grp, jac_t, jac;   // Jacobian runs: group edges, group of every layer, per-slot paths, tally
+    size_t njac = 0;
+    bool jac_valid = false;      // the last run (since the last upload) was a Jacobian run: `jac` holds its tally
+    std::vector<int> jac_edges;  // its group edges
     DevBuf flux, rad, heat;
     size_t nflux = 0, nrad = 0, nheat = 0;
     std::vector<float> h_zgrd;
@@ -1931,7 +2032,7 @@ int b200rt_destroy(void* handle) {
                      &H->st_e, &H->st_o, &H->st_a, &H->st_b, &H->f2c, &H->slab_cg, &H->group_lo, &H->group_cz, &H->group_maj1d, &H->gz_lo, &H->empty3, &H->runcode,
                      &H->ext3tot, &H->prop3, &H->ext3, &H->maj, &H->tu3, &H->pmu, &H->pp, &H->pcdf, &H->pgs, &H->pge, &H->sfc_type,
                      &H->sfc_param, &H->jobs, &H->job_abs, &H->job_cabs, &H->job_fscale, &H->counter, &H->stats, &H->flag,
-                     &H->kd_tab, &H->kd_rf, &H->kd_r, &H->flux, &H->rad, &H->heat};
+                     &H->kd_tab, &H->kd_rf, &H->kd_r, &H->jac_lev, &H->jac_grp, &H->jac_t, &H->jac, &H->flux, &H->rad, &H->heat};
     for (DevBuf* b : all) b->release();
     if (H->ev0) cudaEventDestroy(H->ev0);
     if (H->ev1) cudaEventDestroy(H->ev1);
@@ -2405,13 +2506,16 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     H->opt = *opt;
     H->have_scene = true;
     H->ran = false;
+    H->jac_valid = false;
     return B200RT_OK;
 }
 
 }  // extern "C"
 
-// b200rt_run (kd == nullptr) and b200rt_run_kd (kd[njob]: the gas-absorption terms of every job)
-static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream) {
+// b200rt_run (kd == nullptr, edges == nullptr), b200rt_run_kd (kd[njob]: the gas-absorption terms of every job) and
+// b200rt_run_jac (edges[ngrp+1]: the layer groups of the Jacobian tally)
+static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, const int32_t* edges, int ngrp, int njob, int accumulate,
+                    void* cuda_stream) {
     if (!H->have_scene) return fail(H, B200RT_ERR_STATE, "b200rt_run called before b200rt_upload_scene");
     if (!jobs || njob < 1) return fail(H, B200RT_ERR_ARG, "no jobs");
     if (njob > 65535) return fail(H, B200RT_ERR_ARG, "at most 65535 jobs per run");
@@ -2443,6 +2547,22 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
             kd_n = std::max(kd_n, k.nkd);
         }
     }
+    const int jac_n = edges ? ngrp : 0;
+    if (edges) {
+        if (H->k_pl)
+            return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: radiance targets only (no flux / heating; tiny radiance tallies held in shared memory "
+                                           "need options.smem_tally = -1)");
+        if (!k_rad) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: needs the radiance target and at least one sensor");
+        if (H->k_cam) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: the all-sky camera (Rad_mrkind = 1) is not supported");
+        if (kver == 9) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: not available with options.kernel = 9");
+        if (ngrp < 1 || ngrp > 64) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: ngrp must be 1 ... 64");
+        if (edges[0] != 0 || edges[ngrp] != nz)
+            return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: edges must start at layer 0 and end at nz (" + std::to_string(nz) + ")");
+        for (int j = 0; j < ngrp; ++j)
+            if (!(edges[j + 1] > edges[j])) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: edges must be strictly increasing");
+        if (accumulate && H->ran && !(H->jac_valid && H->jac_edges == std::vector<int>(edges, edges + ngrp + 1)))
+            return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: accumulate needs the previous run to be a Jacobian run with the same edges");
+    }
     CK(cudaSetDevice(H->device));
     CK(drain(H));                 // one run in flight per handle: the previous one still reads the job tables and counters
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
@@ -2450,10 +2570,11 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
     // asynchronously on the caller's stream
     auto al = [](size_t b) { return (b + 15) & ~size_t(15); };
     const size_t b_jobs = size_t(njob) * sizeof(DevJob), b_abs = size_t(njob) * nz * 4, b_cabs = size_t(njob) * (nz + 1) * 4,
-                 b_fs = size_t(njob) * (nz + 1) * 8, b_kt = size_t(njob) * (nz + 2) * kd_n * 8, b_kr = size_t(njob) * kd_n * 8;
+                 b_fs = size_t(njob) * (nz + 1) * 8, b_kt = size_t(njob) * (nz + 2) * kd_n * 8, b_kr = size_t(njob) * kd_n * 8,
+                 b_jl = edges ? size_t(jac_n + 1) * 4 : 0, b_jg = edges ? size_t(nz) : 0;
     const size_t o_jobs = 0, o_fs = al(b_jobs), o_abs = o_fs + al(b_fs), o_cabs = o_abs + al(b_abs), o_kt = o_cabs + al(b_cabs),
-                 o_kr = o_kt + al(b_kt);
-    const size_t need = o_kr + b_kr + 16;
+                 o_kr = o_kt + al(b_kt), o_jl = o_kr + al(b_kr), o_jg = o_jl + al(b_jl);
+    const size_t need = o_jg + b_jg + 16;
     if (need > H->pin_bytes) {
         if (H->pin) cudaFreeHost(H->pin);
         H->pin = nullptr; H->pin_bytes = 0;
@@ -2467,6 +2588,13 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
     float* jcabs = reinterpret_cast<float*>(pin + o_cabs);
     float2* kt = reinterpret_cast<float2*>(pin + o_kt);
     double* kr = reinterpret_cast<double*>(pin + o_kr);
+    int* jl = reinterpret_cast<int*>(pin + o_jl);
+    unsigned char* jg = reinterpret_cast<unsigned char*>(pin + o_jg);
+    for (int j = 0; j < jac_n; ++j) {
+        jl[j] = edges[j];
+        for (int i = edges[j]; i < edges[j + 1]; ++i) jg[i] = (unsigned char)j;
+    }
+    if (edges) jl[jac_n] = nz;
     std::memset(jabs, 0, b_abs);
     std::memset(jcabs, 0, b_cabs);
     std::memset(kt, 0, b_kt);                    // terms beyond a job's nkd: no absorption, weight 0, radiance factor 0
@@ -2536,6 +2664,15 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
         CK(cudaMemcpyAsync(H->kd_tab.p, kt, b_kt, cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(H->kd_rf.p, kr, b_kr, cudaMemcpyHostToDevice, st));
     }
+    if (edges) {
+        if ((rc = dev_alloc(H, H->jac_lev, b_jl)) || (rc = dev_alloc(H, H->jac_grp, b_jg)) || (rc = dev_alloc(H, H->jac, H->nrad * jac_n * 8)))
+            return rc;
+        CK(cudaMemcpyAsync(H->jac_lev.p, jl, b_jl, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(H->jac_grp.p, jg, b_jg, cudaMemcpyHostToDevice, st));
+        // zeroed unless this run adds to the previous Jacobian run (the radiance tally is zero after an upload anyway)
+        if (!accumulate || !H->ran) CK(cudaMemsetAsync(H->jac.p, 0, H->nrad * jac_n * 8, st));
+    }
+    S.jac_n = jac_n; S.jac_lev = (const int*)H->jac_lev.p; S.jac_grp = (const unsigned char*)H->jac_grp.p; S.jac = (double*)H->jac.p;
     S.kd_n = kd_n; S.kd_tab = (const float2*)H->kd_tab.p; S.kd_rf = (const double*)H->kd_rf.p;
     S.njob = njob; S.jobs = (const DevJob*)H->jobs.p; S.job_abs = (const float*)H->job_abs.p;
     S.job_cabs = (const float*)H->job_cabs.p; S.job_fscale = (const double*)H->job_fscale.p;
@@ -2583,7 +2720,7 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
     int bps = 0;
     // UZ kernels: equally thick 3-D layers with runs (S.uz_ok) -- or no 3-D block at all (the layer search is dead code then)
     const bool k_uz = H->k_pl ? (S.nz3 <= 0 || size_t(S.nx) * S.ny <= 64) : ((S.uz_ok != 0 && H->cmz == 1) || S.nz3 <= 0);
-    transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, kd != nullptr, np);
+    transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, kd ? XM_KD : (edges ? XM_JAC : XM_NONE), np);
     const size_t smem = H->smem_tables + 32 * (4 * 8 + 8 * 4) + size_t(tpb) * 8 + size_t(tpb / 32) * size_t(POOL_WORDS(np)) * 4 +
                         8 * size_t(S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem) * size_t(S.tal_per_warp ? RT_TPB / 32 : 1);
     if (smem > 227 * 1024) return fail(H, B200RT_ERR_ARG, "photon pools + 1-D tables exceed shared memory; lower threads_per_block or pool_slots");
@@ -2598,6 +2735,11 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
         if ((rc = dev_alloc(H, H->kd_r, size_t(grid) * (tpb / 32) * np * kd_n * 4))) return rc;
         S.kd_r = (float*)H->kd_r.p;
     }
+    if (edges) {
+        // per-group path of every pool slot of the launch: [block][warp][slot][jac_n]
+        if ((rc = dev_alloc(H, H->jac_t, size_t(grid) * (tpb / 32) * np * jac_n * 4))) return rc;
+        S.jac_t = (float*)H->jac_t.p;
+    }
     CK(cudaEventRecord(H->ev0, st));
     kern<<<grid, tpb, smem, st>>>(S);
     CK(cudaGetLastError());
@@ -2607,6 +2749,11 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, int 
     H->ran = true;
     H->inflight = true;
     H->launches = 1;
+    H->jac_valid = edges != nullptr;
+    if (edges) {
+        H->jac_edges.assign(edges, edges + jac_n + 1);
+        H->njac = H->nrad * jac_n;
+    }
     return B200RT_OK;
 }
 
@@ -2615,14 +2762,21 @@ extern "C" {
 int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
-    return run_jobs(H, jobs, nullptr, njob, accumulate, cuda_stream);
+    return run_jobs(H, jobs, nullptr, nullptr, 0, njob, accumulate, cuda_stream);
 }
 
 int b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
     if (!kd) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: kd is NULL");
-    return run_jobs(H, jobs, kd, njob, accumulate, cuda_stream);
+    return run_jobs(H, jobs, kd, nullptr, 0, njob, accumulate, cuda_stream);
+}
+
+int b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, const int32_t* edges, int ngrp, int accumulate, void* cuda_stream) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    if (!edges) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: edges is NULL");
+    return run_jobs(H, jobs, nullptr, edges, ngrp, njob, accumulate, cuda_stream);
 }
 
 int b200rt_sync(void* handle) {
@@ -2636,7 +2790,9 @@ int b200rt_sync(void* handle) {
     if (H->nflux) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->flux.p, H->nflux, (int*)H->flag.p);
     if (H->nrad) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->rad.p, H->nrad, (int*)H->flag.p);
     if (H->nheat) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->heat.p, H->nheat, (int*)H->flag.p);
-    H->launches = 1 + (H->nflux ? 1 : 0) + (H->nrad ? 1 : 0) + (H->nheat ? 1 : 0);
+    const bool jac = H->jac_valid && H->njac > 0;
+    if (jac) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->jac.p, H->njac, (int*)H->flag.p);
+    H->launches = 1 + (H->nflux ? 1 : 0) + (H->nrad ? 1 : 0) + (H->nheat ? 1 : 0) + (jac ? 1 : 0);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));
     H->inflight = false;
@@ -2684,6 +2840,22 @@ int b200rt_read_heat(void* handle, double* dst, int64_t count) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
     return read_any(H, H->heat, H->nheat, dst, count, "heating");
+}
+
+int b200rt_read_jac(void* handle, double* dst, int64_t count) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    if (!H->ran || !H->jac_valid) return fail(H, B200RT_ERR_STATE, "the last run was not a Jacobian run (b200rt_run_jac)");
+    return read_any(H, H->jac, H->njac, dst, count, "Jacobian");
+}
+
+int b200rt_jac_ptr(void* handle, double** p, int64_t* n) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    if (!H->ran || !H->jac_valid) return fail(H, B200RT_ERR_STATE, "the last run was not a Jacobian run (b200rt_run_jac)");
+    if (p) *p = (double*)H->jac.p;
+    if (n) *n = int64_t(H->njac);
+    return B200RT_OK;
 }
 
 int b200rt_tally_ptrs(void* handle, double** flux, int64_t* nflux, double** rad, int64_t* nrad, double** heat, int64_t* nheat) {

@@ -52,7 +52,7 @@ def allreduce_results(solver, to_host=True):
     """
     Sum the tallies of all ranks.  With NCCL the all-reduce runs IN PLACE on the library's own device buffers (no staging
     tensor, no device-to-device copy): afterwards every rank's handle holds the global tallies and `solver.results()` /
-    `b200rt_read_*` return them.  With gloo (CPU tests) the host arrays are reduced.  The run is waited for first
+    `b200rt_read_*` return them.  After a Jacobian run (`Solver.run_jac`) its tally is reduced too (`res['jac']`).  With gloo (CPU tests) the host arrays are reduced.  The run is waited for first
     (`solver.sync()`: NaN guard + fresh event counters), and the event counters are reduced with the same collective.
     """
     import torch
@@ -63,9 +63,14 @@ def allreduce_results(solver, to_host=True):
     if hasattr(solver, 'sync'):
         solver.sync()
     st = solver.stats()
+    has_jac = bool(getattr(solver, '_jac_ngrp', 0))
+    keys = ('flux', 'rad', 'heat') + (('jac',) if has_jac else ())
     if use_cuda:
         views = tally_views(solver)
-        for key in ('flux', 'rad', 'heat'):
+        if has_jac:
+            ptr, n = solver.jac_ptr()
+            views['jac'] = torch.as_tensor(_DeviceDoubles(ptr, n), device='cuda:%d' % solver.device)
+        for key in keys:
             t = views[key]
             if t is None:
                 continue
@@ -74,11 +79,11 @@ def allreduce_results(solver, to_host=True):
         if to_host:
             torch.cuda.synchronize()
             host = solver.results()
-            for key in ('flux', 'rad', 'heat'):
+            for key in keys:
                 res[key] = host[key]
     else:
         host = solver.results()
-        for key in ('flux', 'rad', 'heat'):
+        for key in keys:
             a = host[key]
             if a is None:
                 continue

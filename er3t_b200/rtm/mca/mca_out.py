@@ -185,7 +185,9 @@ def read_flux_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
 
 
 def read_radiance_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
-    """Radiance (W/m^2/nm/sr): rad (+ rad_std), toa, N_photon, N_run (mca_out.py:412-505)."""
+    """Radiance (W/m^2/nm/sr): rad (+ rad_std), toa, N_photon, N_run (mca_out.py:412-505).  When the simulation carried a
+    gas-absorption Jacobian (mcarats_ng(gas_jacobian=...)) also rad_jac (+ rad_jac_std): dI / dln(a_j) per layer group j
+    in place of the Nz axis, and jac_levels (km): the group edges."""
     mode = mode.lower()
     rad, = _per_run_arrays(mca_obj, abs_obj, 'radiance')
     _, toa = cal_factors(mca_obj.date, abs_obj, 1, mca_obj.Ng)
@@ -200,6 +202,19 @@ def read_radiance_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
         raise OSError('Error [read_radiance_mca_out]: Do not support <mode=%s>.' % mode)
     d['N_photon'] = {'data': mca_obj.photons, 'name': 'Number of photons', 'units': 'N/A'}
     d['N_run'] = {'data': mca_obj.Nrun, 'name': 'Number of runs', 'units': 'N/A'}
+    fused = getattr(mca_obj, 'fused', None)
+    if fused is not None and fused.get('jacobian') is not None:
+        # (weighted with the simulation's own absorption object, which _per_run_arrays has just checked against abs_obj)
+        jac, jdims = _finish(np.asarray(fused['jacobian'][0], dtype=np.float32), squeeze)
+        jdims = ['Ngroup' if k == 'Nz' else k for k in jdims]
+        if mode == 'all':
+            d['rad_jac'] = {'data': jac, 'name': 'Radiance Jacobian dI/dln(gas absorption) per layer group', 'units': 'W/m^2/nm/sr', 'dims_info': jdims}
+        else:
+            d['rad_jac'] = {'data': np.mean(jac, axis=-1), 'name': 'Radiance Jacobian dI/dln(gas absorption) per layer group (mean)',
+                            'units': 'W/m^2/nm/sr', 'dims_info': jdims[:-1]}
+            d['rad_jac_std'] = {'data': np.std(jac, axis=-1), 'name': 'Radiance Jacobian dI/dln(gas absorption) per layer group (standard deviation)',
+                                'units': 'W/m^2/nm/sr', 'dims_info': jdims[:-1]}
+        d['jac_levels'] = {'data': np.asarray(mca_obj.jac_levels, dtype=np.float64), 'name': 'Level heights bounding the layer groups', 'units': 'km'}
     return d
 
 
@@ -231,6 +246,7 @@ class mca_out_ng:
     squeeze=  : drop axes of length 1
 
     self.data['f_up'|'f_down'|'f_down_direct'|'f_down_diffuse'|...'_std'|'rad'|'rad_std'|'toa'|'N_photon'|'N_run']
+    (+ 'rad_jac', 'rad_jac_std', 'jac_levels' when the simulation carried a gas-absorption Jacobian)
     Same loading rules as the reference (mca_out.py:160-177).
     """
 

@@ -12,7 +12,8 @@ What is new (keyword-only, all optional): `seed` (reproducible Philox streams; d
 mcarats.py:432), `device`, `raw` (keep per-job fields instead of g-weighted per-run sums), `write_files` (emit the
 namelist text and MCARaTS-style .bin/.ctl outputs), `iz3l_fix`, `supervoxel`, `shard` / `reduce` (multi-GPU),
 `extra_sensors`, `solver_obj` (reuse a handle), `camera_pixels` (all-sky camera grid instead of the reference's fixed
-500 x 500), `spectral` (MCARaTS's multi-term mode, Atm_nkd = Ng: one history serves every g of the wavelength).
+500 x 500), `spectral` (MCARaTS's multi-term mode, Atm_nkd = Ng: one history serves every g of the wavelength),
+`gas_jacobian` (the radiance's derivatives with respect to the gas absorption of layer groups, from the same histories).
 """
 
 import datetime
@@ -80,11 +81,20 @@ class mcarats_ng:
                  wmin=None,
                  camera_pixels=None,
                  dry_run=False,
-                 spectral=False):
+                 spectral=False,
+                 gas_jacobian=None):
         """spectral=True: one job per run traces `photons` histories (not photons per g), each of which carries all Ng
         terms of the correlated-k set (Atm_nkd = Ng, Atm_wkd0 = weights; Iwabuchi and Okamura 2017).  `self.fused` has the
         same layout and meaning as without it.  Needs target='radiance' with the satellite sensor and an `abs` object;
-        `raw`, `write_files`, flux / heating targets and the all-sky camera raise OSError."""
+        `raw`, `write_files`, flux / heating targets and the all-sky camera raise OSError.
+
+        gas_jacobian: also estimate dI / dln(a_j) in the same histories, where a_j multiplies the gas absorption (Atm_abs1d)
+        of every layer of group j, for every g.  True: one group per layer; a sequence of level heights (km), which must be
+        levels of the atmosphere including its bottom and top: contiguous groups between them.  Results:
+        `self.fused['jacobian']` (nx, ny, ngrp, 1, Nrun), `self.jac_extra` for the extra sensors (like `rad_extra`),
+        `self.jac_levels` (km) and `self.jac_edges` (layer indices).  Atm_abst3d and particle absorption are not
+        differentiated.  Needs target='radiance' with the satellite sensor and an `abs` object; `spectral`, `raw`,
+        `write_files`, flux / heating targets and the all-sky camera raise OSError."""
 
         add_reference(self.reference)
 
@@ -127,6 +137,10 @@ class mcarats_ng:
         self.camera_pixels = camera_pixels
         self.dry_run = dry_run
         self.spectral = spectral
+        self.gas_jacobian = gas_jacobian
+        self.jac_edges = None
+        self.jac_levels = None
+        self.jac_extra = None
         self.atm_1ds = atm_1ds
         self.atm_3ds = atm_3ds
 
@@ -419,6 +433,20 @@ class mcarats_ng:
                 raise OSError('Error [mcarats_ng]: <spectral=True> supports the satellite sensor only (not the all-sky camera).')
             if self.abs is None:
                 raise OSError('Error [mcarats_ng]: <spectral=True> needs the gas absorption object of <atm_1ds> (its g weights and solar factors).')
+        jac = self.gas_jacobian is not None and self.gas_jacobian is not False
+        if jac:
+            if self.spectral:
+                raise OSError('Error [mcarats_ng]: <gas_jacobian> is not available with <spectral=True>.')
+            if self.keep_raw:
+                raise OSError('Error [mcarats_ng]: <gas_jacobian> is tallied per run: <raw> and <write_files> are not available.')
+            if self.target != 'radiance':
+                raise OSError('Error [mcarats_ng]: <gas_jacobian> supports target=\'radiance\' only (flux and heating rates are not available).')
+            if 'satellite' not in self.sensor_type.lower():
+                raise OSError('Error [mcarats_ng]: <gas_jacobian> supports the satellite sensor only (not the all-sky camera).')
+            if self.abs is None:
+                raise OSError('Error [mcarats_ng]: <gas_jacobian> needs the gas absorption object of <atm_1ds>.')
+            self.jac_edges = jacobian_edges(self.gas_jacobian, scene.zgrd)
+            self.jac_levels = scene.zgrd[self.jac_edges] / 1000.0
         fuse = (not self.keep_raw) and (self.abs is not None)
         self.fuse = fuse
         if fuse:
@@ -464,7 +492,7 @@ class mcarats_ng:
         # per-level ones, which have no spectral variant)
         opt = abi.make_options(solver=solvers[self.solver], target=tflag, nslab=nslab, shard_rank=self.shard[0], shard_world=self.shard[1],
                                sv=self.supervoxel, iso_ss=DEFAULTS['Pho_iso_SS'], iso_max=DEFAULTS['Pho_iso_max'], wmin=wmin, wfac=DEFAULTS['Pho_wfac'],
-                               smem_tally=-1 if self.spectral else 0)
+                               smem_tally=-1 if (self.spectral or jac) else 0)
         jobs_args = dict(nphot=nphot, seeds=seeds, slabs=slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc)
         self.kd_args = kd
         self.options, self.jobs_args, self.nslab = opt, jobs_args, nslab
@@ -475,7 +503,8 @@ class mcarats_ng:
             return
         # the reference hands the job list to `mca_run` (mcarats.py:468); so does this class -- one launch instead of a pool
         runner = mca_run(scene, opt, nphot, seeds, slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc, device=self.device,
-                         solver_obj=self._solver_obj, Ncpu=self.Ncpu, mp_mode=self.mp_mode, quiet=True, run=False, kd=kd)
+                         solver_obj=self._solver_obj, Ncpu=self.Ncpu, mp_mode=self.mp_mode, quiet=True, run=False, kd=kd,
+                         jac_edges=self.jac_edges)
         try:
             self.h2d_bytes = scene.nbytes() + sum(a.nbytes for a in runner._keep)
             runner.launch()
@@ -514,6 +543,18 @@ class mcarats_ng:
             self.fused = {'flux': None if flux is None else [flux[0], flux[1], flux[2]],
                           'radiance': None if rad is None else [rad],
                           'heating': None if heat is None else [heat]}
+            if res.get('jac') is not None:
+                # [nslab][sum_k nyr_k * nxr_k][ngrp] -> (nxr, nyr, ngrp, 1, nslab) per sensor
+                jr = np.asarray(res['jac']).reshape(nslab, scene.rad_size(1), -1)
+                ng = jr.shape[-1]
+                off, views = 0, []
+                for k in range(scene.struct.nrad):
+                    sk = scene.sensors[k]
+                    nk = sk.nxr * sk.nyr
+                    views.append(np.transpose(jr[:, off:off + nk].reshape(nslab, sk.nyr, sk.nxr, ng), (2, 1, 3, 0)))
+                    off += nk
+                self.fused['jacobian'] = [views[0][:, :, :, np.newaxis, :]]
+                self.jac_extra = views[1:]
         else:
             self.raw = []
             for ir in range(Nrun):
@@ -565,6 +606,32 @@ class mcarats_ng:
         print('Message [mcarats_ng]: run summary')
         for k, v in rows:
             print('    %s : %s' % (k.rjust(width), v))
+
+
+def jacobian_edges(gas_jacobian, zgrd_m):
+    """Layer-group edges (layer indices, 0 ... nz) of `mcarats_ng(gas_jacobian=...)`: True gives one group per layer; a
+    sequence of level heights in km, which must be levels of the atmosphere (`zgrd_m`, metres) and include its bottom and
+    top, gives the contiguous groups between them."""
+    zgrd_m = np.asarray(zgrd_m, dtype=np.float64)
+    nz = zgrd_m.size - 1
+    if gas_jacobian is True:
+        edges = np.arange(nz + 1)
+    else:
+        try:
+            lev = np.asarray(gas_jacobian, dtype=np.float64).ravel() * 1000.0
+        except (TypeError, ValueError):
+            raise OSError('Error [mcarats_ng]: <gas_jacobian> must be True or a sequence of level heights in km.')
+        if lev.size < 2 or np.any(np.diff(lev) <= 0.0):
+            raise OSError('Error [mcarats_ng]: <gas_jacobian> levels must be at least two strictly increasing heights in km.')
+        idx = np.abs(lev[:, None] - zgrd_m[None, :]).argmin(axis=1)
+        if np.any(np.abs(zgrd_m[idx] - lev) > 1e-6 * np.maximum(1.0, np.abs(lev))):
+            raise OSError('Error [mcarats_ng]: <gas_jacobian> levels must be levels of the atmosphere (Atm_zgrd0).')
+        if idx[0] != 0 or idx[-1] != nz:
+            raise OSError('Error [mcarats_ng]: <gas_jacobian> levels must include the bottom and the top of the atmosphere.')
+        edges = idx
+    if edges.size - 1 > 64:
+        raise OSError('Error [mcarats_ng]: <gas_jacobian> supports at most 64 layer groups (%d asked for).' % (edges.size - 1))
+    return edges.astype(np.int32)
 
 
 def cal_mca_azimuth(normal_azimuth_angle):

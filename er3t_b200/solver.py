@@ -28,6 +28,7 @@ class Solver:
         self.scene = None
         self.options = None
         self._keep = None
+        self._jac_ngrp = 0       # layer groups of the last run when it was a Jacobian run, else 0
 
     # ------------------------------------------------------------------ helpers
     def _check(self, rc, where):
@@ -57,6 +58,7 @@ class Solver:
     def run(self, jobs, accumulate=False, stream=None, sync=True):
         """jobs: ctypes array of abi.Job (see abi.make_jobs)."""
         self._keep = jobs
+        self._jac_ngrp = 0
         self._check(self.lib.b200rt_run(self.handle, jobs, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run')
         if sync:
             self.sync()
@@ -65,7 +67,21 @@ class Solver:
         """Spectral run: jobs (abi.make_jobs, without abs1d / flx_scale) and kd (abi.make_kd, one record per job): every
         history serves all k-distribution terms of its job."""
         self._keep = (jobs, kd)
+        self._jac_ngrp = 0
         self._check(self.lib.b200rt_run_kd(self.handle, jobs, kd, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run_kd')
+        if sync:
+            self.sync()
+
+    def run_jac(self, jobs, edges, accumulate=False, stream=None, sync=True):
+        """b200rt_run that also tallies dI / dln(a_j) for the gas absorption of the layer groups [edges[j], edges[j+1]) (layer
+        indices, 0 = edges[0] < ... < edges[-1] = nz, at most 64 groups): same histories, same radiance."""
+        e = np.ascontiguousarray(edges, dtype=np.int32)
+        if e.ndim != 1 or e.size < 2:
+            raise ValueError('Error [er3t_b200]: <edges> must be a 1-D sequence of at least two layer indices.')
+        self._keep = (jobs, e)
+        self._check(self.lib.b200rt_run_jac(self.handle, jobs, len(jobs), e.ctypes.data, e.size - 1, 1 if accumulate else 0, stream),
+                    'b200rt_run_jac')
+        self._jac_ngrp = e.size - 1
         if sync:
             self.sync()
 
@@ -99,6 +115,25 @@ class Solver:
         self._check(self.lib.b200rt_read_rad(self.handle, out.ctypes.data, out.size), 'b200rt_read_rad')
         return out
 
+    def read_jac(self, out=None):
+        """Jacobian tally of the last run (run_jac): (nslab, sum_k nyr_k * nxr_k, ngrp), group fastest."""
+        if not self._jac_ngrp:
+            raise OSError('Error [er3t_b200]: read_jac: the last run was not a Jacobian run (run_jac).')
+        n = self.scene.rad_size(self.options.nslab)
+        if out is None:
+            out = np.empty(n * self._jac_ngrp, dtype=np.float64)
+        self._check(self.lib.b200rt_read_jac(self.handle, out.ctypes.data, out.size), 'b200rt_read_jac')
+        return out.reshape(self.options.nslab, -1, self._jac_ngrp)
+
+    def jac_ptr(self):
+        """(device pointer, doubles) of the Jacobian tally of the last run (b200rt_jac_ptr), or (None, 0) when it was not a
+        Jacobian run."""
+        if not self._jac_ngrp:
+            return None, 0
+        p, n = C.c_void_p(), C.c_int64()
+        self._check(self.lib.b200rt_jac_ptr(self.handle, C.byref(p), C.byref(n)), 'b200rt_jac_ptr')
+        return p.value, n.value
+
     def read_heat(self, out=None):
         shape = self.scene.heat_shape(self.options.nslab)
         if out is None:
@@ -116,6 +151,8 @@ class Solver:
             res['rad'] = self.read_rad()
         if t & abi.TARGET_HEATING:
             res['heat'] = self.read_heat()
+        if self._jac_ngrp:
+            res['jac'] = self.read_jac()
         res['stats'] = self.stats()
         return res
 

@@ -12,6 +12,8 @@
  *                                       per-job seed of mcarats.py:432-437)
  *   b200rt_run_kd                    <- MCARaTS's multi-term mode (Atm_nkd > 1, Atm_wkd0; Iwabuchi and Okamura 2017):
  *                                       one job per run serves all Ng terms of a wavelength
+ *   b200rt_run_jac                   <- finite differences of whole runs with the gas absorption of a layer group
+ *                                       scaled (no counterpart in MCARaTS: Rad_mplen stays 0, as er3t sets it)
  *   b200rt_read_flux / _rad / _heat  <- `.bin` + `.ctl` parsing, er3t/rtm/mca/mca_out.py:48-103
  *                                       (and, through job.flx_scale / job.rad_scale, the g-weighting of
  *                                        mca_out.py:319-327,354-366,444-452,475-481)
@@ -225,6 +227,19 @@ int          b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accu
  * jobs[j].rad_scale is a factor common to all terms.  Same asynchronous contract as b200rt_run. */
 int          b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream);
 
+/* b200rt_run that also tallies the radiance's derivatives with respect to the gas absorption of ngrp layer groups:
+ * jac = dI / dln(a_j), where a_j multiplies jobs[].abs1d of layers edges[j] ... edges[j+1]-1 (host array of ngrp+1 layer
+ * indices, 0 = edges[0] < ... < edges[ngrp] = nz, 1 <= ngrp <= 64).  Estimated inside the same histories, without bias:
+ * every local estimate with contribution c (as tallied into the radiance) adds -c (T_j + tau_j) to pixel and group j, where
+ * T_j is the gas optical path the history has collected in group j and tau_j that of the segment toward the sensor.  The
+ * radiance, draws and event counters are those of b200rt_run (stats.n_tally also counts the Jacobian updates).  Atm_abst3d
+ * and particle absorption are not differentiated.  Radiance target with satellite sensors only (flux / heating targets,
+ * options.smem_tally >= 0 on scenes whose radiance tally fits shared memory, the all-sky camera and options.kernel = 9
+ * are rejected).  With accumulate != 0 the previous run since the last upload, if any, must be a Jacobian run with the
+ * same edges.  Same asynchronous contract as b200rt_run. */
+int          b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, const int32_t* edges, int ngrp, int accumulate,
+                            void* cuda_stream);
+
 /* Wait for the stream of the last run; checks tallies for NaN/Inf. */
 int          b200rt_sync(void* handle);
 
@@ -234,6 +249,10 @@ int          b200rt_sync(void* handle);
 int          b200rt_read_flux(void* handle, double* dst, int64_t count);
 int          b200rt_read_rad (void* handle, double* dst, int64_t count);
 int          b200rt_read_heat(void* handle, double* dst, int64_t count);
+/* Jacobian tally of the last run, which must have been a b200rt_run_jac: [nslab][nrad][nyr][nxr][ngrp] (group fastest),
+ * count = doubles the caller provides.  b200rt_jac_ptr: its device pointer and size (in-place NCCL all-reduce). */
+int          b200rt_read_jac(void* handle, double* dst, int64_t count);
+int          b200rt_jac_ptr(void* handle, double** p, int64_t* n);
 /* Device pointers to the library-owned tallies (for in-place NCCL all-reduce by the caller). */
 int          b200rt_tally_ptrs(void* handle, double** flux, int64_t* nflux, double** rad, int64_t* nrad,
                                double** heat, int64_t* nheat);

@@ -161,8 +161,13 @@ struct DevScene {
     int jac_n;
     const int* jac_lev;       // [jac_n+1] group edges as layer indices, 0 = jac_lev[0] < ... < jac_lev[jac_n] = nz
     const unsigned char* jac_grp;   // [nz] group of every layer
-    float* jac_t;             // [block][warp][pool slot][jac_n] gas optical path of the slot's history per group (see jac_leg)
-    double* jac;              // [nslab][rad_slab][jac_n] tally of dI / dln(a_j)
+    // per-slot state and per-pixel tally of the JAC and PLEN kernels
+    float* xs;                // JAC: [block][warp][pool slot][jac_n] gas optical path of the slot's history per group (see jac_leg)
+                              // PLEN: [block][warp][pool slot] geometric path of the slot's history so far (m)
+    double* xt;               // JAC: [nslab][rad_slab][jac_n] tally of dI / dln(a_j); PLEN: [nslab][rad_slab][pl_ntp+3] (plen_deposit)
+    // path-length distributions (b200rt_run_plen, read by the PLEN kernels only): pl_ntp bins on [pl_lo, pl_hi) metres
+    int pl_ntp;
+    float pl_lo, pl_hi, pl_inv_w;   // pl_inv_w = pl_ntp / (pl_hi - pl_lo)
 };
 
 // ============================================================================ setup kernels
@@ -707,7 +712,7 @@ __device__ __forceinline__ float* kd_state(const DevScene& S, int slot) {
 // on a_j only through the gas optical paths, and d c / d ln(a_j) = -c (T_j + tau_LE_j): T_j the gas optical path the
 // history has collected inside group j since it started, tau_LE_j that of the event -> sensor segment.  The score is the
 // photon weight times a function of the history, so Russian roulette (which keeps the expected weight given the past)
-// leaves it unbiased.  The slot carries T_j in global scratch (DevScene::jac_t), updated where a leg ends at a collision
+// leaves it unbiased.  The slot carries T_j in global scratch (DevScene::xs), updated where a leg ends at a collision
 // or the surface; an escape leg needs nothing (no local estimate follows it).
 // jac_leg splits the gas optical path of the leg from (dza above the bottom of layer iza) to (dzb above the bottom of izb)
 // over the groups it crosses, exactly as abs_tau_at computes the leg's whole path: inside one layer abs * f (f = length),
@@ -760,7 +765,25 @@ __device__ __noinline__ void jac_init(float* __restrict__ t, int ngrp) {
 // the per-group state of pool slot `slot` of the calling warp (ordered like kd_state)
 template <int NP>
 __device__ __forceinline__ float* jac_state(const DevScene& S, int slot) {
-    return S.jac_t + ((size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot)) * S.jac_n;
+    return S.xs + ((size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot)) * S.jac_n;
+}
+
+// ---- radiance path-length distributions: the geometric path L (m) behind every local-estimate contribution c -------------
+// L runs from the photon's entry at TOA along every leg of its history to the event, then along the event -> sensor segment
+// to the sensor's target level.  L is geometry only (it never changes a trajectory) and the score is the photon weight times
+// a function of the history, so Russian roulette leaves it unbiased, as for the Jacobian.  The slot carries the path of its
+// finished legs in global scratch (DevScene::xs), updated where a leg ends at a collision or the surface; an escape leg needs
+// nothing.  plen_deposit adds c to the bin of L (index ntp: L < lo, ntp + 1: L >= hi) and c L to the first moment (ntp + 2)
+// of one radiance pixel's row out[0 .. ntp+3); the bin index is computed in fp32 from the fp32 path.
+__device__ __forceinline__ void plen_deposit(double* __restrict__ out, int ntp, float lo, float hi, float inv_w, float L, double c) {
+    const int b = L < lo ? ntp : (L >= hi ? ntp + 1 : min(ntp - 1, int((L - lo) * inv_w)));
+    tally_add(out + b, c);
+    tally_add(out + ntp + 2, c * double(L));
+}
+// the path of pool slot `slot` of the calling warp (ordered like kd_state)
+template <int NP>
+__device__ __forceinline__ float* plen_state(const DevScene& S, int slot) {
+    return S.xs + (size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot);
 }
 
 // Exact optical depth toward a sensor for oblique views and sensors inside the atmosphere.
@@ -919,7 +942,8 @@ __device__ __forceinline__ float le_tau(const DevScene& S, const Smem& sm, const
 // deposit one local-estimate contribution (fw = weight x angular density toward the sensor, 1/sr)
 // KD: kdr = the photon's per-term state; the radiance factor is the sum over the terms (kd_le_sum) instead of the job's
 // JAC: kdr = the photon's per-group gas optical paths; the same contribution also goes to the Jacobian tally (jac_deposit)
-template <bool SMT, bool KD = false, bool JAC = false>
+// PLEN: kdr = the photon's path so far; the same contribution also goes to the path-length tally (plen_deposit)
+template <bool SMT, bool KD = false, bool JAC = false, bool PLEN = false>
 __device__ __forceinline__ void le_deposit(const DevScene& S, const Smem& sm, const DevSensor& se, const Photon& p, float fw,
                                            int fx, int fy, float s3, const float* kdr = nullptr) {
     const float tau = le_tau<KD>(S, sm, se, p, fx, fy, s3);
@@ -944,11 +968,16 @@ __device__ __forceinline__ void le_deposit(const DevScene& S, const Smem& sm, co
         const double c = double(contrib) * J.rad_fac * se.npix;
         rad_add<SMT>(S, sm, idx, c);
         if (p.flags & FL_ABS) {
-            const unsigned n = jac_deposit(S.jac + idx * S.jac_n, kdr, S.jac_n, S.job_abs + size_t(p.job) * S.nz,
+            const unsigned n = jac_deposit(S.xt + idx * S.jac_n, kdr, S.jac_n, S.job_abs + size_t(p.job) * S.nz,
                                            S.job_cabs + size_t(p.job) * (S.nz + 1), S.jac_lev, S.jac_grp, p.z - sm.z[p.iz], p.iz,
                                            se.zt - sm.z[se.lt], se.lt, se.inv_sz, c);
             CNT_ADD(CNT_TALLY, n);
         }
+    } else if (PLEN) {
+        const double c = double(contrib) * J.rad_fac * se.npix;
+        rad_add<SMT>(S, sm, idx, c);
+        plen_deposit(S.xt + idx * (S.pl_ntp + 3), S.pl_ntp, S.pl_lo, S.pl_hi, S.pl_inv_w, *kdr + (se.zt - p.z) * se.inv_szs, c);
+        CNT_ADD(CNT_TALLY, 2u);
     } else rad_add<SMT>(S, sm, idx, double(contrib) * J.rad_fac * se.npix);
     CNT_ADD(CNT_LE, 1u);
 }
@@ -1077,12 +1106,14 @@ __device__ __noinline__ float2 pick_component3(const float* __restrict__ ext3, c
 //   XM_KD (b200rt_run_kd): every history serves S.kd_n gas-absorption terms (kd_leg, kd_le_sum).
 //   XM_JAC (b200rt_run_jac): every history also tallies the radiance's derivatives with respect to the gas absorption of
 //     S.jac_n layer groups (jac_leg, jac_deposit); radiance, draws and event counters are those of XM_NONE.
+//   XM_PLEN (b200rt_run_plen): every history also tallies the distribution of the geometric path lengths behind each
+//     pixel's radiance (plen_state, plen_deposit); radiance, draws and event counters are those of XM_NONE.
 //   With XM_NONE none of that code exists, so the other kernels are unchanged.
-enum { XM_NONE = 0, XM_KD = 1, XM_JAC = 2 };
+enum { XM_NONE = 0, XM_KD = 1, XM_JAC = 2, XM_PLEN = 3 };
 template <bool PL, bool FZ, int NP, bool CAM, bool UZ, bool RAD, bool NO3, int XM>
 __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid_constant__ DevScene S) {
     extern __shared__ float4 smem_f4[];
-    constexpr bool KD = XM == XM_KD, JAC = XM == XM_JAC;
+    constexpr bool KD = XM == XM_KD, JAC = XM == XM_JAC, PLEN = XM == XM_PLEN;
     constexpr bool SMT = PL && UZ;      // block-private tallies exist only in the kernels of plane-parallel / few-column scenes
     Smem sm;
     float* pool;
@@ -1256,6 +1287,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                 pool_store<NP>(pool, slot, p, S.inv_Sx, S.inv_Sy);
                 if (KD) kd_init(kd_state<NP>(S, slot), S.kd_n);
                 if (JAC && (p.flags & FL_ABS)) jac_init(jac_state<NP>(S, slot), S.jac_n);
+                if (PLEN) *plen_state<NP>(S, slot) = 0.0f;
             }
             QPUSH(qF, nF, born, slot);
             if (exhausted) nD = ND_DONE;
@@ -1548,6 +1580,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                         ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                         p.w = wn;
                     }
+                    if (PLEN) *plen_state<NP>(S, slot) += p.leg;     // with or without gas absorption
                     float omg = 1.0f, apf = 0.0f;
                     bool found = false;
                     if (uc < s3) {
@@ -1642,6 +1675,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     ACC_ADD(ACC_ATM, double(p.w) - double(wn));
                     p.w = wn;
                 }
+                if (PLEN) *plen_state<NP>(S, slot) += p.leg;
                 CNT_ADD(CNT_SFC, 1u);
                 RNG4(u);
                 const bool frozen = FZ && (p.flags & FL_FROZEN);
@@ -1693,8 +1727,9 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                         f = se.s.z > 0.0f ? brdf_eval(sfc_type, prm[0], prm[1], prm[2], prm[3], prm[4], wi, se.s) * se.s.z : 0.0f;
                     }
                     if (f > 0.0f)
-                        le_deposit<SMT, KD, JAC>(S, sm, se, p, f * p.w, fx, fy, s3,
-                                                 KD ? kd_state<NP>(S, slot) : (JAC ? jac_state<NP>(S, slot) : nullptr));
+                        le_deposit<SMT, KD, JAC, PLEN>(S, sm, se, p, f * p.w, fx, fy, s3,
+                                                       KD ? kd_state<NP>(S, slot)
+                                                          : (JAC ? jac_state<NP>(S, slot) : (PLEN ? plen_state<NP>(S, slot) : nullptr)));
                 }
             }
 
@@ -1827,6 +1862,11 @@ static transport_fn pick_transport_np(bool pl, bool fz, bool cam, bool uz, bool 
         if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, XM_JAC> : transport_kernel<false, true, NP, false, false, true, false, XM_JAC>;
         return uz ? transport_kernel<false, false, NP, false, true, true, false, XM_JAC> : transport_kernel<false, false, NP, false, false, true, false, XM_JAC>;
     }
+    // PLEN (b200rt_run_plen): the same kernels, carrying the path-length tally
+    if (xm == XM_PLEN) {
+        if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, XM_PLEN> : transport_kernel<false, true, NP, false, false, true, false, XM_PLEN>;
+        return uz ? transport_kernel<false, false, NP, false, true, true, false, XM_PLEN> : transport_kernel<false, false, NP, false, false, true, false, XM_PLEN>;
+    }
     if (pl) {
         if (cam) return transport_kernel<true, false, NP, true, false, true, false, XM_NONE>;
         if (rad) {
@@ -1902,10 +1942,12 @@ struct Handle {
     DevBuf ext3tot, prop3, ext3, maj, tu3, pmu, pp, pcdf, pgs, pge, sfc_type, sfc_param;
     DevBuf jobs, job_abs, job_cabs, job_fscale, counter, stats, flag;
     DevBuf kd_tab, kd_rf, kd_r;   // spectral runs: per-term tables and the per-slot term state
-    DevBuf jac_lev, jac_grp, jac_t, jac;   // Jacobian runs: group edges, group of every layer, per-slot paths, tally
-    size_t njac = 0;
-    bool jac_valid = false;      // the last run (since the last upload) was a Jacobian run: `jac` holds its tally
-    std::vector<int> jac_edges;  // its group edges
+    DevBuf jac_lev, jac_grp;     // Jacobian runs: group edges, group of every layer
+    DevBuf xs, xt;               // Jacobian and path-length runs: per-slot state, per-pixel tally (DevScene::xs, xt)
+    size_t nxt = 0;
+    int xt_mode = 0;             // XM_JAC / XM_PLEN: the last run (since the last upload) was such a run and `xt` holds its
+                                 // tally; XM_NONE otherwise
+    std::vector<double> xt_key;  // its parameters (group edges, or tpmin, tpmax, ntp): what `accumulate` must match
     DevBuf flux, rad, heat;
     size_t nflux = 0, nrad = 0, nheat = 0;
     std::vector<float> h_zgrd;
@@ -2032,7 +2074,7 @@ int b200rt_destroy(void* handle) {
                      &H->st_e, &H->st_o, &H->st_a, &H->st_b, &H->f2c, &H->slab_cg, &H->group_lo, &H->group_cz, &H->group_maj1d, &H->gz_lo, &H->empty3, &H->runcode,
                      &H->ext3tot, &H->prop3, &H->ext3, &H->maj, &H->tu3, &H->pmu, &H->pp, &H->pcdf, &H->pgs, &H->pge, &H->sfc_type,
                      &H->sfc_param, &H->jobs, &H->job_abs, &H->job_cabs, &H->job_fscale, &H->counter, &H->stats, &H->flag,
-                     &H->kd_tab, &H->kd_rf, &H->kd_r, &H->jac_lev, &H->jac_grp, &H->jac_t, &H->jac, &H->flux, &H->rad, &H->heat};
+                     &H->kd_tab, &H->kd_rf, &H->kd_r, &H->jac_lev, &H->jac_grp, &H->xs, &H->xt, &H->flux, &H->rad, &H->heat};
     for (DevBuf* b : all) b->release();
     if (H->ev0) cudaEventDestroy(H->ev0);
     if (H->ev1) cudaEventDestroy(H->ev1);
@@ -2506,15 +2548,24 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     H->opt = *opt;
     H->have_scene = true;
     H->ran = false;
-    H->jac_valid = false;
+    H->xt_mode = XM_NONE;
     return B200RT_OK;
 }
 
 }  // extern "C"
 
-// b200rt_run (kd == nullptr, edges == nullptr), b200rt_run_kd (kd[njob]: the gas-absorption terms of every job) and
-// b200rt_run_jac (edges[ngrp+1]: the layer groups of the Jacobian tally)
-static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, const int32_t* edges, int ngrp, int njob, int accumulate,
+// what a Jacobian or path-length run adds to b200rt_run: the kernels' mode and its parameters
+struct XtArgs {
+    int mode = XM_NONE;                        // XM_NONE, XM_JAC or XM_PLEN
+    const int32_t* edges = nullptr;            // XM_JAC: edges[ngrp+1], the layer groups of the Jacobian tally
+    int ngrp = 0;
+    double tpmin = 0.0, tpmax = 0.0;           // XM_PLEN: ntp bins on [tpmin, tpmax) metres
+    int ntp = 0;
+};
+
+// b200rt_run (kd == nullptr, xa.mode = XM_NONE), b200rt_run_kd (kd[njob]: the gas-absorption terms of every job),
+// b200rt_run_jac and b200rt_run_plen (xa)
+static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, const XtArgs& xa, int njob, int accumulate,
                     void* cuda_stream) {
     if (!H->have_scene) return fail(H, B200RT_ERR_STATE, "b200rt_run called before b200rt_upload_scene");
     if (!jobs || njob < 1) return fail(H, B200RT_ERR_ARG, "no jobs");
@@ -2547,21 +2598,40 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
             kd_n = std::max(kd_n, k.nkd);
         }
     }
-    const int jac_n = edges ? ngrp : 0;
-    if (edges) {
+    const bool plen = xa.mode == XM_PLEN;
+    const int32_t* edges = xa.mode == XM_JAC ? xa.edges : nullptr;
+    const int jac_n = edges ? xa.ngrp : 0;
+    size_t xt_n = 0;              // doubles per radiance pixel of the extra tally (DevScene::xt)
+    std::vector<double> xt_key;
+    if (xa.mode != XM_NONE) {
+        const std::string who = edges ? "b200rt_run_jac: " : "b200rt_run_plen: ";
         if (H->k_pl)
-            return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: radiance targets only (no flux / heating; tiny radiance tallies held in shared memory "
-                                           "need options.smem_tally = -1)");
-        if (!k_rad) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: needs the radiance target and at least one sensor");
-        if (H->k_cam) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: the all-sky camera (Rad_mrkind = 1) is not supported");
-        if (kver == 9) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: not available with options.kernel = 9");
-        if (ngrp < 1 || ngrp > 64) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: ngrp must be 1 ... 64");
-        if (edges[0] != 0 || edges[ngrp] != nz)
-            return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: edges must start at layer 0 and end at nz (" + std::to_string(nz) + ")");
-        for (int j = 0; j < ngrp; ++j)
-            if (!(edges[j + 1] > edges[j])) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: edges must be strictly increasing");
-        if (accumulate && H->ran && !(H->jac_valid && H->jac_edges == std::vector<int>(edges, edges + ngrp + 1)))
-            return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: accumulate needs the previous run to be a Jacobian run with the same edges");
+            return fail(H, B200RT_ERR_ARG, who + "radiance targets only (no flux / heating; tiny radiance tallies held in shared memory "
+                                                 "need options.smem_tally = -1)");
+        if (!k_rad) return fail(H, B200RT_ERR_ARG, who + "needs the radiance target and at least one sensor");
+        if (H->k_cam) return fail(H, B200RT_ERR_ARG, who + "the all-sky camera (Rad_mrkind = 1) is not supported");
+        if (kver == 9) return fail(H, B200RT_ERR_ARG, who + "not available with options.kernel = 9");
+        if (edges) {
+            const int ngrp = xa.ngrp;
+            if (ngrp < 1 || ngrp > 64) return fail(H, B200RT_ERR_ARG, who + "ngrp must be 1 ... 64");
+            if (edges[0] != 0 || edges[ngrp] != nz)
+                return fail(H, B200RT_ERR_ARG, who + "edges must start at layer 0 and end at nz (" + std::to_string(nz) + ")");
+            for (int j = 0; j < ngrp; ++j)
+                if (!(edges[j + 1] > edges[j])) return fail(H, B200RT_ERR_ARG, who + "edges must be strictly increasing");
+            xt_n = size_t(ngrp);
+            xt_key.assign(edges, edges + ngrp + 1);
+        } else {
+            if (xa.ntp < 1 || xa.ntp > 1024) return fail(H, B200RT_ERR_ARG, who + "ntp must be 1 ... 1024");
+            // (the kernels bin in fp32: the edges must stay finite and distinct there too)
+            if (!std::isfinite(float(xa.tpmin)) || !std::isfinite(float(xa.tpmax)) || !(xa.tpmin >= 0.0) ||
+                !(float(xa.tpmax) > float(xa.tpmin)))
+                return fail(H, B200RT_ERR_ARG, who + "tpmin and tpmax must be finite with 0 <= tpmin < tpmax");
+            xt_n = size_t(xa.ntp) + 3;
+            xt_key = {xa.tpmin, xa.tpmax, double(xa.ntp)};
+        }
+        if (accumulate && H->ran && !(H->xt_mode == xa.mode && H->xt_key == xt_key))
+            return fail(H, B200RT_ERR_ARG, who + (edges ? "accumulate needs the previous run to be a Jacobian run with the same edges"
+                                                        : "accumulate needs the previous run to be a path-length run with the same binning"));
     }
     CK(cudaSetDevice(H->device));
     CK(drain(H));                 // one run in flight per handle: the previous one still reads the job tables and counters
@@ -2665,14 +2735,21 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
         CK(cudaMemcpyAsync(H->kd_rf.p, kr, b_kr, cudaMemcpyHostToDevice, st));
     }
     if (edges) {
-        if ((rc = dev_alloc(H, H->jac_lev, b_jl)) || (rc = dev_alloc(H, H->jac_grp, b_jg)) || (rc = dev_alloc(H, H->jac, H->nrad * jac_n * 8)))
-            return rc;
+        if ((rc = dev_alloc(H, H->jac_lev, b_jl)) || (rc = dev_alloc(H, H->jac_grp, b_jg))) return rc;
         CK(cudaMemcpyAsync(H->jac_lev.p, jl, b_jl, cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(H->jac_grp.p, jg, b_jg, cudaMemcpyHostToDevice, st));
-        // zeroed unless this run adds to the previous Jacobian run (the radiance tally is zero after an upload anyway)
-        if (!accumulate || !H->ran) CK(cudaMemsetAsync(H->jac.p, 0, H->nrad * jac_n * 8, st));
     }
-    S.jac_n = jac_n; S.jac_lev = (const int*)H->jac_lev.p; S.jac_grp = (const unsigned char*)H->jac_grp.p; S.jac = (double*)H->jac.p;
+    if (xt_n) {
+        // `xt` is resized / zeroed from here on: until this run has launched it holds no valid tally (a failure below must
+        // not leave b200rt_read_jac / _plen reading the previous run's size out of this buffer)
+        H->xt_mode = XM_NONE;
+        if ((rc = dev_alloc(H, H->xt, H->nrad * xt_n * 8))) return rc;
+        // zeroed unless this run adds to the previous run of the same kind (the radiance tally is zero after an upload anyway)
+        if (!accumulate || !H->ran) CK(cudaMemsetAsync(H->xt.p, 0, H->nrad * xt_n * 8, st));
+    }
+    S.jac_n = jac_n; S.jac_lev = (const int*)H->jac_lev.p; S.jac_grp = (const unsigned char*)H->jac_grp.p; S.xt = (double*)H->xt.p;
+    S.pl_ntp = plen ? xa.ntp : 0; S.pl_lo = float(xa.tpmin); S.pl_hi = float(xa.tpmax);
+    S.pl_inv_w = plen ? float(double(xa.ntp) / (double(S.pl_hi) - double(S.pl_lo))) : 0.0f;
     S.kd_n = kd_n; S.kd_tab = (const float2*)H->kd_tab.p; S.kd_rf = (const double*)H->kd_rf.p;
     S.njob = njob; S.jobs = (const DevJob*)H->jobs.p; S.job_abs = (const float*)H->job_abs.p;
     S.job_cabs = (const float*)H->job_cabs.p; S.job_fscale = (const double*)H->job_fscale.p;
@@ -2720,7 +2797,7 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     int bps = 0;
     // UZ kernels: equally thick 3-D layers with runs (S.uz_ok) -- or no 3-D block at all (the layer search is dead code then)
     const bool k_uz = H->k_pl ? (S.nz3 <= 0 || size_t(S.nx) * S.ny <= 64) : ((S.uz_ok != 0 && H->cmz == 1) || S.nz3 <= 0);
-    transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, kd ? XM_KD : (edges ? XM_JAC : XM_NONE), np);
+    transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, kd ? XM_KD : xa.mode, np);
     const size_t smem = H->smem_tables + 32 * (4 * 8 + 8 * 4) + size_t(tpb) * 8 + size_t(tpb / 32) * size_t(POOL_WORDS(np)) * 4 +
                         8 * size_t(S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem) * size_t(S.tal_per_warp ? RT_TPB / 32 : 1);
     if (smem > 227 * 1024) return fail(H, B200RT_ERR_ARG, "photon pools + 1-D tables exceed shared memory; lower threads_per_block or pool_slots");
@@ -2735,10 +2812,10 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
         if ((rc = dev_alloc(H, H->kd_r, size_t(grid) * (tpb / 32) * np * kd_n * 4))) return rc;
         S.kd_r = (float*)H->kd_r.p;
     }
-    if (edges) {
-        // per-group path of every pool slot of the launch: [block][warp][slot][jac_n]
-        if ((rc = dev_alloc(H, H->jac_t, size_t(grid) * (tpb / 32) * np * jac_n * 4))) return rc;
-        S.jac_t = (float*)H->jac_t.p;
+    if (xt_n) {
+        // per-slot state of every pool slot of the launch: [block][warp][slot][jac_n] per-group paths, or [block][warp][slot] path
+        if ((rc = dev_alloc(H, H->xs, size_t(grid) * (tpb / 32) * np * (edges ? jac_n : 1) * 4))) return rc;
+        S.xs = (float*)H->xs.p;
     }
     CK(cudaEventRecord(H->ev0, st));
     kern<<<grid, tpb, smem, st>>>(S);
@@ -2749,10 +2826,10 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     H->ran = true;
     H->inflight = true;
     H->launches = 1;
-    H->jac_valid = edges != nullptr;
-    if (edges) {
-        H->jac_edges.assign(edges, edges + jac_n + 1);
-        H->njac = H->nrad * jac_n;
+    H->xt_mode = xa.mode;
+    if (xt_n) {
+        H->xt_key = xt_key;
+        H->nxt = H->nrad * xt_n;
     }
     return B200RT_OK;
 }
@@ -2762,21 +2839,32 @@ extern "C" {
 int b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
-    return run_jobs(H, jobs, nullptr, nullptr, 0, njob, accumulate, cuda_stream);
+    return run_jobs(H, jobs, nullptr, XtArgs(), njob, accumulate, cuda_stream);
 }
 
 int b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
     if (!kd) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: kd is NULL");
-    return run_jobs(H, jobs, kd, nullptr, 0, njob, accumulate, cuda_stream);
+    return run_jobs(H, jobs, kd, XtArgs(), njob, accumulate, cuda_stream);
 }
 
 int b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, const int32_t* edges, int ngrp, int accumulate, void* cuda_stream) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
     if (!edges) return fail(H, B200RT_ERR_ARG, "b200rt_run_jac: edges is NULL");
-    return run_jobs(H, jobs, nullptr, edges, ngrp, njob, accumulate, cuda_stream);
+    XtArgs xa;
+    xa.mode = XM_JAC; xa.edges = edges; xa.ngrp = ngrp;
+    return run_jobs(H, jobs, nullptr, xa, njob, accumulate, cuda_stream);
+}
+
+int b200rt_run_plen(void* handle, const b200rt_job* jobs, int njob, double tpmin, double tpmax, int ntp, int accumulate,
+                    void* cuda_stream) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    XtArgs xa;
+    xa.mode = XM_PLEN; xa.tpmin = tpmin; xa.tpmax = tpmax; xa.ntp = ntp;
+    return run_jobs(H, jobs, nullptr, xa, njob, accumulate, cuda_stream);
 }
 
 int b200rt_sync(void* handle) {
@@ -2790,9 +2878,9 @@ int b200rt_sync(void* handle) {
     if (H->nflux) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->flux.p, H->nflux, (int*)H->flag.p);
     if (H->nrad) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->rad.p, H->nrad, (int*)H->flag.p);
     if (H->nheat) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->heat.p, H->nheat, (int*)H->flag.p);
-    const bool jac = H->jac_valid && H->njac > 0;
-    if (jac) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->jac.p, H->njac, (int*)H->flag.p);
-    H->launches = 1 + (H->nflux ? 1 : 0) + (H->nrad ? 1 : 0) + (H->nheat ? 1 : 0) + (jac ? 1 : 0);
+    const bool xt = H->xt_mode != XM_NONE && H->nxt > 0;
+    if (xt) check_finite_kernel<<<nb, 256, 0, st>>>((const double*)H->xt.p, H->nxt, (int*)H->flag.p);
+    H->launches = 1 + (H->nflux ? 1 : 0) + (H->nrad ? 1 : 0) + (H->nheat ? 1 : 0) + (xt ? 1 : 0);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));
     H->inflight = false;
@@ -2842,21 +2930,32 @@ int b200rt_read_heat(void* handle, double* dst, int64_t count) {
     return read_any(H, H->heat, H->nheat, dst, count, "heating");
 }
 
-int b200rt_read_jac(void* handle, double* dst, int64_t count) {
-    Handle* H = static_cast<Handle*>(handle);
-    if (!H) return B200RT_ERR_ARG;
-    if (!H->ran || !H->jac_valid) return fail(H, B200RT_ERR_STATE, "the last run was not a Jacobian run (b200rt_run_jac)");
-    return read_any(H, H->jac, H->njac, dst, count, "Jacobian");
-}
-
-int b200rt_jac_ptr(void* handle, double** p, int64_t* n) {
-    Handle* H = static_cast<Handle*>(handle);
-    if (!H) return B200RT_ERR_ARG;
-    if (!H->ran || !H->jac_valid) return fail(H, B200RT_ERR_STATE, "the last run was not a Jacobian run (b200rt_run_jac)");
-    if (p) *p = (double*)H->jac.p;
-    if (n) *n = int64_t(H->njac);
+// the per-pixel tally of the last run, which must have been a run of kind `mode` (XM_JAC or XM_PLEN)
+static int check_xt(Handle* H, int mode) {
+    if (!H->ran || H->xt_mode != mode)
+        return fail(H, B200RT_ERR_STATE, mode == XM_JAC ? "the last run was not a Jacobian run (b200rt_run_jac)"
+                                                        : "the last run was not a path-length run (b200rt_run_plen)");
     return B200RT_OK;
 }
+static int read_xt(void* handle, int mode, double* dst, int64_t count) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    if (int rc = check_xt(H, mode)) return rc;
+    return read_any(H, H->xt, H->nxt, dst, count, mode == XM_JAC ? "Jacobian" : "path-length tally");
+}
+static int xt_ptr(void* handle, int mode, double** p, int64_t* n) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    if (int rc = check_xt(H, mode)) return rc;
+    if (p) *p = (double*)H->xt.p;
+    if (n) *n = int64_t(H->nxt);
+    return B200RT_OK;
+}
+
+int b200rt_read_jac(void* handle, double* dst, int64_t count) { return read_xt(handle, XM_JAC, dst, count); }
+int b200rt_jac_ptr(void* handle, double** p, int64_t* n) { return xt_ptr(handle, XM_JAC, p, n); }
+int b200rt_read_plen(void* handle, double* dst, int64_t count) { return read_xt(handle, XM_PLEN, dst, count); }
+int b200rt_plen_ptr(void* handle, double** p, int64_t* n) { return xt_ptr(handle, XM_PLEN, p, n); }
 
 int b200rt_tally_ptrs(void* handle, double** flux, int64_t* nflux, double** rad, int64_t* nrad, double** heat, int64_t* nheat) {
     Handle* H = static_cast<Handle*>(handle);

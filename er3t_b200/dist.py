@@ -52,7 +52,8 @@ def allreduce_results(solver, to_host=True):
     """
     Sum the tallies of all ranks.  With NCCL the all-reduce runs IN PLACE on the library's own device buffers (no staging
     tensor, no device-to-device copy): afterwards every rank's handle holds the global tallies and `solver.results()` /
-    `b200rt_read_*` return them.  After a Jacobian run (`Solver.run_jac`) its tally is reduced too (`res['jac']`).  With gloo (CPU tests) the host arrays are reduced.  The run is waited for first
+    `b200rt_read_*` return them.  After a Jacobian run (`Solver.run_jac`) or a path-length run (`Solver.run_plen`) its tally
+    is reduced too (`res['jac']` / `res['plen']`).  With gloo (CPU tests) the host arrays are reduced.  The run is waited for first
     (`solver.sync()`: NaN guard + fresh event counters), and the event counters are reduced with the same collective.
     """
     import torch
@@ -63,13 +64,13 @@ def allreduce_results(solver, to_host=True):
     if hasattr(solver, 'sync'):
         solver.sync()
     st = solver.stats()
-    has_jac = bool(getattr(solver, '_jac_ngrp', 0))
-    keys = ('flux', 'rad', 'heat') + (('jac',) if has_jac else ())
+    xt = getattr(solver, '_xt_key', None)       # 'jac' / 'plen': the per-pixel tally of a Jacobian / path-length run
+    keys = ('flux', 'rad', 'heat') + ((xt,) if xt else ())
     if use_cuda:
         views = tally_views(solver)
-        if has_jac:
-            ptr, n = solver.jac_ptr()
-            views['jac'] = torch.as_tensor(_DeviceDoubles(ptr, n), device='cuda:%d' % solver.device)
+        if xt:
+            ptr, n = getattr(solver, xt + '_ptr')()
+            views[xt] = torch.as_tensor(_DeviceDoubles(ptr, n), device='cuda:%d' % solver.device)
         for key in keys:
             t = views[key]
             if t is None:

@@ -147,13 +147,15 @@ def _per_run_arrays(mca_obj, abs_obj, kind):
     return out
 
 
-def _finish(arr, squeeze):
-    """(Nx, Ny, Nz, Nt, Nrun) -> squeezed array + dims_info, like mca_out.py:333-338."""
+def _finish(arr, squeeze, keep_z=False):
+    """(Nx, Ny, Nz, Nt, Nrun) -> squeezed array + dims_info, like mca_out.py:333-338.  keep_z: never drop the third axis
+    (the bins of a path-length tally keep their axis even when there is one bin)."""
     dims_info = ['Nx', 'Ny', 'Nz', 'Nt']
     dims = list(arr.shape[:4])
     if squeeze:
-        dims_info = [dims_info[i] for i in range(4) if dims[i] > 1]
-        dims = [d for d in dims if d > 1]
+        keep = [dims[i] > 1 or (keep_z and i == 2) for i in range(4)]
+        dims_info = [dims_info[i] for i in range(4) if keep[i]]
+        dims = [dims[i] for i in range(4) if keep[i]]
     return arr.reshape(dims + [arr.shape[-1]]), dims_info + ['Nr']
 
 
@@ -187,7 +189,10 @@ def read_flux_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
 def read_radiance_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
     """Radiance (W/m^2/nm/sr): rad (+ rad_std), toa, N_photon, N_run (mca_out.py:412-505).  When the simulation carried a
     gas-absorption Jacobian (mcarats_ng(gas_jacobian=...)) also rad_jac (+ rad_jac_std): dI / dln(a_j) per layer group j
-    in place of the Nz axis, and jac_levels (km): the group edges."""
+    in place of the Nz axis, and jac_levels (km): the group edges.  When it carried a path-length tally
+    (mcarats_ng(path_length=...)) also rad_plen (+ rad_plen_std): the radiance per path-length bin in place of the Nz
+    axis, rad_plen_out: the radiance of the paths below and above the bins, rad_mean_plen (km): the mean path, the sum
+    over runs of the first moment over that of the radiance (NaN where the radiance is 0), and plen_edges (km)."""
     mode = mode.lower()
     rad, = _per_run_arrays(mca_obj, abs_obj, 'radiance')
     _, toa = cal_factors(mca_obj.date, abs_obj, 1, mca_obj.Ng)
@@ -215,6 +220,28 @@ def read_radiance_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
             d['rad_jac_std'] = {'data': np.std(jac, axis=-1), 'name': 'Radiance Jacobian dI/dln(gas absorption) per layer group (standard deviation)',
                                 'units': 'W/m^2/nm/sr', 'dims_info': jdims[:-1]}
         d['jac_levels'] = {'data': np.asarray(mca_obj.jac_levels, dtype=np.float64), 'name': 'Level heights bounding the layer groups', 'units': 'km'}
+    if fused is not None and fused.get('path_length') is not None:
+        pl = np.asarray(fused['path_length'][0], dtype=np.float64)          # (nx, ny, ntp+3, 1, Nrun)
+        ntp = pl.shape[2] - 3
+        for key, arr, dim, name in (('rad_plen', pl[:, :, :ntp], 'Nbin', 'Radiance per path-length bin'),
+                                    ('rad_plen_out', pl[:, :, ntp:ntp + 2], 'Nout', 'Radiance of paths below / above the bins')):
+            a, adims = _finish(arr.astype(np.float32), squeeze, keep_z=True)
+            adims = [dim if k == 'Nz' else k for k in adims]
+            if mode == 'all':
+                d[key] = {'data': a, 'name': name, 'units': 'W/m^2/nm/sr', 'dims_info': adims}
+            else:
+                d[key] = {'data': np.mean(a, axis=-1), 'name': name + ' (mean)', 'units': 'W/m^2/nm/sr', 'dims_info': adims[:-1]}
+                if key == 'rad_plen':
+                    d[key + '_std'] = {'data': np.std(a, axis=-1), 'name': name + ' (standard deviation)', 'units': 'W/m^2/nm/sr',
+                                       'dims_info': adims[:-1]}
+        # ratio of sums over runs, in fp64
+        num = pl[:, :, ntp + 2].sum(axis=-1)
+        den = np.asarray(fused['radiance'][0], dtype=np.float64)[:, :, 0].sum(axis=-1)
+        with np.errstate(divide='ignore', invalid='ignore'):
+            mean = np.where(den != 0.0, num / np.where(den != 0.0, den, 1.0) / 1000.0, np.nan)
+        m, mdims = _finish(mean[:, :, np.newaxis, :, np.newaxis], squeeze)
+        d['rad_mean_plen'] = {'data': m[..., 0], 'name': 'Mean photon path length', 'units': 'km', 'dims_info': mdims[:-1]}
+        d['plen_edges'] = {'data': np.asarray(mca_obj.plen_edges, dtype=np.float64), 'name': 'Edges of the path-length bins', 'units': 'km'}
     return d
 
 
@@ -247,6 +274,7 @@ class mca_out_ng:
 
     self.data['f_up'|'f_down'|'f_down_direct'|'f_down_diffuse'|...'_std'|'rad'|'rad_std'|'toa'|'N_photon'|'N_run']
     (+ 'rad_jac', 'rad_jac_std', 'jac_levels' when the simulation carried a gas-absorption Jacobian)
+    (+ 'rad_plen', 'rad_plen_std', 'rad_plen_out', 'rad_mean_plen', 'plen_edges' when it carried a path-length tally)
     Same loading rules as the reference (mca_out.py:160-177).
     """
 

@@ -13,7 +13,8 @@ mcarats.py:432), `device`, `raw` (keep per-job fields instead of g-weighted per-
 namelist text and MCARaTS-style .bin/.ctl outputs), `iz3l_fix`, `supervoxel`, `shard` / `reduce` (multi-GPU),
 `extra_sensors`, `solver_obj` (reuse a handle), `camera_pixels` (all-sky camera grid instead of the reference's fixed
 500 x 500), `spectral` (MCARaTS's multi-term mode, Atm_nkd = Ng: one history serves every g of the wavelength),
-`gas_jacobian` (the radiance's derivatives with respect to the gas absorption of layer groups, from the same histories).
+`gas_jacobian` (the radiance's derivatives with respect to the gas absorption of layer groups, from the same histories),
+`path_length` (per-pixel histograms and mean of the photon path lengths behind the radiance, from the same histories).
 """
 
 import datetime
@@ -82,7 +83,8 @@ class mcarats_ng:
                  camera_pixels=None,
                  dry_run=False,
                  spectral=False,
-                 gas_jacobian=None):
+                 gas_jacobian=None,
+                 path_length=None):
         """spectral=True: one job per run traces `photons` histories (not photons per g), each of which carries all Ng
         terms of the correlated-k set (Atm_nkd = Ng, Atm_wkd0 = weights; Iwabuchi and Okamura 2017).  `self.fused` has the
         same layout and meaning as without it.  Needs target='radiance' with the satellite sensor and an `abs` object;
@@ -94,7 +96,14 @@ class mcarats_ng:
         `self.fused['jacobian']` (nx, ny, ngrp, 1, Nrun), `self.jac_extra` for the extra sensors (like `rad_extra`),
         `self.jac_levels` (km) and `self.jac_edges` (layer indices).  Atm_abst3d and particle absorption are not
         differentiated.  Needs target='radiance' with the satellite sensor and an `abs` object; `spectral`, `raw`,
-        `write_files`, flux / heating targets and the all-sky camera raise OSError."""
+        `write_files`, flux / heating targets and the all-sky camera raise OSError.
+
+        path_length=(tpmin_km, tpmax_km, ntp): also tally, in the same histories, how long the photon paths behind each
+        pixel's radiance were (MCARaTS's Rad_mplen / Rad_ntp / Rad_tpmin / Rad_tpmax, which this sets in `self.nml`).  The
+        path of one local-estimate contribution runs from TOA along the whole history to the event and on to the sensor
+        level.  Results: `self.fused['path_length']` (nx, ny, ntp+3, 1, Nrun): ntp uniform bins on [tpmin, tpmax), underflow,
+        overflow and the first moment sum(c L) in metres (include/b200rt.h); `self.plen_extra` for the extra sensors and
+        `self.plen_edges` (km).  Same rules as `gas_jacobian`, with which it cannot be combined."""
 
         add_reference(self.reference)
 
@@ -141,6 +150,10 @@ class mcarats_ng:
         self.jac_edges = None
         self.jac_levels = None
         self.jac_extra = None
+        self.path_length = path_length
+        self.plen = None if path_length is None else path_length_bins(path_length)     # (tpmin, tpmax, ntp), metres
+        self.plen_edges = None if self.plen is None else np.linspace(self.plen[0], self.plen[1], self.plen[2] + 1) / 1000.0
+        self.plen_extra = None
         self.atm_1ds = atm_1ds
         self.atm_3ds = atm_3ds
 
@@ -241,6 +254,9 @@ class mcarats_ng:
                     n['Rad_xpos'] = sensor_xpos
                     n['Rad_ypos'] = sensor_ypos
                 n['Rad_mplen'] = 0
+                if self.plen is not None:
+                    n['Rad_mplen'] = 1
+                    n['Rad_tpmin'], n['Rad_tpmax'], n['Rad_ntp'] = self.plen
                 n['Rad_mpmap'] = 1
                 n['Rad_nrad'] = 1
                 n['Rad_difr0'] = 7.5
@@ -447,6 +463,19 @@ class mcarats_ng:
                 raise OSError('Error [mcarats_ng]: <gas_jacobian> needs the gas absorption object of <atm_1ds>.')
             self.jac_edges = jacobian_edges(self.gas_jacobian, scene.zgrd)
             self.jac_levels = scene.zgrd[self.jac_edges] / 1000.0
+        if self.plen is not None:
+            if jac:
+                raise OSError('Error [mcarats_ng]: <path_length> cannot be combined with <gas_jacobian> (one extra tally per run).')
+            if self.spectral:
+                raise OSError('Error [mcarats_ng]: <path_length> is not available with <spectral=True>.')
+            if self.keep_raw:
+                raise OSError('Error [mcarats_ng]: <path_length> is tallied per run: <raw> and <write_files> are not available.')
+            if self.target != 'radiance':
+                raise OSError('Error [mcarats_ng]: <path_length> supports target=\'radiance\' only (flux and heating rates are not available).')
+            if 'satellite' not in self.sensor_type.lower():
+                raise OSError('Error [mcarats_ng]: <path_length> supports the satellite sensor only (not the all-sky camera).')
+            if self.abs is None:
+                raise OSError('Error [mcarats_ng]: <path_length> needs the gas absorption object of <atm_1ds>.')
         fuse = (not self.keep_raw) and (self.abs is not None)
         self.fuse = fuse
         if fuse:
@@ -492,7 +521,7 @@ class mcarats_ng:
         # per-level ones, which have no spectral variant)
         opt = abi.make_options(solver=solvers[self.solver], target=tflag, nslab=nslab, shard_rank=self.shard[0], shard_world=self.shard[1],
                                sv=self.supervoxel, iso_ss=DEFAULTS['Pho_iso_SS'], iso_max=DEFAULTS['Pho_iso_max'], wmin=wmin, wfac=DEFAULTS['Pho_wfac'],
-                               smem_tally=-1 if (self.spectral or jac) else 0)
+                               smem_tally=-1 if (self.spectral or jac or self.plen is not None) else 0)
         jobs_args = dict(nphot=nphot, seeds=seeds, slabs=slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc)
         self.kd_args = kd
         self.options, self.jobs_args, self.nslab = opt, jobs_args, nslab
@@ -504,7 +533,7 @@ class mcarats_ng:
         # the reference hands the job list to `mca_run` (mcarats.py:468); so does this class -- one launch instead of a pool
         runner = mca_run(scene, opt, nphot, seeds, slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc, device=self.device,
                          solver_obj=self._solver_obj, Ncpu=self.Ncpu, mp_mode=self.mp_mode, quiet=True, run=False, kd=kd,
-                         jac_edges=self.jac_edges)
+                         jac_edges=self.jac_edges, plen=self.plen)
         try:
             self.h2d_bytes = scene.nbytes() + sum(a.nbytes for a in runner._keep)
             runner.launch()
@@ -543,9 +572,11 @@ class mcarats_ng:
             self.fused = {'flux': None if flux is None else [flux[0], flux[1], flux[2]],
                           'radiance': None if rad is None else [rad],
                           'heating': None if heat is None else [heat]}
-            if res.get('jac') is not None:
-                # [nslab][sum_k nyr_k * nxr_k][ngrp] -> (nxr, nyr, ngrp, 1, nslab) per sensor
-                jr = np.asarray(res['jac']).reshape(nslab, scene.rad_size(1), -1)
+            for key, name, extra in (('jac', 'jacobian', 'jac_extra'), ('plen', 'path_length', 'plen_extra')):
+                if res.get(key) is None:
+                    continue
+                # [nslab][sum_k nyr_k * nxr_k][ngrp or ntp+3] -> (nxr, nyr, ngrp or ntp+3, 1, nslab) per sensor
+                jr = np.asarray(res[key]).reshape(nslab, scene.rad_size(1), -1)
                 ng = jr.shape[-1]
                 off, views = 0, []
                 for k in range(scene.struct.nrad):
@@ -553,8 +584,8 @@ class mcarats_ng:
                     nk = sk.nxr * sk.nyr
                     views.append(np.transpose(jr[:, off:off + nk].reshape(nslab, sk.nyr, sk.nxr, ng), (2, 1, 3, 0)))
                     off += nk
-                self.fused['jacobian'] = [views[0][:, :, :, np.newaxis, :]]
-                self.jac_extra = views[1:]
+                self.fused[name] = [views[0][:, :, :, np.newaxis, :]]
+                setattr(self, extra, views[1:])
         else:
             self.raw = []
             for ir in range(Nrun):
@@ -632,6 +663,22 @@ def jacobian_edges(gas_jacobian, zgrd_m):
     if edges.size - 1 > 64:
         raise OSError('Error [mcarats_ng]: <gas_jacobian> supports at most 64 layer groups (%d asked for).' % (edges.size - 1))
     return edges.astype(np.int32)
+
+
+def path_length_bins(path_length):
+    """(tpmin, tpmax, ntp), tpmin and tpmax in metres, of `mcarats_ng(path_length=(tpmin_km, tpmax_km, ntp))`:
+    1 <= ntp <= 1024, 0 <= tpmin < tpmax, finite."""
+    try:
+        lo, hi, n = path_length
+        lo, hi = float(lo) * 1000.0, float(hi) * 1000.0
+        ntp = int(n)
+    except (TypeError, ValueError):
+        raise OSError('Error [mcarats_ng]: <path_length> must be (tpmin_km, tpmax_km, ntp).')
+    if ntp != n or not 1 <= ntp <= 1024:
+        raise OSError('Error [mcarats_ng]: <path_length> needs an integer number of bins ntp, 1 ... 1024.')
+    if not (np.isfinite(lo) and np.isfinite(hi) and 0.0 <= lo < hi):
+        raise OSError('Error [mcarats_ng]: <path_length> needs finite 0 <= tpmin_km < tpmax_km.')
+    return lo, hi, ntp
 
 
 def cal_mca_azimuth(normal_azimuth_angle):

@@ -28,7 +28,8 @@ class Solver:
         self.scene = None
         self.options = None
         self._keep = None
-        self._jac_ngrp = 0       # layer groups of the last run when it was a Jacobian run, else 0
+        self._xt_key = None      # 'jac' / 'plen' when the last run was a Jacobian / path-length run, else None
+        self._xt_width = 0       # doubles per radiance pixel of that run's tally (ngrp, or ntp + 3)
 
     # ------------------------------------------------------------------ helpers
     def _check(self, rc, where):
@@ -58,7 +59,7 @@ class Solver:
     def run(self, jobs, accumulate=False, stream=None, sync=True):
         """jobs: ctypes array of abi.Job (see abi.make_jobs)."""
         self._keep = jobs
-        self._jac_ngrp = 0
+        self._xt_key, self._xt_width = None, 0
         self._check(self.lib.b200rt_run(self.handle, jobs, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run')
         if sync:
             self.sync()
@@ -67,7 +68,7 @@ class Solver:
         """Spectral run: jobs (abi.make_jobs, without abs1d / flx_scale) and kd (abi.make_kd, one record per job): every
         history serves all k-distribution terms of its job."""
         self._keep = (jobs, kd)
-        self._jac_ngrp = 0
+        self._xt_key, self._xt_width = None, 0
         self._check(self.lib.b200rt_run_kd(self.handle, jobs, kd, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run_kd')
         if sync:
             self.sync()
@@ -81,7 +82,18 @@ class Solver:
         self._keep = (jobs, e)
         self._check(self.lib.b200rt_run_jac(self.handle, jobs, len(jobs), e.ctypes.data, e.size - 1, 1 if accumulate else 0, stream),
                     'b200rt_run_jac')
-        self._jac_ngrp = e.size - 1
+        self._xt_key, self._xt_width = 'jac', e.size - 1
+        if sync:
+            self.sync()
+
+    def run_plen(self, jobs, tpmin, tpmax, ntp, accumulate=False, stream=None, sync=True):
+        """b200rt_run that also tallies, per radiance pixel, the distribution of the geometric path lengths L (m) behind the
+        radiance: ntp uniform bins on [tpmin, tpmax), underflow, overflow and the first moment sum(c L) (include/b200rt.h);
+        same histories, same radiance."""
+        self._keep = jobs
+        self._check(self.lib.b200rt_run_plen(self.handle, jobs, len(jobs), float(tpmin), float(tpmax), int(ntp), 1 if accumulate else 0,
+                                             stream), 'b200rt_run_plen')
+        self._xt_key, self._xt_width = 'plen', int(ntp) + 3
         if sync:
             self.sync()
 
@@ -115,24 +127,42 @@ class Solver:
         self._check(self.lib.b200rt_read_rad(self.handle, out.ctypes.data, out.size), 'b200rt_read_rad')
         return out
 
-    def read_jac(self, out=None):
-        """Jacobian tally of the last run (run_jac): (nslab, sum_k nyr_k * nxr_k, ngrp), group fastest."""
-        if not self._jac_ngrp:
-            raise OSError('Error [er3t_b200]: read_jac: the last run was not a Jacobian run (run_jac).')
+    _XT_RUN = {'jac': ('Jacobian', 'run_jac'), 'plen': ('path-length', 'run_plen')}
+
+    def _read_xt(self, key, out):
+        if self._xt_key != key:
+            raise OSError('Error [er3t_b200]: read_%s: the last run was not a %s run (%s).' % ((key,) + self._XT_RUN[key]))
         n = self.scene.rad_size(self.options.nslab)
         if out is None:
-            out = np.empty(n * self._jac_ngrp, dtype=np.float64)
-        self._check(self.lib.b200rt_read_jac(self.handle, out.ctypes.data, out.size), 'b200rt_read_jac')
-        return out.reshape(self.options.nslab, -1, self._jac_ngrp)
+            out = np.empty(n * self._xt_width, dtype=np.float64)
+        self._check(getattr(self.lib, 'b200rt_read_' + key)(self.handle, out.ctypes.data, out.size), 'b200rt_read_' + key)
+        return out.reshape(self.options.nslab, -1, self._xt_width)
+
+    def _xt_ptr(self, key):
+        if self._xt_key != key:
+            return None, 0
+        p, n = C.c_void_p(), C.c_int64()
+        self._check(getattr(self.lib, 'b200rt_%s_ptr' % key)(self.handle, C.byref(p), C.byref(n)), 'b200rt_%s_ptr' % key)
+        return p.value, n.value
+
+    def read_jac(self, out=None):
+        """Jacobian tally of the last run (run_jac): (nslab, sum_k nyr_k * nxr_k, ngrp), group fastest."""
+        return self._read_xt('jac', out)
 
     def jac_ptr(self):
         """(device pointer, doubles) of the Jacobian tally of the last run (b200rt_jac_ptr), or (None, 0) when it was not a
         Jacobian run."""
-        if not self._jac_ngrp:
-            return None, 0
-        p, n = C.c_void_p(), C.c_int64()
-        self._check(self.lib.b200rt_jac_ptr(self.handle, C.byref(p), C.byref(n)), 'b200rt_jac_ptr')
-        return p.value, n.value
+        return self._xt_ptr('jac')
+
+    def read_plen(self, out=None):
+        """Path-length tally of the last run (run_plen): (nslab, sum_k nyr_k * nxr_k, ntp + 3), bins fastest: ntp bins,
+        underflow, overflow, first moment."""
+        return self._read_xt('plen', out)
+
+    def plen_ptr(self):
+        """(device pointer, doubles) of the path-length tally of the last run (b200rt_plen_ptr), or (None, 0) when it was not
+        a path-length run."""
+        return self._xt_ptr('plen')
 
     def read_heat(self, out=None):
         shape = self.scene.heat_shape(self.options.nslab)
@@ -151,8 +181,8 @@ class Solver:
             res['rad'] = self.read_rad()
         if t & abi.TARGET_HEATING:
             res['heat'] = self.read_heat()
-        if self._jac_ngrp:
-            res['jac'] = self.read_jac()
+        if self._xt_key:
+            res[self._xt_key] = self._read_xt(self._xt_key, None)
         res['stats'] = self.stats()
         return res
 

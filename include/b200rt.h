@@ -14,6 +14,8 @@
  *                                       one job per run serves all Ng terms of a wavelength
  *   b200rt_run_jac                   <- finite differences of whole runs with the gas absorption of a layer group
  *                                       scaled (no counterpart in MCARaTS: Rad_mplen stays 0, as er3t sets it)
+ *   b200rt_run_plen                  <- MCARaTS's path-length statistics (Rad_mplen, Rad_ntp, Rad_tpmin, Rad_tpmax),
+ *                                       which er3t switches off (Rad_mplen = 0); own layout, not MCARaTS's record
  *   b200rt_read_flux / _rad / _heat  <- `.bin` + `.ctl` parsing, er3t/rtm/mca/mca_out.py:48-103
  *                                       (and, through job.flx_scale / job.rad_scale, the g-weighting of
  *                                        mca_out.py:319-327,354-366,444-452,475-481)
@@ -240,6 +242,23 @@ int          b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd
 int          b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, const int32_t* edges, int ngrp, int accumulate,
                             void* cuda_stream);
 
+/* b200rt_run that also tallies the distribution of the photon path lengths behind every radiance pixel.  L (metres) is
+ * the geometric path of one local-estimate contribution c (as tallied into the radiance, job.rad_scale and the pixel
+ * factor included): from the photon's entry at TOA along every leg of its history to the event, then along the
+ * event -> sensor segment to the sensor's target level min(Rad_zloc, TOA).  Per pixel the tally holds ntp + 3 doubles:
+ *   0 ... ntp-1  c summed into uniform bins of width (tpmax - tpmin) / ntp on [tpmin, tpmax)
+ *   ntp          underflow, L < tpmin
+ *   ntp + 1      overflow, L >= tpmax
+ *   ntp + 2      the first moment, sum of c L
+ * so that entries 0 ... ntp+1 sum to the radiance and <L> = moment / radiance.  The bin index is computed in fp32 from
+ * the fp32 path.  1 <= ntp <= 1024, 0 <= tpmin < tpmax, all finite.  The radiance, draws and event counters are those of
+ * b200rt_run (stats.n_tally also counts the two updates per local estimate).  Radiance target with satellite sensors only,
+ * every solver mode (flux / heating targets, options.smem_tally >= 0 on scenes whose radiance tally fits shared memory,
+ * the all-sky camera and options.kernel = 9 are rejected).  With accumulate != 0 the previous run since the last upload,
+ * if any, must be a path-length run with the same tpmin, tpmax and ntp.  Same asynchronous contract as b200rt_run. */
+int          b200rt_run_plen(void* handle, const b200rt_job* jobs, int njob, double tpmin, double tpmax, int ntp, int accumulate,
+                             void* cuda_stream);
+
 /* Wait for the stream of the last run; checks tallies for NaN/Inf. */
 int          b200rt_sync(void* handle);
 
@@ -253,6 +272,10 @@ int          b200rt_read_heat(void* handle, double* dst, int64_t count);
  * count = doubles the caller provides.  b200rt_jac_ptr: its device pointer and size (in-place NCCL all-reduce). */
 int          b200rt_read_jac(void* handle, double* dst, int64_t count);
 int          b200rt_jac_ptr(void* handle, double** p, int64_t* n);
+/* Path-length tally of the last run, which must have been a b200rt_run_plen: [nslab][nrad][nyr][nxr][ntp+3] (bin
+ * fastest).  b200rt_plen_ptr: its device pointer and size. */
+int          b200rt_read_plen(void* handle, double* dst, int64_t count);
+int          b200rt_plen_ptr(void* handle, double** p, int64_t* n);
 /* Device pointers to the library-owned tallies (for in-place NCCL all-reduce by the caller). */
 int          b200rt_tally_ptrs(void* handle, double** flux, int64_t* nflux, double** rad, int64_t* nrad,
                                double** heat, int64_t* nheat);

@@ -88,8 +88,9 @@ class Stats(C.Structure):
 
 # every symbol include/b200rt.h declares (tests check the library exports all of them)
 EXPORTS = ['b200rt_version', 'b200rt_create', 'b200rt_destroy', 'b200rt_last_error', 'b200rt_upload_scene',
-           'b200rt_run', 'b200rt_run_kd', 'b200rt_run_jac', 'b200rt_run_plen', 'b200rt_sync', 'b200rt_read_flux', 'b200rt_read_rad',
-           'b200rt_read_heat', 'b200rt_read_jac', 'b200rt_jac_ptr', 'b200rt_read_plen', 'b200rt_plen_ptr', 'b200rt_tally_ptrs',
+           'b200rt_run', 'b200rt_run_kd', 'b200rt_run_jac', 'b200rt_run_plen', 'b200rt_run_act', 'b200rt_sync', 'b200rt_read_flux', 'b200rt_read_rad',
+           'b200rt_read_heat', 'b200rt_read_jac', 'b200rt_jac_ptr', 'b200rt_read_plen', 'b200rt_plen_ptr', 'b200rt_read_act',
+           'b200rt_act_ptr', 'b200rt_tally_ptrs',
            'b200rt_stats_get', 'b200rt_philox_fill', 'b200rt_phase_eval', 'b200rt_phase_sample', 'b200rt_brdf_eval']
 
 
@@ -128,13 +129,15 @@ def load_library(path=None):
     lib.b200rt_run_kd.argtypes = [vp, C.POINTER(Job), C.POINTER(Kd), C.c_int, C.c_int, vp]
     lib.b200rt_run_jac.argtypes = [vp, C.POINTER(Job), C.c_int, vp, C.c_int, C.c_int, vp]
     lib.b200rt_run_plen.argtypes = [vp, C.POINTER(Job), C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, vp]
+    lib.b200rt_run_act.argtypes = [vp, C.POINTER(Job), C.c_int, C.c_int, vp]
     lib.b200rt_sync.argtypes = [vp]
-    for name in ('b200rt_read_flux', 'b200rt_read_rad', 'b200rt_read_heat', 'b200rt_read_jac', 'b200rt_read_plen'):
+    for name in ('b200rt_read_flux', 'b200rt_read_rad', 'b200rt_read_heat', 'b200rt_read_jac', 'b200rt_read_plen', 'b200rt_read_act'):
         getattr(lib, name).argtypes = [vp, vp, C.c_int64]
     lib.b200rt_tally_ptrs.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_int64), C.POINTER(vp), C.POINTER(C.c_int64),
                                       C.POINTER(vp), C.POINTER(C.c_int64)]
     lib.b200rt_jac_ptr.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_int64)]
     lib.b200rt_plen_ptr.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_int64)]
+    lib.b200rt_act_ptr.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_int64)]
     lib.b200rt_stats_get.argtypes = [vp, C.POINTER(Stats)]
     lib.b200rt_philox_fill.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, vp, C.c_int64]
     lib.b200rt_phase_eval.argtypes = [vp, C.c_double, vp, vp, C.c_int64]

@@ -10,6 +10,7 @@
 //   tau_up_kernel          optical depth from each voxel to the top of the 3-D block (vertical local estimates)
 //   transport_kernel       persistent-thread photon transport with in-place regeneration, Philox streams,
 //                          two-level majorant grid + null-collision tracking, local-estimate radiance, fp64 tallies
+//                          (and, on request, track-length actinic flux, radiance Jacobians, path-length distributions)
 //   check_finite_kernel    NaN/Inf guard over the tallies
 // No CPU fallback exists: every entry point fails with an error code if CUDA fails.
 
@@ -164,10 +165,14 @@ struct DevScene {
     // per-slot state and per-pixel tally of the JAC and PLEN kernels
     float* xs;                // JAC: [block][warp][pool slot][jac_n] gas optical path of the slot's history per group (see jac_leg)
                               // PLEN: [block][warp][pool slot] geometric path of the slot's history so far (m)
-    double* xt;               // JAC: [nslab][rad_slab][jac_n] tally of dI / dln(a_j); PLEN: [nslab][rad_slab][pl_ntp+3] (plen_deposit)
+    double* xt;               // JAC: [nslab][rad_slab][jac_n] tally of dI / dln(a_j); PLEN: [nslab][rad_slab][pl_ntp+3] (plen_deposit);
+                              // ACT: [nslab][2][nz][ny][nx] actinic flux (act_move)
     // path-length distributions (b200rt_run_plen, read by the PLEN kernels only): pl_ntp bins on [pl_lo, pl_hi) metres
     int pl_ntp;
     float pl_lo, pl_hi, pl_inv_w;   // pl_inv_w = pl_ntp / (pl_hi - pl_lo)
+    // actinic flux (b200rt_run_act, read by the ACT kernels only): the tally is xt, [nslab][2][nz][ny][nx]; doubles of it held
+    // in the block-private shared tally next to flux and heating (0: global atomics)
+    int ntal_act_smem;
 };
 
 // ============================================================================ setup kernels
@@ -372,6 +377,7 @@ struct Smem {
     double* ftal;         // block- or warp-private flux tally (same layout as the global one) or nullptr
     double* htal;         // block- or warp-private heating tally or nullptr
     double* rtal;         // block- or warp-private radiance tally or nullptr
+    double* atal;         // block- or warp-private actinic tally or nullptr (ACT kernels only)
     int tal_mode;         // 1: one copy per block (shared atomics); 2: one copy per warp (plain read-modify-write)
     unsigned* cnt;        // event counters [8][32]: one slot per lane and block (flushed to 64-bit totals per block)
 };
@@ -786,6 +792,74 @@ __device__ __forceinline__ float* plen_state(const DevScene& S, int slot) {
     return S.xs + (size_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * NP + size_t(slot);
 }
 
+// ---- actinic flux: track-length estimate of the layer-and-column mean of F_act = integral of I over 4 pi ----------------
+// A flight move of length `len` inside layer iz adds the integral of the weight along the track, per column it crosses,
+// divided by the layer's thickness dz and scaled like the heating (fs = the job's heating scale of the layer).  With gas absorption k
+// the weight falls along the move: a segment of length l starting at weight w_a adds w_a (1 - exp(-k l)) / k, then
+// w_a <- w_a exp(-k l) -- the heating deposit of the segment over k, so that sum over the layer of k dz act = heating.
+// The kernel's own weight update stays the only one (this never touches the photon).  The move starts at (ux, uy) in fine
+// cells (svx x svy columns each) and runs along (dux, duy) per metre; the walk crosses column faces, periodic wraps
+// included.  col >= 0: the column of a frozen photon (no walk).  A move that crosses more than ACT_MAX_CROSS faces (a
+// near-horizontal photon in a transparent 1-D layer wraps the domain many times) puts the rest of its track into the
+// column where the walk stops: the domain mean stays exact.  out: the (slab, var 0, iz) plane of the tally, vstride the
+// distance to the var-1 (total) plane; direct photons add to both.  mode as tally_agg (0: global atomics).  Returns the
+// number of global updates.
+#define ACT_MAX_CROSS 65536
+__device__ __noinline__ unsigned act_move(double* __restrict__ out, size_t vstride, int mode, int direct, int nx, int ny, int svx,
+                                          int svy, float ux, float uy, float dux, float duy, float len, float w, float k,
+                                          double fs, float dz, int col) {
+    const double sc = fs / double(dz);
+    const float ik = k > 0.0f ? 1.0f / k : 0.0f;
+    float px = ux * float(svx), py = uy * float(svy);
+    const float vx = dux * float(svx), vy = duy * float(svy);
+    int ix = col >= 0 ? col % nx : min(nx - 1, max(0, __float2int_rd(px)));
+    int iy = col >= 0 ? col / nx : min(ny - 1, max(0, __float2int_rd(py)));
+    const int stx = vx > 0.0f ? 1 : -1, sty = vy > 0.0f ? 1 : -1;
+    const float ax = fabsf(1.0f / vx), ay = fabsf(1.0f / vy);      // metres per column crossed (|v| >= 1e-20 per fine cell)
+    float tx = col >= 0 ? RT_INF : fmaxf(0.0f, (float(ix + (stx > 0 ? 1 : 0)) - px) / vx);
+    float ty = col >= 0 ? RT_INF : fmaxf(0.0f, (float(iy + (sty > 0 ? 1 : 0)) - py) / vy);
+    float rem = len, wa = w;
+    unsigned n = 0;
+    for (int c = 0;; ++c) {
+        const float l = c < ACT_MAX_CROSS ? fmaxf(0.0f, fminf(rem, fminf(tx, ty))) : rem;
+        if (l > 0.0f) {
+            const float f = -expm1f(-k * l);                // fraction of w_a absorbed over the segment
+            const double d = double(k > 0.0f ? wa * f * ik : wa * l) * sc;
+            double* o = out + size_t(iy) * size_t(nx) + size_t(ix);
+            if (mode == 0) {
+                tally_add(o + vstride, d);
+                n++;
+                if (direct) { tally_add(o, d); n++; }
+            } else {
+                tally_agg(o + vstride, d, mode);
+                if (direct) tally_agg(o, d, mode);
+            }
+            wa -= wa * f;
+        }
+        rem -= l;
+        if (!(rem > 0.0f) || !(wa > 0.0f)) break;
+        if (tx <= ty) {
+            ix += stx; ix = ix >= nx ? 0 : (ix < 0 ? nx - 1 : ix);
+            ty -= l; tx = ax;
+        } else {
+            iy += sty; iy = iy >= ny ? 0 : (iy < 0 ? ny - 1 : iy);
+            tx -= l; ty = ay;
+        }
+    }
+    return n;
+}
+// one flight move of photon p (still at its start, weight before the move) in its layer p.is; col as act_move
+template <bool SMT>
+__device__ __forceinline__ unsigned act_add(const DevScene& S, const Smem& sm, const TallyCtx& t, const Photon& p, float ux, float uy,
+                                            float dux, float duy, float len, int col) {
+    const size_t nxy = size_t(S.nx) * size_t(S.ny);
+    const bool priv = SMT && sm.atal;
+    double* out = (priv ? sm.atal : S.xt) + 2 * size_t(t.hoff) + size_t(p.is) * nxy;
+    const float k = (p.flags & FL_ABS) ? __ldg(S.job_abs + size_t(p.job) * S.nz + p.is) : 0.0f;
+    return act_move(out, size_t(S.nz) * nxy, priv ? sm.tal_mode : 0, p.flags & FL_DIRECT, S.nx, S.ny, S.svx, S.svy, ux, uy, dux, duy,
+                    len, p.w, k, __ldg(t.fs + p.is), sm.z[p.is + 1] - sm.z[p.is], col);
+}
+
 // Exact optical depth toward a sensor for oblique views and sensors inside the atmosphere.
 //   * 1-D extinction and gas absorption are horizontally uniform: their integral over the whole segment is a difference
 //     of the cumulative profiles, O(1) whatever the number of layers;
@@ -1108,12 +1182,14 @@ __device__ __noinline__ float2 pick_component3(const float* __restrict__ ext3, c
 //     S.jac_n layer groups (jac_leg, jac_deposit); radiance, draws and event counters are those of XM_NONE.
 //   XM_PLEN (b200rt_run_plen): every history also tallies the distribution of the geometric path lengths behind each
 //     pixel's radiance (plen_state, plen_deposit); radiance, draws and event counters are those of XM_NONE.
+//   XM_ACT (b200rt_run_act, per-level kernels without radiance): every flight move also adds its track to the actinic flux
+//     tally (act_add); flux, heating, draws and event counters are those of XM_NONE.
 //   With XM_NONE none of that code exists, so the other kernels are unchanged.
-enum { XM_NONE = 0, XM_KD = 1, XM_JAC = 2, XM_PLEN = 3 };
+enum { XM_NONE = 0, XM_KD = 1, XM_JAC = 2, XM_PLEN = 3, XM_ACT = 4 };
 template <bool PL, bool FZ, int NP, bool CAM, bool UZ, bool RAD, bool NO3, int XM>
 __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid_constant__ DevScene S) {
     extern __shared__ float4 smem_f4[];
-    constexpr bool KD = XM == XM_KD, JAC = XM == XM_JAC, PLEN = XM == XM_PLEN;
+    constexpr bool KD = XM == XM_KD, JAC = XM == XM_JAC, PLEN = XM == XM_PLEN, ACT = XM == XM_ACT;
     constexpr bool SMT = PL && UZ;      // block-private tallies exist only in the kernels of plane-parallel / few-column scenes
     Smem sm;
     float* pool;
@@ -1129,7 +1205,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
         double* acc_atm = acc + 4 * 32;
         double* tal = acc_atm + blockDim.x;
         // private tallies: one copy per block (shared atomics) or one per warp (tal_per_warp)
-        const int ntal1 = SMT ? S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem : 0;
+        const int ntal1 = SMT ? S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem + (ACT ? S.ntal_act_smem : 0) : 0;
         const int ntal = ntal1 * (S.tal_per_warp ? int(blockDim.x >> 5) : 1);
         unsigned* cnt = reinterpret_cast<unsigned*>(tal + ntal);
         float* q = reinterpret_cast<float*>(cnt + 8 * 32);
@@ -1174,6 +1250,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
             sm.ftal = nf > 0 ? mine : nullptr;
             sm.htal = nh > 0 ? mine + nf : nullptr;
             sm.rtal = (SMT && S.ntal_rad_smem > 0) ? mine + nf + nh : nullptr;
+            sm.atal = (ACT && SMT && S.ntal_act_smem > 0) ? mine + nf + nh + S.ntal_rad_smem : nullptr;
             sm.tal_mode = S.tal_per_warp ? 2 : 1;
         }
         for (int i = (threadIdx.x & 31); i < NP; i += 32) qD[i] = (unsigned short)i;
@@ -1353,6 +1430,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                         const float M = A1.z;
                         const bool hit = p.tau < M * seg;
                         const float dmove = hit ? __fdividef(p.tau, M) : seg;
+                        if (ACT) CNT_ADD(CNT_TALLY, act_add<SMT>(S, sm, tcf, p, ux, uy, dux, duy, dmove, frozen ? p.ciy * S.nx + p.cix : -1));
                         if (p.flags & FL_ABS) {
                             const float wn = p.w * __expf(-__ldg(S.job_abs + size_t(p.job) * S.nz + p.is) * dmove);
                             ACC_ADD(ACC_ATM, double(p.w) - double(wn));
@@ -1442,6 +1520,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
                     const bool yc = !hit && !zc && !xc;
 
                     // ---- move
+                    if (ACT) CNT_ADD(CNT_TALLY, act_add<SMT>(S, sm, tcf, p, ux, uy, dux, duy, dmove, frozen ? p.ciy * S.nx + p.cix : -1));
                     if (PL && (p.flags & FL_ABS)) {
                         // flux / heating targets: weight must be current at every level (slabs are single layers here)
                         const float wn = p.w * __expf(-__ldg(S.job_abs + size_t(p.job) * S.nz + p.is) * dmove);
@@ -1785,19 +1864,23 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
 #undef QPUSH_DEAD
 
     // ---- flush the block-private tallies (one global atomic per non-zero entry and block)
-    if (SMT && (sm.ftal || sm.htal || sm.rtal)) {
+    if (SMT && (sm.ftal || sm.htal || sm.rtal || (ACT && sm.atal))) {
         __syncthreads();
         const int nf = sm.ftal ? S.ntal_flux_smem : 0, nh = sm.htal ? S.ntal_heat_smem : 0, nr = S.ntal_rad_smem;
-        const int ntal1 = nf + nh + nr;
+        const int na = ACT && sm.atal ? S.ntal_act_smem : 0;
+        const int ntal1 = nf + nh + nr + na;
         const int ncopy = S.tal_per_warp ? int(blockDim.x >> 5) : 1;
         // every warp computed its own `mine`; copy 0 starts where warp 0's (or the block's) copy does
-        const double* tal0 = (sm.ftal ? sm.ftal : (sm.htal ? sm.htal : sm.rtal)) - (S.tal_per_warp ? (threadIdx.x >> 5) * ntal1 : 0);
+        const double* mine = ACT ? (sm.ftal ? sm.ftal : (sm.htal ? sm.htal : (sm.rtal ? sm.rtal : sm.atal)))
+                                 : (sm.ftal ? sm.ftal : (sm.htal ? sm.htal : sm.rtal));
+        const double* tal0 = mine - (S.tal_per_warp ? (threadIdx.x >> 5) * ntal1 : 0);
         for (int i = threadIdx.x; i < ntal1; i += blockDim.x) {
             double v = 0.0;
             for (int c = 0; c < ncopy; ++c) v += tal0[c * ntal1 + i];
             if (v != 0.0) {
                 if (i < nf) tally_add(S.flux + i, v);
                 else if (i < nf + nh) tally_add(S.heat + (i - nf), v);
+                else if (ACT && i >= nf + nh + nr) tally_add(S.xt + (i - nf - nh - nr), v);
                 else tally_add(S.rad + (i - nf - nh), v);
                 CNT_ADD(CNT_TALLY, 1u);
             }
@@ -1866,6 +1949,12 @@ static transport_fn pick_transport_np(bool pl, bool fz, bool cam, bool uz, bool 
     if (xm == XM_PLEN) {
         if (fz) return uz ? transport_kernel<false, true, NP, false, true, true, false, XM_PLEN> : transport_kernel<false, true, NP, false, false, true, false, XM_PLEN>;
         return uz ? transport_kernel<false, false, NP, false, true, true, false, XM_PLEN> : transport_kernel<false, false, NP, false, false, true, false, XM_PLEN>;
+    }
+    // ACT (b200rt_run_act): the per-level kernels without radiance, carrying the actinic tally
+    if (xm == XM_ACT) {
+        if (fz) return uz ? transport_kernel<true, true, NP, false, true, false, false, XM_ACT> : transport_kernel<true, true, NP, false, false, false, false, XM_ACT>;
+        if (uz && no3) return transport_kernel<true, false, NP, false, true, false, true, XM_ACT>;
+        return uz ? transport_kernel<true, false, NP, false, true, false, false, XM_ACT> : transport_kernel<true, false, NP, false, false, false, false, XM_ACT>;
     }
     if (pl) {
         if (cam) return transport_kernel<true, false, NP, true, false, true, false, XM_NONE>;
@@ -1943,11 +2032,13 @@ struct Handle {
     DevBuf jobs, job_abs, job_cabs, job_fscale, counter, stats, flag;
     DevBuf kd_tab, kd_rf, kd_r;   // spectral runs: per-term tables and the per-slot term state
     DevBuf jac_lev, jac_grp;     // Jacobian runs: group edges, group of every layer
-    DevBuf xs, xt;               // Jacobian and path-length runs: per-slot state, per-pixel tally (DevScene::xs, xt)
+    DevBuf xs, xt;               // Jacobian and path-length runs: per-slot state, per-pixel tally (DevScene::xs, xt);
+                                 // actinic runs: the per-layer tally in xt
     size_t nxt = 0;
-    int xt_mode = 0;             // XM_JAC / XM_PLEN: the last run (since the last upload) was such a run and `xt` holds its
-                                 // tally; XM_NONE otherwise
+    int xt_mode = 0;             // XM_JAC / XM_PLEN / XM_ACT: the last run (since the last upload) was such a run and `xt`
+                                 // holds its tally; XM_NONE otherwise
     std::vector<double> xt_key;  // its parameters (group edges, or tpmin, tpmax, ntp): what `accumulate` must match
+    int ntal_act_smem = 0;       // doubles of an actinic tally that go to the block-private shared tally (DevScene::ntal_act_smem)
     DevBuf flux, rad, heat;
     size_t nflux = 0, nrad = 0, nheat = 0;
     std::vector<float> h_zgrd;
@@ -2526,7 +2617,8 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     // block-private tallies when the whole flux + heating tally is small (plane-parallel / few-column scenes)
     // (smem_tally: < 0 off; 0 auto = one copy per block, warp-aggregated shared atomics; 2 = one copy per warp when that
     // fits 24 KB, plain read-modify-write after the aggregation)
-    S.ntal_flux_smem = 0; S.ntal_heat_smem = 0; S.ntal_rad_smem = 0; S.tal_per_warp = 0;
+    S.ntal_flux_smem = 0; S.ntal_heat_smem = 0; S.ntal_rad_smem = 0; S.tal_per_warp = 0; S.ntal_act_smem = 0;
+    H->ntal_act_smem = 0;
     if (opt->smem_tally >= 0 && per_level && (nz3 <= 0 || size_t(sc->nx) * sc->ny <= 64)) {      // the scenes whose kernels hold private tallies
         // two blocks per SM must still fit (pools of 96 slots per warp + tables + accumulators + the private tallies)
         auto fits2 = [&](size_t ntal) {
@@ -2537,6 +2629,11 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
         if (H->nrad > 0 && H->nrad <= 512 && fits2(size_t(S.ntal_flux_smem) + S.ntal_heat_smem + H->nrad)) S.ntal_rad_smem = int(H->nrad);
         const size_t tot = size_t(S.ntal_flux_smem) + S.ntal_heat_smem + S.ntal_rad_smem;
         if (opt->smem_tally == 2 && tot > 0 && tot * 8 * (RT_TPB / 32) <= 24 * 1024) S.tal_per_warp = 1;
+        // an actinic run's tally joins them when all of it still fits (same limits, per-warp copies included)
+        const size_t nact = 2 * size_t(opt->nslab) * nz * nxy;
+        if (tot > 0 && tot == H->nflux + H->nheat + H->nrad && tot + nact <= 2048 && fits2(tot + nact) &&
+            (!S.tal_per_warp || (tot + nact) * 8 * (RT_TPB / 32) <= 24 * 1024))
+            H->ntal_act_smem = int(nact);
     }
     H->k_pl = per_level; H->k_fz = (opt->solver != B200RT_SOLVER_3D);
     H->k_cam = false;
@@ -2554,9 +2651,9 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
 
 }  // extern "C"
 
-// what a Jacobian or path-length run adds to b200rt_run: the kernels' mode and its parameters
+// what a Jacobian, path-length or actinic run adds to b200rt_run: the kernels' mode and its parameters
 struct XtArgs {
-    int mode = XM_NONE;                        // XM_NONE, XM_JAC or XM_PLEN
+    int mode = XM_NONE;                        // XM_NONE, XM_JAC, XM_PLEN or XM_ACT
     const int32_t* edges = nullptr;            // XM_JAC: edges[ngrp+1], the layer groups of the Jacobian tally
     int ngrp = 0;
     double tpmin = 0.0, tpmax = 0.0;           // XM_PLEN: ntp bins on [tpmin, tpmax) metres
@@ -2564,7 +2661,7 @@ struct XtArgs {
 };
 
 // b200rt_run (kd == nullptr, xa.mode = XM_NONE), b200rt_run_kd (kd[njob]: the gas-absorption terms of every job),
-// b200rt_run_jac and b200rt_run_plen (xa)
+// b200rt_run_jac, b200rt_run_plen and b200rt_run_act (xa)
 static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, const XtArgs& xa, int njob, int accumulate,
                     void* cuda_stream) {
     if (!H->have_scene) return fail(H, B200RT_ERR_STATE, "b200rt_run called before b200rt_upload_scene");
@@ -2598,12 +2695,23 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
             kd_n = std::max(kd_n, k.nkd);
         }
     }
-    const bool plen = xa.mode == XM_PLEN;
+    const bool plen = xa.mode == XM_PLEN, act = xa.mode == XM_ACT;
     const int32_t* edges = xa.mode == XM_JAC ? xa.edges : nullptr;
     const int jac_n = edges ? xa.ngrp : 0;
     size_t xt_n = 0;              // doubles per radiance pixel of the extra tally (DevScene::xt)
+    size_t nxt = 0;               // doubles of the whole extra tally
     std::vector<double> xt_key;
-    if (xa.mode != XM_NONE) {
+    if (act) {
+        const std::string who = "b200rt_run_act: ";
+        if (!(S.target & (B200RT_TARGET_FLUX | B200RT_TARGET_HEATING)))
+            return fail(H, B200RT_ERR_ARG, who + "needs the flux or heating target");
+        if (H->k_cam) return fail(H, B200RT_ERR_ARG, who + "the all-sky camera (Rad_mrkind = 1) is not supported");
+        if (k_rad) return fail(H, B200RT_ERR_ARG, who + "no radiance sensors in the same run (drop the radiance target)");
+        if (kver == 9) return fail(H, B200RT_ERR_ARG, who + "not available with options.kernel = 9");
+        if (accumulate && H->ran && H->xt_mode != XM_ACT)
+            return fail(H, B200RT_ERR_ARG, who + "accumulate needs the previous run to be an actinic run");
+        nxt = 2 * size_t(H->opt.nslab) * nz * size_t(S.nx) * size_t(S.ny);
+    } else if (xa.mode != XM_NONE) {
         const std::string who = edges ? "b200rt_run_jac: " : "b200rt_run_plen: ";
         if (H->k_pl)
             return fail(H, B200RT_ERR_ARG, who + "radiance targets only (no flux / heating; tiny radiance tallies held in shared memory "
@@ -2632,6 +2740,7 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
         if (accumulate && H->ran && !(H->xt_mode == xa.mode && H->xt_key == xt_key))
             return fail(H, B200RT_ERR_ARG, who + (edges ? "accumulate needs the previous run to be a Jacobian run with the same edges"
                                                         : "accumulate needs the previous run to be a path-length run with the same binning"));
+        nxt = H->nrad * xt_n;
     }
     CK(cudaSetDevice(H->device));
     CK(drain(H));                 // one run in flight per handle: the previous one still reads the job tables and counters
@@ -2739,14 +2848,15 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
         CK(cudaMemcpyAsync(H->jac_lev.p, jl, b_jl, cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(H->jac_grp.p, jg, b_jg, cudaMemcpyHostToDevice, st));
     }
-    if (xt_n) {
+    if (nxt) {
         // `xt` is resized / zeroed from here on: until this run has launched it holds no valid tally (a failure below must
-        // not leave b200rt_read_jac / _plen reading the previous run's size out of this buffer)
+        // not leave b200rt_read_jac / _plen / _act reading the previous run's size out of this buffer)
         H->xt_mode = XM_NONE;
-        if ((rc = dev_alloc(H, H->xt, H->nrad * xt_n * 8))) return rc;
-        // zeroed unless this run adds to the previous run of the same kind (the radiance tally is zero after an upload anyway)
-        if (!accumulate || !H->ran) CK(cudaMemsetAsync(H->xt.p, 0, H->nrad * xt_n * 8, st));
+        if ((rc = dev_alloc(H, H->xt, nxt * 8))) return rc;
+        // zeroed unless this run adds to the previous run of the same kind (the other tallies are zero after an upload anyway)
+        if (!accumulate || !H->ran) CK(cudaMemsetAsync(H->xt.p, 0, nxt * 8, st));
     }
+    S.ntal_act_smem = act ? H->ntal_act_smem : 0;
     S.jac_n = jac_n; S.jac_lev = (const int*)H->jac_lev.p; S.jac_grp = (const unsigned char*)H->jac_grp.p; S.xt = (double*)H->xt.p;
     S.pl_ntp = plen ? xa.ntp : 0; S.pl_lo = float(xa.tpmin); S.pl_hi = float(xa.tpmax);
     S.pl_inv_w = plen ? float(double(xa.ntp) / (double(S.pl_hi) - double(S.pl_lo))) : 0.0f;
@@ -2799,7 +2909,7 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     const bool k_uz = H->k_pl ? (S.nz3 <= 0 || size_t(S.nx) * S.ny <= 64) : ((S.uz_ok != 0 && H->cmz == 1) || S.nz3 <= 0);
     transport_fn kern = pick_transport(H->k_pl, H->k_fz, H->k_cam, k_uz, k_rad, S.nz3 <= 0, kd ? XM_KD : xa.mode, np);
     const size_t smem = H->smem_tables + 32 * (4 * 8 + 8 * 4) + size_t(tpb) * 8 + size_t(tpb / 32) * size_t(POOL_WORDS(np)) * 4 +
-                        8 * size_t(S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem) * size_t(S.tal_per_warp ? RT_TPB / 32 : 1);
+                        8 * size_t(S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem + S.ntal_act_smem) * size_t(S.tal_per_warp ? RT_TPB / 32 : 1);
     if (smem > 227 * 1024) return fail(H, B200RT_ERR_ARG, "photon pools + 1-D tables exceed shared memory; lower threads_per_block or pool_slots");
     CK(set_smem_attr(H, (const void*)kern, smem));
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, tpb, smem));
@@ -2812,7 +2922,7 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
         if ((rc = dev_alloc(H, H->kd_r, size_t(grid) * (tpb / 32) * np * kd_n * 4))) return rc;
         S.kd_r = (float*)H->kd_r.p;
     }
-    if (xt_n) {
+    if (xt_n) {     // (JAC, PLEN)
         // per-slot state of every pool slot of the launch: [block][warp][slot][jac_n] per-group paths, or [block][warp][slot] path
         if ((rc = dev_alloc(H, H->xs, size_t(grid) * (tpb / 32) * np * (edges ? jac_n : 1) * 4))) return rc;
         S.xs = (float*)H->xs.p;
@@ -2827,9 +2937,9 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     H->inflight = true;
     H->launches = 1;
     H->xt_mode = xa.mode;
-    if (xt_n) {
+    if (nxt) {
         H->xt_key = xt_key;
-        H->nxt = H->nrad * xt_n;
+        H->nxt = nxt;
     }
     return B200RT_OK;
 }
@@ -2864,6 +2974,14 @@ int b200rt_run_plen(void* handle, const b200rt_job* jobs, int njob, double tpmin
     if (!H) return B200RT_ERR_ARG;
     XtArgs xa;
     xa.mode = XM_PLEN; xa.tpmin = tpmin; xa.tpmax = tpmax; xa.ntp = ntp;
+    return run_jobs(H, jobs, nullptr, xa, njob, accumulate, cuda_stream);
+}
+
+int b200rt_run_act(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream) {
+    Handle* H = static_cast<Handle*>(handle);
+    if (!H) return B200RT_ERR_ARG;
+    XtArgs xa;
+    xa.mode = XM_ACT;
     return run_jobs(H, jobs, nullptr, xa, njob, accumulate, cuda_stream);
 }
 
@@ -2930,18 +3048,19 @@ int b200rt_read_heat(void* handle, double* dst, int64_t count) {
     return read_any(H, H->heat, H->nheat, dst, count, "heating");
 }
 
-// the per-pixel tally of the last run, which must have been a run of kind `mode` (XM_JAC or XM_PLEN)
+// the extra tally of the last run, which must have been a run of kind `mode` (XM_JAC, XM_PLEN or XM_ACT)
 static int check_xt(Handle* H, int mode) {
     if (!H->ran || H->xt_mode != mode)
-        return fail(H, B200RT_ERR_STATE, mode == XM_JAC ? "the last run was not a Jacobian run (b200rt_run_jac)"
-                                                        : "the last run was not a path-length run (b200rt_run_plen)");
+        return fail(H, B200RT_ERR_STATE, mode == XM_JAC    ? "the last run was not a Jacobian run (b200rt_run_jac)"
+                                         : mode == XM_PLEN ? "the last run was not a path-length run (b200rt_run_plen)"
+                                                           : "the last run was not an actinic run (b200rt_run_act)");
     return B200RT_OK;
 }
 static int read_xt(void* handle, int mode, double* dst, int64_t count) {
     Handle* H = static_cast<Handle*>(handle);
     if (!H) return B200RT_ERR_ARG;
     if (int rc = check_xt(H, mode)) return rc;
-    return read_any(H, H->xt, H->nxt, dst, count, mode == XM_JAC ? "Jacobian" : "path-length tally");
+    return read_any(H, H->xt, H->nxt, dst, count, mode == XM_JAC ? "Jacobian" : (mode == XM_PLEN ? "path-length tally" : "actinic flux"));
 }
 static int xt_ptr(void* handle, int mode, double** p, int64_t* n) {
     Handle* H = static_cast<Handle*>(handle);
@@ -2956,6 +3075,8 @@ int b200rt_read_jac(void* handle, double* dst, int64_t count) { return read_xt(h
 int b200rt_jac_ptr(void* handle, double** p, int64_t* n) { return xt_ptr(handle, XM_JAC, p, n); }
 int b200rt_read_plen(void* handle, double* dst, int64_t count) { return read_xt(handle, XM_PLEN, dst, count); }
 int b200rt_plen_ptr(void* handle, double** p, int64_t* n) { return xt_ptr(handle, XM_PLEN, p, n); }
+int b200rt_read_act(void* handle, double* dst, int64_t count) { return read_xt(handle, XM_ACT, dst, count); }
+int b200rt_act_ptr(void* handle, double** p, int64_t* n) { return xt_ptr(handle, XM_ACT, p, n); }
 
 int b200rt_tally_ptrs(void* handle, double** flux, int64_t* nflux, double** rad, int64_t* nrad, double** heat, int64_t* nheat) {
     Handle* H = static_cast<Handle*>(handle);

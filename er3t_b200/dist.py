@@ -52,8 +52,8 @@ def allreduce_results(solver, to_host=True):
     """
     Sum the tallies of all ranks.  With NCCL the all-reduce runs IN PLACE on the library's own device buffers (no staging
     tensor, no device-to-device copy): afterwards every rank's handle holds the global tallies and `solver.results()` /
-    `b200rt_read_*` return them.  After a Jacobian run (`Solver.run_jac`) or a path-length run (`Solver.run_plen`) its tally
-    is reduced too (`res['jac']` / `res['plen']`).  With gloo (CPU tests) the host arrays are reduced.  The run is waited for first
+    `b200rt_read_*` return them.  After a Jacobian run (`Solver.run_jac`), a path-length run (`Solver.run_plen`) or an
+    actinic run (`Solver.run_act`) its tally is reduced too (`res['jac']` / `res['plen']` / `res['act']`).  With gloo (CPU tests) the host arrays are reduced.  The run is waited for first
     (`solver.sync()`: NaN guard + fresh event counters), and the event counters are reduced with the same collective.
     """
     import torch
@@ -64,7 +64,7 @@ def allreduce_results(solver, to_host=True):
     if hasattr(solver, 'sync'):
         solver.sync()
     st = solver.stats()
-    xt = getattr(solver, '_xt_key', None)       # 'jac' / 'plen': the per-pixel tally of a Jacobian / path-length run
+    xt = getattr(solver, '_xt_key', None)       # 'jac' / 'plen' / 'act': the extra tally of a Jacobian / path-length / actinic run
     keys = ('flux', 'rad', 'heat') + ((xt,) if xt else ())
     if use_cuda:
         views = tally_views(solver)

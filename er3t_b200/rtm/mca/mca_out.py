@@ -262,6 +262,29 @@ def read_heating_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
     return d
 
 
+def read_actinic_mca_out(mca_obj, abs_obj, mode='mean', squeeze=True):
+    """Actinic flux (spherical irradiance, W/m^2/nm) of a simulation that carried it (mcarats_ng(actinic=True)): f_act,
+    f_act_direct, f_act_diffuse (+ _std), the mean over every layer and column, g-weighted like the heating."""
+    mode = mode.lower()
+    act, = _per_run_arrays(mca_obj, abs_obj, 'actinic')           # (Nx, Ny, Nz, 2, Nrun): direct, total
+    direct, dims_info = _finish(act[:, :, :, 0:1, :], squeeze)
+    total, _ = _finish(act[:, :, :, 1:2, :], squeeze)
+    fields = (('f_act', total, 'Actinic flux'), ('f_act_direct', direct, 'Direct actinic flux'),
+              ('f_act_diffuse', total - direct, 'Diffuse actinic flux'))
+    d = {}
+    if mode == 'all':
+        for key, arr, name in fields:
+            d[key] = {'data': arr, 'name': name, 'units': 'W/m^2/nm', 'dims_info': dims_info}
+    elif mode == 'mean':
+        for key, arr, name in fields:
+            d[key] = {'data': np.mean(arr, axis=-1), 'name': name + ' (mean)', 'units': 'W/m^2/nm', 'dims_info': dims_info[:-1]}
+        for key, arr, name in fields:
+            d[key + '_std'] = {'data': np.std(arr, axis=-1), 'name': name + ' (standard deviation)', 'units': 'W/m^2/nm', 'dims_info': dims_info[:-1]}
+    else:
+        raise OSError('Error [read_actinic_mca_out]: Do not support <mode=%s>.' % mode)
+    return d
+
+
 class mca_out_ng:
 
     """
@@ -275,6 +298,7 @@ class mca_out_ng:
     self.data['f_up'|'f_down'|'f_down_direct'|'f_down_diffuse'|...'_std'|'rad'|'rad_std'|'toa'|'N_photon'|'N_run']
     (+ 'rad_jac', 'rad_jac_std', 'jac_levels' when the simulation carried a gas-absorption Jacobian)
     (+ 'rad_plen', 'rad_plen_std', 'rad_plen_out', 'rad_mean_plen', 'plen_edges' when it carried a path-length tally)
+    (+ 'f_act', 'f_act_direct', 'f_act_diffuse' and their '_std' when it carried the actinic flux)
     Same loading rules as the reference (mca_out.py:160-177).
     """
 
@@ -308,6 +332,9 @@ class mca_out_ng:
         elif self.mca.target == 'heating rate':
             self.data = read_flux_mca_out(self.mca, self.abs, mode=self.mode, squeeze=self.squeeze)
             self.data.update(read_heating_mca_out(self.mca, self.abs, mode=self.mode, squeeze=self.squeeze))
+        fused = getattr(self.mca, 'fused', None)
+        if self.mca.target != 'radiance' and fused is not None and fused.get('actinic') is not None:
+            self.data.update(read_actinic_mca_out(self.mca, self.abs, mode=self.mode, squeeze=self.squeeze))
 
     # ---- persistence: HDF5 group '<mode>/<key>' with attrs name/units/dims_info (mca_out.py:209-233)
     def dump(self):

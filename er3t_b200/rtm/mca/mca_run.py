@@ -28,13 +28,14 @@ class mca_run:
     kd      : keywords of abi.make_kd (spectral run, b200rt_run_kd: every job serves all these terms) or None
     jac_edges : layer-group edges of a Jacobian run (b200rt_run_jac) or None
     plen    : (tpmin, tpmax, ntp), metres, of a path-length run (b200rt_run_plen) or None
+    act     : True for an actinic run (b200rt_run_act)
 
     Ncpu, mp_mode are accepted for signature compatibility and ignored.
     """
 
     def __init__(self, scene, options, photons, seeds, slabs, abs1d=None, flx_scale=None, rad_scale=None,
                  device=0, solver_obj=None, Ncpu=None, mp_mode='py', verbose=False, quiet=False, run=True, kd=None,
-                 jac_edges=None, plen=None):
+                 jac_edges=None, plen=None, act=False):
         self.scene = scene
         self.options = options
         self.quiet = quiet
@@ -42,6 +43,7 @@ class mca_run:
         self.jobs, self._keep = abi.make_jobs(photons, seeds, slabs, abs1d=abs1d, flx_scale=flx_scale, rad_scale=rad_scale)
         self.jac_edges = jac_edges
         self.plen = plen
+        self.act = act
         self.kd = None
         if kd is not None:
             self.kd, keep = abi.make_kd(njob=len(self.jobs), **kd)
@@ -61,6 +63,8 @@ class mca_run:
             self.solver.run_jac(self.jobs, self.jac_edges)
         elif self.plen is not None:
             self.solver.run_plen(self.jobs, *self.plen)
+        elif self.act:
+            self.solver.run_act(self.jobs)
         else:
             self.solver.run(self.jobs)
 

@@ -84,7 +84,8 @@ class mcarats_ng:
                  dry_run=False,
                  spectral=False,
                  gas_jacobian=None,
-                 path_length=None):
+                 path_length=None,
+                 actinic=False):
         """spectral=True: one job per run traces `photons` histories (not photons per g), each of which carries all Ng
         terms of the correlated-k set (Atm_nkd = Ng, Atm_wkd0 = weights; Iwabuchi and Okamura 2017).  `self.fused` has the
         same layout and meaning as without it.  Needs target='radiance' with the satellite sensor and an `abs` object;
@@ -103,7 +104,13 @@ class mcarats_ng:
         path of one local-estimate contribution runs from TOA along the whole history to the event and on to the sensor
         level.  Results: `self.fused['path_length']` (nx, ny, ntp+3, 1, Nrun): ntp uniform bins on [tpmin, tpmax), underflow,
         overflow and the first moment sum(c L) in metres (include/b200rt.h); `self.plen_extra` for the extra sensors and
-        `self.plen_edges` (km).  Same rules as `gas_jacobian`, with which it cannot be combined."""
+        `self.plen_edges` (km).  Same rules as `gas_jacobian`, with which it cannot be combined.
+
+        actinic=True: also tally, in the same histories, the actinic flux (spherical irradiance, the radiance integrated over
+        all directions) as the mean over every layer and column, direct and total, in the units of the flux and with its
+        g-weighting.  Result: `self.fused['actinic']` (nx, ny, nz, 2, Nrun), variable 0 direct, 1 total.  Needs
+        target='flux', 'flux0' or 'heating rate' and an `abs` object; the radiance target, `spectral`, `raw` and
+        `write_files` raise OSError."""
 
         add_reference(self.reference)
 
@@ -154,6 +161,7 @@ class mcarats_ng:
         self.plen = None if path_length is None else path_length_bins(path_length)     # (tpmin, tpmax, ntp), metres
         self.plen_edges = None if self.plen is None else np.linspace(self.plen[0], self.plen[1], self.plen[2] + 1) / 1000.0
         self.plen_extra = None
+        self.actinic = bool(actinic)
         self.atm_1ds = atm_1ds
         self.atm_3ds = atm_3ds
 
@@ -440,6 +448,15 @@ class mcarats_ng:
         else:
             tflag = abi.TARGET_RADIANCE
 
+        if self.actinic:
+            if self.target == 'radiance':
+                raise OSError('Error [mcarats_ng]: <actinic=True> supports target=\'flux\', \'flux0\' and \'heating rate\' only (not radiance).')
+            if self.spectral:
+                raise OSError('Error [mcarats_ng]: <actinic=True> is not available with <spectral=True>.')
+            if self.keep_raw:
+                raise OSError('Error [mcarats_ng]: <actinic=True> is tallied per run: <raw> and <write_files> are not available.')
+            if self.abs is None:
+                raise OSError('Error [mcarats_ng]: <actinic=True> needs the gas absorption object of <atm_1ds>.')
         if self.spectral:
             if self.keep_raw:
                 raise OSError('Error [mcarats_ng]: <spectral=True> sums the g terms in every history: <raw> and <write_files> are not available.')
@@ -533,7 +550,7 @@ class mcarats_ng:
         # the reference hands the job list to `mca_run` (mcarats.py:468); so does this class -- one launch instead of a pool
         runner = mca_run(scene, opt, nphot, seeds, slabs, abs1d=abs1d, flx_scale=fsc, rad_scale=rsc, device=self.device,
                          solver_obj=self._solver_obj, Ncpu=self.Ncpu, mp_mode=self.mp_mode, quiet=True, run=False, kd=kd,
-                         jac_edges=self.jac_edges, plen=self.plen)
+                         jac_edges=self.jac_edges, plen=self.plen, act=self.actinic)
         try:
             self.h2d_bytes = scene.nbytes() + sum(a.nbytes for a in runner._keep)
             runner.launch()
@@ -586,6 +603,9 @@ class mcarats_ng:
                     off += nk
                 self.fused[name] = [views[0][:, :, :, np.newaxis, :]]
                 setattr(self, extra, views[1:])
+            if res.get('act') is not None:
+                # [nslab][2][nz][ny][nx] -> (nx, ny, nz, 2, nslab)
+                self.fused['actinic'] = [np.transpose(np.asarray(res['act']).reshape(nslab, 2, nz, ny, nx), (4, 3, 2, 1, 0))]
         else:
             self.raw = []
             for ir in range(Nrun):

@@ -28,8 +28,8 @@ class Solver:
         self.scene = None
         self.options = None
         self._keep = None
-        self._xt_key = None      # 'jac' / 'plen' when the last run was a Jacobian / path-length run, else None
-        self._xt_width = 0       # doubles per radiance pixel of that run's tally (ngrp, or ntp + 3)
+        self._xt_key = None      # 'jac' / 'plen' / 'act' when the last run was a Jacobian / path-length / actinic run, else None
+        self._xt_shape = None    # shape of that run's tally
 
     # ------------------------------------------------------------------ helpers
     def _check(self, rc, where):
@@ -59,7 +59,7 @@ class Solver:
     def run(self, jobs, accumulate=False, stream=None, sync=True):
         """jobs: ctypes array of abi.Job (see abi.make_jobs)."""
         self._keep = jobs
-        self._xt_key, self._xt_width = None, 0
+        self._xt_key, self._xt_shape = None, None
         self._check(self.lib.b200rt_run(self.handle, jobs, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run')
         if sync:
             self.sync()
@@ -68,7 +68,7 @@ class Solver:
         """Spectral run: jobs (abi.make_jobs, without abs1d / flx_scale) and kd (abi.make_kd, one record per job): every
         history serves all k-distribution terms of its job."""
         self._keep = (jobs, kd)
-        self._xt_key, self._xt_width = None, 0
+        self._xt_key, self._xt_shape = None, None
         self._check(self.lib.b200rt_run_kd(self.handle, jobs, kd, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run_kd')
         if sync:
             self.sync()
@@ -82,7 +82,7 @@ class Solver:
         self._keep = (jobs, e)
         self._check(self.lib.b200rt_run_jac(self.handle, jobs, len(jobs), e.ctypes.data, e.size - 1, 1 if accumulate else 0, stream),
                     'b200rt_run_jac')
-        self._xt_key, self._xt_width = 'jac', e.size - 1
+        self._xt_key, self._xt_shape = 'jac', (self.options.nslab, self.scene.rad_size(1), e.size - 1)
         if sync:
             self.sync()
 
@@ -93,7 +93,17 @@ class Solver:
         self._keep = jobs
         self._check(self.lib.b200rt_run_plen(self.handle, jobs, len(jobs), float(tpmin), float(tpmax), int(ntp), 1 if accumulate else 0,
                                              stream), 'b200rt_run_plen')
-        self._xt_key, self._xt_width = 'plen', int(ntp) + 3
+        self._xt_key, self._xt_shape = 'plen', (self.options.nslab, self.scene.rad_size(1), int(ntp) + 3)
+        if sync:
+            self.sync()
+
+    def run_act(self, jobs, accumulate=False, stream=None, sync=True):
+        """b200rt_run that also tallies the actinic flux (spherical irradiance): the mean over every layer and column,
+        direct and total, in the units of the flux (include/b200rt.h); same histories, same flux and heating."""
+        self._keep = jobs
+        self._check(self.lib.b200rt_run_act(self.handle, jobs, len(jobs), 1 if accumulate else 0, stream), 'b200rt_run_act')
+        hs = self.scene.heat_shape(self.options.nslab)
+        self._xt_key, self._xt_shape = 'act', (hs[0], 2) + tuple(hs[1:])
         if sync:
             self.sync()
 
@@ -127,16 +137,15 @@ class Solver:
         self._check(self.lib.b200rt_read_rad(self.handle, out.ctypes.data, out.size), 'b200rt_read_rad')
         return out
 
-    _XT_RUN = {'jac': ('Jacobian', 'run_jac'), 'plen': ('path-length', 'run_plen')}
+    _XT_RUN = {'jac': ('a Jacobian', 'run_jac'), 'plen': ('a path-length', 'run_plen'), 'act': ('an actinic', 'run_act')}
 
     def _read_xt(self, key, out):
         if self._xt_key != key:
-            raise OSError('Error [er3t_b200]: read_%s: the last run was not a %s run (%s).' % ((key,) + self._XT_RUN[key]))
-        n = self.scene.rad_size(self.options.nslab)
+            raise OSError('Error [er3t_b200]: read_%s: the last run was not %s run (%s).' % ((key,) + self._XT_RUN[key]))
         if out is None:
-            out = np.empty(n * self._xt_width, dtype=np.float64)
+            out = np.empty(int(np.prod(self._xt_shape)), dtype=np.float64)
         self._check(getattr(self.lib, 'b200rt_read_' + key)(self.handle, out.ctypes.data, out.size), 'b200rt_read_' + key)
-        return out.reshape(self.options.nslab, -1, self._xt_width)
+        return out.reshape(self._xt_shape)
 
     def _xt_ptr(self, key):
         if self._xt_key != key:
@@ -163,6 +172,15 @@ class Solver:
         """(device pointer, doubles) of the path-length tally of the last run (b200rt_plen_ptr), or (None, 0) when it was not
         a path-length run."""
         return self._xt_ptr('plen')
+
+    def read_act(self, out=None):
+        """Actinic flux of the last run (run_act): (nslab, 2, nz, ny, nx), variable 0 direct, 1 total."""
+        return self._read_xt('act', out)
+
+    def act_ptr(self):
+        """(device pointer, doubles) of the actinic tally of the last run (b200rt_act_ptr), or (None, 0) when it was not an
+        actinic run."""
+        return self._xt_ptr('act')
 
     def read_heat(self, out=None):
         shape = self.scene.heat_shape(self.options.nslab)

@@ -16,6 +16,7 @@
  *                                       scaled (no counterpart in MCARaTS: Rad_mplen stays 0, as er3t sets it)
  *   b200rt_run_plen                  <- MCARaTS's path-length statistics (Rad_mplen, Rad_ntp, Rad_tpmin, Rad_tpmax),
  *                                       which er3t switches off (Rad_mplen = 0); own layout, not MCARaTS's record
+ *   b200rt_run_act                   <- nothing: MCARaTS reports no actinic flux (mean radiance); own definition and layout
  *   b200rt_read_flux / _rad / _heat  <- `.bin` + `.ctl` parsing, er3t/rtm/mca/mca_out.py:48-103
  *                                       (and, through job.flx_scale / job.rad_scale, the g-weighting of
  *                                        mca_out.py:319-327,354-366,444-452,475-481)
@@ -259,6 +260,17 @@ int          b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, cons
 int          b200rt_run_plen(void* handle, const b200rt_job* jobs, int njob, double tpmin, double tpmax, int ntp, int accumulate,
                              void* cuda_stream);
 
+/* b200rt_run that also tallies the actinic flux (spherical irradiance, F_act = integral of the radiance over 4 pi sr) as
+ * the volume mean over every layer iz and atmosphere column, from the track length of every flight move in the voxel:
+ * sum of the integral of the weight along the track / dz, the weight falling with the layer's gas absorption along it.
+ * Same units and per-job factors as the flux (job.flx_scale of layer iz included): per unit Src_flx normal to the beam,
+ * so that a direct beam in vacuum gives Src_flx.  Two variables: 0 direct (photons that have not scattered), 1 total.
+ * Trajectories never change, so flux, heating, draws and event counters are those of b200rt_run (stats.n_tally also
+ * counts the actinic updates that go to global memory).  Flux and / or heating target only: radiance sensors in the same
+ * run, the all-sky camera and options.kernel = 9 are rejected.  With accumulate != 0 the previous run since the last
+ * upload, if any, must be an actinic run.  Same asynchronous contract as b200rt_run. */
+int          b200rt_run_act(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream);
+
 /* Wait for the stream of the last run; checks tallies for NaN/Inf. */
 int          b200rt_sync(void* handle);
 
@@ -276,6 +288,10 @@ int          b200rt_jac_ptr(void* handle, double** p, int64_t* n);
  * fastest).  b200rt_plen_ptr: its device pointer and size. */
 int          b200rt_read_plen(void* handle, double* dst, int64_t count);
 int          b200rt_plen_ptr(void* handle, double** p, int64_t* n);
+/* Actinic flux of the last run, which must have been a b200rt_run_act: [nslab][2][nz][ny][nx] (variable 0 direct, 1 total;
+ * laid out like the heating tally with the variable axis added).  b200rt_act_ptr: its device pointer and size. */
+int          b200rt_read_act(void* handle, double* dst, int64_t count);
+int          b200rt_act_ptr(void* handle, double** p, int64_t* n);
 /* Device pointers to the library-owned tallies (for in-place NCCL all-reduce by the caller). */
 int          b200rt_tally_ptrs(void* handle, double** flux, int64_t* nflux, double** rad, int64_t* nrad,
                                double** heat, int64_t* nheat);

@@ -78,7 +78,6 @@ struct DevJob {
 struct DevStats {
     unsigned long long photons, n_cell, n_tent, n_coll, n_sfc, n_le, n_le_visit, n_tally, n_kill;
     double w_toa, w_sfc, w_atm, w_rr;
-    unsigned long long hang;     // set by the watchdog of the role-specialised kernel (a warp idled for seconds)
 };
 
 struct DevScene {
@@ -422,7 +421,7 @@ struct Photon {
     uint32_t rc0, rc1, rc2;   // Philox counter: global photon index (lo, hi), draw number
     float M;          // majorant of the cell in which the photon parked at a tentative collision
 };
-enum { FL_DIRECT = 1, FL_FROZEN = 2, FL_STALE = 4, FL_ABS = 8, FL_FSCALE = 16, FL_IN3 = 32, FL_EMPTY = 64, FL_ESC = 128 };
+enum { FL_DIRECT = 1, FL_FROZEN = 2, FL_STALE = 4, FL_ABS = 8, FL_FSCALE = 16, FL_IN3 = 32, FL_EMPTY = 64 };
 
 // pool record: NFIELD 32-bit words per slot, structure-of-arrays ([field][slot]) so that lanes touch distinct banks
 enum { F_X = 0, F_Y, F_Z, F_DX, F_DY, F_DZ, F_W, F_TAU, F_CELL, F_LAY, F_ORD, F_JOB, F_ZA, F_LEG, F_RC0, F_RC1, F_RC2, F_M, F_AUX, NFIELD };
@@ -1274,11 +1273,7 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
     int nD = NP, nF = 0, nE = 0, nC = 0, nS = 0;
     const int ND_DONE = -(1 << 29);
 
-#ifdef RT_NO_POP_SYNC
-#define POP_SYNC()
-#else
 #define POP_SYNC() __syncwarp()
-#endif
 #define RNG4(out)                                                                                     \
     {                                                                                                 \
         const unsigned long long seed_ = S.jobs[p.job].seed;                                          \
@@ -1920,11 +1915,6 @@ __global__ void __launch_bounds__(RT_TPB, RT_MINB) transport_kernel(const __grid
         }
     }
 }
-// The role-specialised variant (geometry warps / event warps, block-level pool, setmaxnreg) is an experiment that
-// measured SLOWER than this kernel on every config (profiles/README.md, r02_c); it is compiled only on request.
-#ifdef B200RT_WITH_V9
-#include "../../experiments/transport_v9.cuh"
-#endif
 #undef ACC_ADD
 #undef CNT_ADD
 
@@ -2217,6 +2207,10 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     if (opt->nslab < 1) return fail(H, B200RT_ERR_ARG, "nslab must be >= 1");
     if (opt->solver < 0 || opt->solver > 2) return fail(H, B200RT_ERR_ARG, "unknown solver mode");
     if (opt->shard_world < 1 || opt->shard_rank < 0 || opt->shard_rank >= opt->shard_world) return fail(H, B200RT_ERR_ARG, "bad shard rank/world");
+    if (opt->pool_slots != 0 && opt->pool_slots != 64 && opt->pool_slots != 96 && opt->pool_slots != 128)
+        return fail(H, B200RT_ERR_ARG, "pool_slots must be 0 (auto), 64, 96 or 128");
+    if (opt->kernel != 0 && opt->kernel != 8)
+        return fail(H, B200RT_ERR_ARG, "options.kernel must be 0 (auto) or 8 (the role-specialised kernel 9 was removed)");
     if (sc->sfc_nx < 1 || sc->sfc_ny < 1 || !sc->sfc_type || !sc->sfc_param) return fail(H, B200RT_ERR_ARG, "surface missing");
 
     std::vector<double> zg, e1, o1, a1;
@@ -2639,9 +2633,6 @@ int b200rt_upload_scene(void* handle, const b200rt_scene* sc, const b200rt_optio
     H->k_cam = false;
     for (int k = 0; k < sc->nrad; ++k) if (sc->sensors[k].kind == 1) H->k_cam = true;
     H->pool_slots = opt->pool_slots;
-    if (H->pool_slots != 0 && H->pool_slots != 64 && H->pool_slots != 96 && H->pool_slots != 128 &&
-        H->pool_slots != 1024 && H->pool_slots != 1536 && H->pool_slots != 2048)
-        return fail(H, B200RT_ERR_ARG, "pool_slots must be 0 (auto), 64, 96 or 128 (per warp) -- or 1024, 1536, 2048 per block in builds with the role-specialised experiment");
     H->opt = *opt;
     H->have_scene = true;
     H->ran = false;
@@ -2670,8 +2661,6 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     DevScene& S = H->S;
     const int nz = S.nz;
     const bool k_rad = (S.target & B200RT_TARGET_RADIANCE) != 0 && S.nrad > 0;
-    const char* kenv = getenv("B200RT_KERNEL");
-    const int kver = kenv ? atoi(kenv) : (H->opt.kernel == 9 ? 9 : 8);
     int kd_n = 0;
     if (kd) {
         if (H->k_pl)
@@ -2679,7 +2668,6 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
                                            "need options.smem_tally = -1)");
         if (!k_rad) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: needs the radiance target and at least one sensor");
         if (H->k_cam) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: the all-sky camera (Rad_mrkind = 1) is not supported");
-        if (kver == 9) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: not available with options.kernel = 9");
         for (int j = 0; j < njob; ++j) {
             const b200rt_kd& k = kd[j];
             if (k.nkd < 1 || k.nkd > 32) return fail(H, B200RT_ERR_ARG, "b200rt_run_kd: nkd must be 1 ... 32");
@@ -2707,7 +2695,6 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
             return fail(H, B200RT_ERR_ARG, who + "needs the flux or heating target");
         if (H->k_cam) return fail(H, B200RT_ERR_ARG, who + "the all-sky camera (Rad_mrkind = 1) is not supported");
         if (k_rad) return fail(H, B200RT_ERR_ARG, who + "no radiance sensors in the same run (drop the radiance target)");
-        if (kver == 9) return fail(H, B200RT_ERR_ARG, who + "not available with options.kernel = 9");
         if (accumulate && H->ran && H->xt_mode != XM_ACT)
             return fail(H, B200RT_ERR_ARG, who + "accumulate needs the previous run to be an actinic run");
         nxt = 2 * size_t(H->opt.nslab) * nz * size_t(S.nx) * size_t(S.ny);
@@ -2718,7 +2705,6 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
                                                  "need options.smem_tally = -1)");
         if (!k_rad) return fail(H, B200RT_ERR_ARG, who + "needs the radiance target and at least one sensor");
         if (H->k_cam) return fail(H, B200RT_ERR_ARG, who + "the all-sky camera (Rad_mrkind = 1) is not supported");
-        if (kver == 9) return fail(H, B200RT_ERR_ARG, who + "not available with options.kernel = 9");
         if (edges) {
             const int ngrp = xa.ngrp;
             if (ngrp < 1 || ngrp > 64) return fail(H, B200RT_ERR_ARG, who + "ngrp must be 1 ... 64");
@@ -2876,34 +2862,7 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     // launch shape: the per-warp photon pools decide how many blocks fit on an SM (shared memory), see DESIGN.md
     int tpb = H->opt.threads_per_block > 0 ? H->opt.threads_per_block : RT_TPB;
     tpb = std::min(RT_TPB, std::max(32, (tpb / 32) * 32));
-#ifndef B200RT_WITH_V9
-    if (kver == 9) return fail(H, B200RT_ERR_ARG, "options.kernel = 9 (role-specialised experiment) is not part of this build (-DB200RT_WITH_V9)");
-#else
-    if (kver == 9) {
-        // role-specialised kernel: one block per SM, block-level photon pool (transport_v9.cuh)
-        int npb = H->pool_slots >= 1024 ? H->pool_slots : V9_NPB;
-        if (const char* e = getenv("B200RT_V9_POOL")) npb = atoi(e);
-#ifdef V9_ALL_POOLS
-        if (npb != 1024 && npb != 2048) npb = V9_NPB;
-#else
-        npb = V9_NPB;
-#endif
-        const bool uz = S.uz_ok != 0;
-        transport_fn9 kern = pick_v9(H->k_pl, H->k_fz, H->k_cam, uz, npb);
-        const size_t smem = H->smem_tables + 32 * (4 * 8 + 8 * 4) + size_t(V9_NT) * 8 + size_t(V9_POOL_WORDS(npb)) * 4 +
-                            8 * size_t(S.ntal_flux_smem + S.ntal_heat_smem + S.ntal_rad_smem) * size_t(S.tal_per_warp ? RT_TPB / 32 : 1);
-        if (smem > 227 * 1024) return fail(H, B200RT_ERR_ARG, "photon pool + 1-D tables exceed shared memory; lower pool_slots");
-        CK(set_smem_attr(H, (const void*)kern, smem));
-        const unsigned long long want = (acc + npb - 1) / npb;
-        const int grid = int(std::min<unsigned long long>((unsigned long long)H->numSM, std::max<unsigned long long>(1, want)));
-        CK(cudaEventRecord(H->ev0, st));
-        kern<<<grid, V9_NT, smem, st>>>(S);
-        CK(cudaGetLastError());
-        CK(cudaEventRecord(H->ev1, st));
-    } else
-#endif
-    {
-    const int np = H->pool_slots > 0 && H->pool_slots <= 128 ? H->pool_slots : 96;
+    const int np = H->pool_slots ? H->pool_slots : 96;
     int bps = 0;
     // UZ kernels: equally thick 3-D layers with runs (S.uz_ok) -- or no 3-D block at all (the layer search is dead code then)
     const bool k_uz = H->k_pl ? (S.nz3 <= 0 || size_t(S.nx) * S.ny <= 64) : ((S.uz_ok != 0 && H->cmz == 1) || S.nz3 <= 0);
@@ -2931,7 +2890,6 @@ static int run_jobs(Handle* H, const b200rt_job* jobs, const b200rt_kd* kd, cons
     kern<<<grid, tpb, smem, st>>>(S);
     CK(cudaGetLastError());
     CK(cudaEventRecord(H->ev1, st));
-    }
     H->last_stream = st;
     H->ran = true;
     H->inflight = true;
@@ -3017,7 +2975,6 @@ int b200rt_sync(void* handle) {
     o.bytes_alg = 4.0 * double(ds.n_cell) + 4.0 * double(ds.n_tent) + 8.0 * double(ds.n_coll) + 4.0 * double(ds.n_le_visit) +
                   8.0 * double(ds.n_tally) + 2.0 * 8.0 * double(H->nflux + H->nrad + H->nheat);
     o.launches = H->launches;
-    if (ds.hang) return fail(H, B200RT_ERR_STATE, "transport kernel watchdog: a warp idled for seconds (internal queue protocol error)");
     if (bad) return fail(H, B200RT_ERR_NUMERIC, "NaN/Inf found in tallies");
     return B200RT_OK;
 }

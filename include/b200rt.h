@@ -172,8 +172,7 @@ typedef struct b200rt_options {
     int32_t event_min;            /* lanes parked at an event that end a flight phase early; 0 = auto */
     int32_t empty_runs;           /* vertical merging of empty coarse cells into one box: 0 = auto (on when the 3-D
                                      layers are equally thick and no per-level tally is asked for), -1 = off        */
-    int32_t pool_slots;           /* photon slots in shared memory per warp: 64, 96 or 128; 0 = auto (96).  (1024, 1536, 2048
-                                     per block: only in builds with the role-specialised experiment, kernel 9) */
+    int32_t pool_slots;           /* photon slots in shared memory per warp: 64, 96 or 128; 0 = auto (96)             */
     int32_t iso_ss;               /* Pho_iso_SS: partial-3D switches to 1-D after this order   */
     int32_t iso_max;              /* Pho_iso_max: max scattering order sampled (0 = 1e6)       */
     int32_t threads_per_block;    /* 0 = auto                                                  */
@@ -182,9 +181,8 @@ typedef struct b200rt_options {
                                      scenes whose whole flux + heating tally is <= 2048 doubles (radiance: <= 512): lanes of a
                                      warp that hit the same address are summed first, one flush per block.  0 = auto (on),
                                      -1 = off (global atomics only), 2 = additionally one private copy per warp           */
-    int32_t kernel;               /* transport kernel: 0 = auto (8), 8 = every warp runs every phase on its own photon pool,
-                                     9 = experiment: role-specialised warps + block-level pool (only in builds made with
-                                     -DB200RT_WITH_V9; measured slower, see DESIGN.md)                                 */
+    int32_t kernel;               /* transport kernel: 0 = auto (8), 8 = every warp runs every phase on its own photon pool;
+                                     other values are rejected at upload                                               */
     int32_t _reserved;
     double  wmin;                 /* Pho_wmin: Russian roulette threshold (0 = no roulette)    */
     double  wfac;                 /* Pho_wfac: weight given to roulette survivors              */
@@ -226,8 +224,8 @@ int          b200rt_upload_scene(void* handle, const b200rt_scene* scene, const 
 int          b200rt_run(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream);
 
 /* b200rt_run with kd[j] the k-distribution terms of jobs[j] (radiance target with satellite sensors only: flux / heating
- * targets, the all-sky camera and options.kernel = 9 are rejected).  jobs[j].abs1d and .flx_scale must be NULL;
- * jobs[j].rad_scale is a factor common to all terms.  Same asynchronous contract as b200rt_run. */
+ * targets and the all-sky camera are rejected).  jobs[j].abs1d and .flx_scale must be NULL; jobs[j].rad_scale is a factor
+ * common to all terms.  Same asynchronous contract as b200rt_run. */
 int          b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd* kd, int njob, int accumulate, void* cuda_stream);
 
 /* b200rt_run that also tallies the radiance's derivatives with respect to the gas absorption of ngrp layer groups:
@@ -237,9 +235,9 @@ int          b200rt_run_kd(void* handle, const b200rt_job* jobs, const b200rt_kd
  * T_j is the gas optical path the history has collected in group j and tau_j that of the segment toward the sensor.  The
  * radiance, draws and event counters are those of b200rt_run (stats.n_tally also counts the Jacobian updates).  Atm_abst3d
  * and particle absorption are not differentiated.  Radiance target with satellite sensors only (flux / heating targets,
- * options.smem_tally >= 0 on scenes whose radiance tally fits shared memory, the all-sky camera and options.kernel = 9
- * are rejected).  With accumulate != 0 the previous run since the last upload, if any, must be a Jacobian run with the
- * same edges.  Same asynchronous contract as b200rt_run. */
+ * options.smem_tally >= 0 on scenes whose radiance tally fits shared memory and the all-sky camera are rejected).  With
+ * accumulate != 0 the previous run since the last upload, if any, must be a Jacobian run with the same edges.  Same
+ * asynchronous contract as b200rt_run. */
 int          b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, const int32_t* edges, int ngrp, int accumulate,
                             void* cuda_stream);
 
@@ -255,8 +253,8 @@ int          b200rt_run_jac(void* handle, const b200rt_job* jobs, int njob, cons
  * the fp32 path.  1 <= ntp <= 1024, 0 <= tpmin < tpmax, all finite.  The radiance, draws and event counters are those of
  * b200rt_run (stats.n_tally also counts the two updates per local estimate).  Radiance target with satellite sensors only,
  * every solver mode (flux / heating targets, options.smem_tally >= 0 on scenes whose radiance tally fits shared memory,
- * the all-sky camera and options.kernel = 9 are rejected).  With accumulate != 0 the previous run since the last upload,
- * if any, must be a path-length run with the same tpmin, tpmax and ntp.  Same asynchronous contract as b200rt_run. */
+ * and the all-sky camera are rejected).  With accumulate != 0 the previous run since the last upload, if any, must be a
+ * path-length run with the same tpmin, tpmax and ntp.  Same asynchronous contract as b200rt_run. */
 int          b200rt_run_plen(void* handle, const b200rt_job* jobs, int njob, double tpmin, double tpmax, int ntp, int accumulate,
                              void* cuda_stream);
 
@@ -267,8 +265,8 @@ int          b200rt_run_plen(void* handle, const b200rt_job* jobs, int njob, dou
  * so that a direct beam in vacuum gives Src_flx.  Two variables: 0 direct (photons that have not scattered), 1 total.
  * Trajectories never change, so flux, heating, draws and event counters are those of b200rt_run (stats.n_tally also
  * counts the actinic updates that go to global memory).  Flux and / or heating target only: radiance sensors in the same
- * run, the all-sky camera and options.kernel = 9 are rejected.  With accumulate != 0 the previous run since the last
- * upload, if any, must be an actinic run.  Same asynchronous contract as b200rt_run. */
+ * run and the all-sky camera are rejected.  With accumulate != 0 the previous run since the last upload, if any, must be
+ * an actinic run.  Same asynchronous contract as b200rt_run. */
 int          b200rt_run_act(void* handle, const b200rt_job* jobs, int njob, int accumulate, void* cuda_stream);
 
 /* Wait for the stream of the last run; checks tallies for NaN/Inf. */

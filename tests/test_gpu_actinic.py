@@ -216,9 +216,8 @@ def test_unsupported_runs_are_rejected_by_the_library(solver):
     solver.upload_scene(sc_rad, abi.make_options(target=abi.TARGET_RADIANCE | abi.TARGET_FLUX))
     with pytest.raises(OSError, match='run_act: no radiance sensors'):
         solver.run_act(jobs)
-    solver.upload_scene(scene, abi.make_options(target=FH, kernel=9))
-    with pytest.raises(OSError, match='run_act: not available with options.kernel = 9'):
-        solver.run_act(jobs)
+    with pytest.raises(OSError, match=r'options.kernel must be 0 \(auto\) or 8'):
+        solver.upload_scene(scene, abi.make_options(target=FH, kernel=9))
     solver.upload_scene(scene, opt)
     solver.run(jobs)
     with pytest.raises(OSError, match='accumulate needs the previous run to be an actinic run'):

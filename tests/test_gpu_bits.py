@@ -174,6 +174,10 @@ def test_errors_are_reported_not_swallowed(solver):
     with pytest.raises(OSError, match='travel downward'):
         solver.upload_scene(abi.HostScene(np.array([0.0, 1000.0]), [[1e-5]], [[1.0]], [[0.0]], src_the=60.0), abi.make_options())
     sc, _ = scenes.plane_parallel()
+    with pytest.raises(OSError, match=r'options.kernel must be 0 \(auto\) or 8'):
+        solver.upload_scene(sc, abi.make_options(target=abi.TARGET_FLUX, nslab=1, kernel=9))
+    with pytest.raises(OSError, match=r'pool_slots must be 0 \(auto\), 64, 96 or 128'):
+        solver.upload_scene(sc, abi.make_options(target=abi.TARGET_FLUX, nslab=1, pool_slots=1024))
     solver.upload_scene(sc, abi.make_options(target=abi.TARGET_FLUX, nslab=1))
     with pytest.raises(OSError, match='slab out of range'):
         jobs, keep = abi.make_jobs([10], [1], [5])

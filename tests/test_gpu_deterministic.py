@@ -25,9 +25,9 @@ NSLAB = 8
 RTOL = 2.0e-4
 
 
-def run_case(solver, fx, nphot_total, hom3d=False, kernel=0):
+def run_case(solver, fx, nphot_total, hom3d=False):
     sc = scenes.ad_scene(fx, hom3d=hom3d)
-    opt = abi.make_options(target=abi.TARGET_FLUX | abi.TARGET_RADIANCE, nslab=NSLAB, wmin=0.2, kernel=kernel)
+    opt = abi.make_options(target=abi.TARGET_FLUX | abi.TARGET_RADIANCE, nslab=NSLAB, wmin=0.2)
     jobs, keep = scenes.multi_seed_jobs(int(nphot_total // NSLAB), NSLAB, abs1d=fx['absg'])
     solver.upload_scene(sc, opt)
     solver.run(jobs)

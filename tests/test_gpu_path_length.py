@@ -241,9 +241,8 @@ def test_unsupported_runs_are_rejected_by_the_library(solver):
     solver.upload_scene(scene, abi.make_options(target=abi.TARGET_RADIANCE | abi.TARGET_FLUX))
     with pytest.raises(OSError, match='run_plen: radiance targets only'):
         solver.run_plen(jobs, *BINS)
-    solver.upload_scene(scene, abi.make_options(target=opt.target, smem_tally=-1, kernel=9))
-    with pytest.raises(OSError, match='run_plen: not available with options.kernel = 9'):
-        solver.run_plen(jobs, *BINS)
+    with pytest.raises(OSError, match=r'options.kernel must be 0 \(auto\) or 8'):
+        solver.upload_scene(scene, abi.make_options(target=opt.target, smem_tally=-1, kernel=9))
     solver.upload_scene(scene, opt)
     for bins, msg in (((0.0, 1e5, 0), 'ntp must be 1 ... 1024'), ((0.0, 1e5, 1025), 'ntp must be 1 ... 1024'),
                       ((-1.0, 1e5, 8), '0 <= tpmin < tpmax'), ((1e5, 1e5, 8), '0 <= tpmin < tpmax'),

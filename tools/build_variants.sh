@@ -1,5 +1,5 @@
 #!/bin/bash
-# Build library variants for on-box A/B runs: tools/build_variants.sh NAME "-DV9_NWF=12 -DV9_NWE=12 ..." [NAME2 "flags2" ...]
+# Build library variants for on-box A/B runs: tools/build_variants.sh NAME "-DRT_MINB=1 ..." [NAME2 "flags2" ...]
 # The result is tools/variants/lib<NAME>.so, selected at run time with $ER3T_B200_LIB (tools/gpu_variants.sh).
 cd "$(dirname "$0")/.."
 mkdir -p tools/variants
